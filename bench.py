@@ -2,7 +2,7 @@
 """Headline benchmark: Vicon CSV loader throughput (GB of CSV per second, output bit-exact) on synthetic 10-minute
 trials of the dynamic_trial.csv layout (BASELINE.json configs[1]).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 One step = one pass of the hot path over one trial per GPU: the single-pass loader kernel (ms_load_fused: every data
 row of both sections -> channel-major float64 in HBM) + Segmenter (40 transitions) + gather of the 32 phase windows
@@ -18,6 +18,12 @@ tmpfs -> host arrays) and `configs[4]` (files -> synergies).
 muscle_synergies.load_vicon_file + project/segment.py Segmenter + the 32 EMG phase windows per trial in a persistent
 multiprocessing.Pool over all host cores, on a bounded sample of the same layout; and scikit-learn's NMF(mu) over
 the same cores.
+
+`--dump-outputs DIR` writes, after the timed steps, what the last streamed step handed its caller (rank 0): the two
+section blocks, the 40 transitions and the 32 EMG phase windows, as DIR/<name>.npy (float64; seeded samples of rows
+where a block is larger than DUMP_ELEMENTS; NaN and infinities written as 0 and marked in a float32 code array), so
+that two builds can be compared output for output.  The benchmark reads the library that `__graft_entry__.build()`
+left in the tree (with a warning if it is older than the CUDA sources) and writes nothing there.
 """
 import argparse
 import json
@@ -346,6 +352,60 @@ def bench_nmf(dev, iters=2000):
     return out
 
 
+# ---- outputs of the timed path ------------------------------------------------------------------------------
+DUMP_ELEMENTS = 1 << 20  # per sampled array: 8 MiB of float64 + 4 MiB of float32 codes, three such pairs under 64 MB
+# codes of `<name>_nonfinite.npy`: what stood where `<name>.npy` holds 0 (a blank CSV field is NaN, as in the reference)
+NONFINITE_CODES = {"nan": 1.0, "+inf": 2.0, "-inf": 3.0}
+
+
+def sample_rows(n_ch, n_rows, seed):
+    """Ascending row indices of a fixed, seeded sample: every row if all of them fit DUMP_ELEMENTS, else as many
+    whole rows (all channels) as fit."""
+    import numpy as np
+
+    keep = max(1, DUMP_ELEMENTS // max(1, n_ch))
+    if keep >= n_rows:
+        return np.arange(n_rows, dtype=np.int64)
+    return np.sort(np.random.default_rng(seed).choice(n_rows, keep, replace=False))
+
+
+def split_nonfinite(a):
+    """(a with every NaN / infinity replaced by 0, float32 array of NONFINITE_CODES, 0 where a is finite)."""
+    import numpy as np
+
+    codes = np.zeros(a.shape, dtype=np.float32)
+    codes[np.isnan(a)] = NONFINITE_CODES["nan"]
+    codes[np.isposinf(a)] = NONFINITE_CODES["+inf"]
+    codes[np.isneginf(a)] = NONFINITE_CODES["-inf"]
+    return np.where(codes == 0, a, 0.0), codes
+
+
+def dump_outputs(out_dir, data, seg, windows):
+    """Writes what one step hands its caller - the trial's section blocks, the Segmenter's transitions and the 32
+    phase windows of the EMG device - as .npy files of finite floats.  A channel-major (channels, rows) array larger
+    than DUMP_ELEMENTS is sampled by rows (`<name>_rows.npy` holds the row indices); its non-finite entries are
+    written as 0 and told apart in `<name>_nonfinite.npy` (NONFINITE_CODES)."""
+    import numpy as np
+    import torch
+
+    def put(name, a, dtype=np.float64):
+        np.save(os.path.join(out_dir, f"{name}.npy"), np.ascontiguousarray(a, dtype=dtype))
+
+    def put_sampled(name, t, seed):
+        rows = sample_rows(int(t.shape[0]), int(t.shape[1]), seed)
+        values, codes = split_nonfinite(t.index_select(1, torch.from_numpy(rows).to(t.device)).cpu().numpy())
+        put(name, values)
+        put(f"{name}_nonfinite", codes, np.float32)
+        put(f"{name}_rows", rows)
+
+    os.makedirs(out_dir, exist_ok=True)
+    for seed, (name, blk) in enumerate(zip(("devices", "trajectories"), data.blocks)):
+        put_sampled(name, blk.tensor[:, : blk.n_rows], seed)
+    put("transitions", np.asarray(seg.transitions))
+    put_sampled("emg_phase_windows", torch.cat(list(windows), dim=1), 2)
+    put("emg_phase_window_bounds", np.cumsum([0] + [int(w.shape[1]) for w in windows]))
+
+
 # ---- our arm ------------------------------------------------------------------------------------------------
 def run_ours(args):
     import ctypes
@@ -371,14 +431,13 @@ def run_ours(args):
 
         dist.init_process_group("nccl", device_id=dev)
 
-    import __graft_entry__ as entry
-
-    if rank == 0:
-        entry.build()
-    if dist is not None:
-        dist.barrier()
     import muscle_synergies_b200 as ms
     from muscle_synergies_b200 import _native
+    from muscle_synergies_b200.csrc import build as cuda_build
+
+    if rank == 0 and cuda_build.stale():
+        print(f"bench.py: warning: {cuda_build.OUT} is missing or older than its CUDA sources; "
+              "run __graft_entry__.build() to time the current code", file=sys.stderr)
     from muscle_synergies_b200.segment import Segmenter
     from muscle_synergies_b200.vicon_data import loader as loader_mod
     from tools.synth_vicon import synth_layout
@@ -443,7 +502,8 @@ def run_ours(args):
     def steps_streamed(k):
         # the same K steps as a stream of trials (what a 1000-trial job is): load_device_many keeps the loader kernel of
         # the next two trials queued on its own stream while the host finishes trial i's objects and runs Segmenter + the
-        # window gather on it - every step still ends with the 40 transitions and the 32 windows of ITS trial on the host
+        # window gather on it - every step still ends with the 40 transitions and the 32 windows of ITS trial on the host.
+        # Returns (data, Segmenter, windows) of the last step.
         out, begun = None, None
         work = loader.work_stream  # high priority: the small kernels of a step run beside the next trial's loader kernel
         for data in loader.load_device_many(((d_bytes, n) for _ in range(k)), depth=args.depth, stream=work):
@@ -452,10 +512,12 @@ def run_ours(args):
             if begun is not None:  # the trial before: its transitions and windows are on the host by now
                 out = begun[0].finish().phase_cuts(begun[1].emg)
             begun = (pending, data)
+        data, seg = None, None
         if begun is not None:
-            out = begun[0].finish().phase_cuts(begun[1].emg)
+            seg, data = begun[0].finish(), begun[1]
+            out = seg.phase_cuts(data.emg)
         torch.cuda.current_stream().wait_stream(work)  # the closing event is recorded after the last step's kernels
-        return out
+        return data, seg, out
 
     for _ in range(max(3, args.warmup)):
         step_resident()
@@ -466,10 +528,14 @@ def run_ours(args):
     steps_streamed(max(12, args.warmup))
     path_used = dict(loader.stats)
     launches0 = _native.launch_count()
+    last = []
     with ClockSampler(local_rank) as clocks:
-        ms_total = timed(lambda: steps_streamed(args.steps), 1)
+        ms_total = timed(lambda: last.append(steps_streamed(args.steps)), 1)
     launches = _native.launch_count() - launches0
     value = world * n * args.steps / (ms_total * 1e-3) / 1e9
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, *last[0])
+    del last
 
     # ---- kernel-only timings on the launching stream (roofline of the loader: ONE kernel reads the CSV and writes the arrays)
     stream = torch.cuda.current_stream()
@@ -715,13 +781,19 @@ def run_ours(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=int(os.environ.get("WORLD_SIZE", "1")))
-    ap.add_argument("--steps", type=int, default=50)
+    ap.add_argument("--steps", type=int, default=50,
+                    help="timed steps of the headline (streamed) and serial legs; the e2e leg times min(max(K, 4), 8) "
+                         "trials and reports its own count")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--layout", default="T10", help="synthetic layout (tools/synth_vicon.py LAYOUTS)")
     ap.add_argument("--no-cpu", action="store_true", help="skip the CPU baseline leg")
     ap.add_argument("--depth", type=int, default=2, help="trials in flight in the streamed headline loop (load_device_many)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed to DIR/<name>.npy (finite floats, at most 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference(args)
     else:

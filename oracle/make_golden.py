@@ -15,6 +15,8 @@ Outputs
   synth_D_digest.json          sha256 of every reference array for the 41.6 MB D-layout trial
   segment_D.json               reference Segmenter output (40 transitions, 32 slices) on it
   float_table.json             CPython float() known answers (Appendix B of SURVEY.md)
+  emg_pinning.npz              EMG preprocessing outputs on a seeded signal (seeded sample of rows)
+  segment_pinning.json         transition search results on seeded on/off force-plate signals
 """
 import hashlib
 import json
@@ -144,6 +146,87 @@ def sha(arr: np.ndarray) -> str:
     return hashlib.sha256(np.ascontiguousarray(arr).tobytes()).hexdigest()
 
 
+# ---- inputs and outputs that pin oracle/emg_oracle.py and oracle/segment_oracle.py to the reference ----------
+EMG_ENVELOPES = (dict(order=4), dict(order=2, zero_lag=False), dict(order=3, filter_type="cheby1", cheby_param=1.0),
+                 dict(order=4, filter_type="cheby2", cheby_param=30.0))
+EMG_GOLDEN_ROWS = 400  # a seeded sample of the 5000 rows keeps emg_pinning.npz small
+
+
+def emg_pinning_input():
+    """The seeded (5000, 6) EMG-like signal the preprocessing functions are compared on."""
+    return np.random.default_rng(0).normal(0.001, 0.01, (5000, 6))
+
+
+def emg_reference_outputs(ms, x):
+    """name -> (rows, channels) output of each reference call; emg_oracle_outputs makes the same calls."""
+    import pandas as pd
+
+    df = pd.DataFrame(x, columns=list("abcdef"))
+    out = {"zero_center": ms.zero_center(df), "rms": ms.rms(df, 0.5, sampling_frequency=2000),
+           "normalize": ms.normalize(df), "time_normalize": ms.time_normalize(df, 200)}
+    for i, kw in enumerate(EMG_ENVELOPES):
+        out[f"linear_envelope_{i}"] = ms.analysis.linear_envelope(df, 6.0, 2000, **kw)
+    out["digital_filter_bandpass"] = ms.analysis.digital_filter(df, (20.0, 450.0), 2000, 4, band_type="bandpass")
+    out["linear_envelope_no_zero_center"] = ms.analysis.linear_envelope(df, 6.0, 2000, 4, zero_center_=False)
+    return {k: v.to_numpy() for k, v in out.items()}
+
+
+def emg_oracle_outputs(x):
+    from oracle import emg_oracle as eo
+
+    out = {"zero_center": eo.zero_center(x), "rms": eo.rms(x, 1000), "normalize": eo.normalize(x),
+           "time_normalize": eo.time_normalize(x, 200)}
+    for i, kw in enumerate(EMG_ENVELOPES):
+        out[f"linear_envelope_{i}"] = eo.linear_envelope(x, 6.0, 2000, **kw)
+    out["digital_filter_bandpass"] = eo.digital_filter(x, (20.0, 450.0), 2000, 4, band_type="bandpass")
+    out["linear_envelope_no_zero_center"] = eo.linear_envelope(x, 6.0, 2000, 4, zero_center_=False)
+    return out
+
+
+def emg_golden_rows(n_rows):
+    if n_rows <= EMG_GOLDEN_ROWS:
+        return np.arange(n_rows)
+    return np.sort(np.random.default_rng(1).choice(n_rows, EMG_GOLDEN_ROWS, replace=False))
+
+
+def segment_pinning_signals():
+    """Six seeded on/off force-plate signal pairs (runs of 1 to 120 samples) for the transition search."""
+    rnd = np.random.default_rng(3)
+    for _ in range(6):
+        n = int(rnd.integers(300, 5000))
+        left, right = np.zeros(n), np.zeros(n)
+        i = 0
+        while i < n:
+            run = int(rnd.choice([1, 3, 9, 10, 11, 30, 120]))
+            state = rnd.integers(0, 4)
+            left[i : i + run] = 1.0 if state & 1 else 0.0
+            right[i : i + run] = 1.0 if state & 2 else 0.0
+            i += run
+        yield left, right
+
+
+def segment_pinning_cases():
+    """(left, right, k) per signal pair that has alternations: k = min(alternations found, 12) transitions asked for."""
+    from oracle import segment_oracle as so
+
+    for left, right in segment_pinning_signals():
+        k = min(len(so.transition_indices(left, right, 10, 0)), 12)
+        if k:
+            yield left, right, k
+
+
+def write_pinning_golden(emg_outputs, segment_transitions, source):
+    """tests/golden/emg_pinning.npz (sampled rows of every EMG output) and segment_pinning.json (transitions)."""
+    x = emg_pinning_input()
+    arrays = {"input": x[emg_golden_rows(len(x))], "source": np.array(source)}
+    for name, a in emg_outputs.items():
+        arrays[name] = np.ascontiguousarray(a[emg_golden_rows(len(a))], dtype=np.float64)
+    np.savez(os.path.join(GOLD, "emg_pinning.npz"), **arrays)
+    cases = [{"n": len(left), "k": k, "transitions": [int(t) for t in segment_transitions(left, right, k)]}
+             for left, right, k in segment_pinning_cases()]
+    json.dump({"source": source, "cases": cases}, open(os.path.join(GOLD, "segment_pinning.json"), "w"), indent=1)
+
+
 def main():
     ms, seg = import_reference()
     os.makedirs(os.path.join(GOLD, "variants"), exist_ok=True)
@@ -249,6 +332,14 @@ def main():
         except ValueError:
             table[t] = "ValueError"
     json.dump(table, open(os.path.join(GOLD, "float_table.json"), "w"), indent=1, sort_keys=True)
+
+    # 6. the preprocessing functions and the transition search on seeded inputs
+    import pandas as pd
+
+    write_pinning_golden(
+        emg_reference_outputs(ms, emg_pinning_input()),
+        lambda left, right, k: seg._transition_indices(pd.Series(left), pd.Series(right), 10, k),
+        "the reference (elvis-sik/muscle_synergies), by oracle/make_golden.py")
     print("golden fixtures written to", GOLD)
 
 

@@ -1,10 +1,37 @@
-"""Pins oracle/emg_oracle.py against the live reference preprocessing functions (build container only)."""
+"""Pins oracle/emg_oracle.py against the reference preprocessing functions: live where a reference checkout is present,
+and against their stored outputs (tests/golden/emg_pinning.npz) everywhere."""
+import os
+
 import numpy as np
-import pandas as pd
 import pytest
 
+from conftest import GOLDEN
 from oracle import emg_oracle as eo
+from oracle import make_golden as mg
 from oracle.refstub import reference_available
+
+
+def golden():
+    with np.load(os.path.join(GOLDEN, "emg_pinning.npz")) as z:
+        return {k: z[k] for k in z.files}
+
+
+def assert_matches_golden(outputs, gold):
+    """The stored rows of every output.  1e-12 relative: the stored values come from another numpy / scipy build,
+    whose vectorised sums (np.convolve's dot products) may add in another order."""
+    assert sorted(outputs) == sorted(k for k in gold if k not in ("input", "source"))
+    for name, a in outputs.items():
+        want = gold[name]
+        got = a[mg.emg_golden_rows(len(a))]
+        assert got.shape == want.shape, name
+        np.testing.assert_allclose(got, want, rtol=1e-12, atol=1e-12 * np.abs(want).max(), err_msg=name)
+
+
+def test_oracle_equals_reference_golden():
+    gold = golden()
+    x = mg.emg_pinning_input()
+    assert np.array_equal(x[mg.emg_golden_rows(len(x))], gold["input"])  # the seeded input is the one recorded
+    assert_matches_golden(mg.emg_oracle_outputs(x), gold)
 
 
 @pytest.mark.reference
@@ -13,22 +40,13 @@ def test_oracle_equals_reference_functions():
     from oracle.refstub import import_reference
 
     ms, _ = import_reference()
-    rng = np.random.default_rng(0)
-    x = rng.normal(0.001, 0.01, (5000, 6))
-    df = pd.DataFrame(x, columns=list("abcdef"))
-    assert np.array_equal(ms.zero_center(df).to_numpy(), eo.zero_center(x))
-    assert np.array_equal(ms.rms(df, 0.5, sampling_frequency=2000).to_numpy(), eo.rms(x, 1000))
-    assert np.array_equal(ms.normalize(df).to_numpy(), eo.normalize(x))
-    assert np.array_equal(ms.time_normalize(df, 200).to_numpy(), eo.time_normalize(x, 200))
-    # filters: the oracle makes the reference's scipy calls
-    for kw in (dict(order=4), dict(order=2, zero_lag=False), dict(order=3, filter_type="cheby1", cheby_param=1.0),
-               dict(order=4, filter_type="cheby2", cheby_param=30.0)):
-        want = ms.analysis.linear_envelope(df, 6.0, 2000, **kw).to_numpy()
-        assert np.array_equal(want, eo.linear_envelope(x, 6.0, 2000, **kw))
-    want = ms.analysis.digital_filter(df, (20.0, 450.0), 2000, 4, band_type="bandpass").to_numpy()
-    assert np.array_equal(want, eo.digital_filter(x, (20.0, 450.0), 2000, 4, band_type="bandpass"))
-    want = ms.analysis.linear_envelope(df, 6.0, 2000, 4, zero_center_=False).to_numpy()
-    assert np.array_equal(want, eo.linear_envelope(x, 6.0, 2000, 4, zero_center_=False))
+    x = mg.emg_pinning_input()
+    want = mg.emg_reference_outputs(ms, x)
+    got = mg.emg_oracle_outputs(x)
+    assert sorted(got) == sorted(want)
+    for name in want:  # the oracle makes the reference's numpy / scipy calls
+        assert np.array_equal(want[name], got[name]), name
+    assert_matches_golden(want, golden())
 
 
 def test_same_convolution_window_alignment():

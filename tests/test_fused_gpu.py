@@ -76,7 +76,7 @@ def test_bit_exact_at_every_tile_size(env, kw):
         assert (bits(got_traj) == bits(want_traj)).all(), tile
 
 
-def test_line_ends_and_eof_shapes(env):
+def test_line_ends_and_eof_shapes(env, tmp_path):
     """LF, CRLF and lone CR files; with and without a final line end; with and without the trailing blank row."""
     from oracle import vicon_oracle as vo
 
@@ -97,7 +97,7 @@ def test_line_ends_and_eof_shapes(env):
                 if trailing_blank:
                     lines.append("," * (1 + 3 * mark))
                 blob = (eol.join(lines) + (eol if final_eol else "")).encode()
-                path = "/tmp/ms_b200_eof_case.csv"
+                path = tmp_path / "eof_case.csv"
                 with open(path, "wb") as f:
                     f.write(blob)
                 want = vo.load_vicon_file_oracle(path)

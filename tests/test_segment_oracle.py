@@ -1,4 +1,5 @@
-"""Pins oracle/segment_oracle.py against the reference Segmenter's own output (golden)."""
+"""Pins oracle/segment_oracle.py against the reference Segmenter: its stored output (golden) everywhere, and live
+where a reference checkout is present."""
 import json
 import os
 
@@ -6,6 +7,7 @@ import numpy as np
 import pytest
 
 from conftest import GOLDEN
+from oracle import make_golden as mg
 from oracle import segment_oracle as so
 from oracle import vicon_oracle_fast as vof
 from oracle.refstub import reference_available
@@ -36,6 +38,17 @@ def test_transitions_and_windows_match_reference(d_arrays):
         assert [b - a, 3] == w["traj0_shape"]
 
 
+def test_transition_search_matches_reference_golden():
+    """Runs shorter than min_phase_size, fewer alternations than asked for: the stored results of the transition
+    search on seeded on/off signals."""
+    gold = json.load(open(os.path.join(GOLDEN, "segment_pinning.json")))["cases"]
+    cases = list(mg.segment_pinning_cases())
+    assert len(cases) == len(gold)
+    for (left, right, k), want in zip(cases, gold):
+        assert (len(left), k) == (want["n"], want["k"])
+        assert so.transition_indices(left, right, 10, k) == want["transitions"]
+
+
 @pytest.mark.reference
 @pytest.mark.skipif(not reference_available(), reason="reference checkout not present")
 def test_oracle_equals_live_reference_on_random_signals():
@@ -44,20 +57,8 @@ def test_oracle_equals_live_reference_on_random_signals():
     from oracle.refstub import import_reference
 
     _ms, seg = import_reference()
-    rnd = np.random.default_rng(3)
-    for _ in range(6):
-        n = int(rnd.integers(300, 5000))
-        left, right = np.zeros(n), np.zeros(n)
-        i = 0
-        while i < n:
-            run = int(rnd.choice([1, 3, 9, 10, 11, 30, 120]))
-            state = rnd.integers(0, 4)
-            left[i : i + run] = 1.0 if state & 1 else 0.0
-            right[i : i + run] = 1.0 if state & 2 else 0.0
-            i += run
-        found_all = so.transition_indices(left, right, 10, 0)
-        k = min(len(found_all), 12)
-        if k == 0:
-            continue
+    gold = json.load(open(os.path.join(GOLDEN, "segment_pinning.json")))["cases"]
+    for (left, right, k), want in zip(mg.segment_pinning_cases(), gold):
         ref = [int(x) for x in seg._transition_indices(pd.Series(left), pd.Series(right), 10, k)]
         assert ref == so.transition_indices(left, right, 10, k)
+        assert ref == want["transitions"]
