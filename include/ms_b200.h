@@ -300,6 +300,41 @@ int ms_nmf_mu_stream(const float* d_X, int64_t n, int32_t m, const int32_t* h_ra
                      int32_t n_problems, float* d_W, float* d_H, int32_t max_iter, float tol, int32_t check_every,
                      void* d_work, int32_t* d_n_iter, float* d_err, float* d_vaf, void* stream);
 
+/* ---- NMF by coordinate descent, NNDSVD initialisation (extension; fp64) ----------------------- */
+
+/* scikit-learn's default solver="cd" (shuffle=False, no regularisation; _nmf.py _fit_coordinate_descent,
+ * _cdnmf_fast.pyx) for a batch of problems, in fp64: per iteration a coordinate sweep of W with H H^T and X H^T of the
+ * current H, then of H with W^T W and X^T W of the updated W; the summed projected-gradient violation of iteration 1
+ * is violation_init, and a problem stops when that is 0 or violation / violation_init <= tol (tol = 0: max_iter
+ * iterations).  Same batch description as the MU entries: d_X one or more [n][m] row-major fp64 matrices, d_table
+ * the 32-byte problem table of ms_nmf_plan in device memory (ranks 1..16, m <= 64), d_W / d_H the initial factors
+ * packed problem after problem (fp64), overwritten with the results.  Outputs per problem: d_n_iter, d_err =
+ * ||X - W H||_F, d_vaf [m + 1] = 1 - SS_res / SS_tot overall, then per column (analysis.py:642-667), all fp64.
+ * ms_nmf_cd_batched_planned keeps each problem in the shared memory of one CTA (n <= ms_nmf_cd_resident_max_rows). */
+int32_t ms_nmf_cd_resident_max_rows(int32_t m, int32_t kmax);
+int ms_nmf_cd_batched_planned(const double* d_X, int32_t n, int32_t m, const void* d_table, int32_t n_problems,
+                              int32_t kmax, double* d_W, double* d_H, int32_t max_iter, double tol, int32_t* d_n_iter,
+                              double* d_err, double* d_vaf, void* stream);
+
+/* Same contract for X of any length: per iteration one pass over X [n][m] and W [n][k] in HBM (the W step, W^T W,
+ * X^T W and the violation; algorithmic bytes 8 n m + P * 16 n k when every problem shares one X), then one small
+ * kernel per problem for the H step and the stop test.  Synchronises `stream` every 64 iterations to stop once every
+ * problem has converged.  d_work: ms_nmf_cd_stream_workspace_bytes(m, n_problems), 256-byte aligned. */
+int64_t ms_nmf_cd_stream_workspace_bytes(int32_t m, int32_t n_problems);
+int ms_nmf_cd_stream(const double* d_X, int64_t n, int32_t m, const void* d_table, int32_t n_problems, int32_t kmax,
+                     double* d_W, double* d_H, int32_t max_iter, double tol, void* d_work, int32_t* d_n_iter,
+                     double* d_err, double* d_vaf, void* stream);
+
+/* _initialize_nmf(X, k, init="nndsvd" (variant 0) or "nndsvda" (variant 1)) for every problem of a batch, written to
+ * the packed d_W / d_H (fp64).  The singular triplets are exact (X^T X, cyclic Jacobi eigensolver, U = X V S^-1),
+ * one SVD per matrix of the stack (n_matrices [n][m] matrices in d_X); scikit-learn's come from a randomized SVD, so
+ * its random_state has no counterpart here.  kmax <= min(n, m).  *d_status (device) is set non-zero when the init
+ * would divide by zero: a singular value needed is 0 (at most m * eps * the largest one) or the chosen part of a
+ * singular vector pair is empty; the factors are then meaningless.  d_work: ms_nndsvd_workspace_bytes(m, n_matrices). */
+int64_t ms_nndsvd_workspace_bytes(int32_t m, int32_t n_matrices);
+int ms_nndsvd_init(const double* d_X, int64_t n, int32_t m, int32_t n_matrices, const void* d_table, int32_t n_problems,
+                   int32_t kmax, int32_t variant, void* d_work, double* d_W, double* d_H, int32_t* d_status, void* stream);
+
 /* ---- misc ------------------------------------------------------------------------------- */
 /* The used part of a channel-major block (rows channels of width_bytes each, src_pitch_bytes apart) to host
  * memory as one 2-D copy on the DMA engine; asynchronous when h_dst is page-locked. */

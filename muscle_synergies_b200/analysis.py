@@ -1,4 +1,4 @@
-"""Muscle-synergy extraction on the GPU: batched NMF by multiplicative updates (EXTENSION).
+"""Muscle-synergy extraction on the GPU: batched NMF by multiplicative updates and by coordinate descent (EXTENSION).
 
 API mirror of the reference's `vaf`, `SynergyRunResult` and `find_synergies`
 (src/muscle_synergies/analysis.py:597-667, 670-710, 713-914).  The reference hands the
@@ -7,13 +7,23 @@ solver="mu", beta_loss="frobenius", init="random" case runs as ONE CUDA launch f
 rank sweep x restarts grid (csrc/ms_nmf.cu), in fp32, with sklearn's initialisation
 (`RandomState(seed)`: H drawn first, then W - sklearn/decomposition/_nmf.py:_initialize_nmf)
 generated on the host so that a run is comparable to `NMF(solver="mu", init="random",
-random_state=seed)` at the same iteration count.  Every other call (sklearn's default solver="cd",
+random_state=seed)` at the same iteration count.  By default every other call (sklearn's default solver="cd",
 nndsvd inits, regularisation ...) is forwarded to scikit-learn, exactly as the reference does
 (analysis.py:848-864): this stage is an extension, not a replacement of scikit-learn.
+
+`find_synergies(..., engine="gpu")` and `nmf_cd_batched` also run sklearn's default solver="cd" (shuffle=False, no
+regularisation) on the GPU, in fp64 (csrc/ms_nmf_cd.cu), with init "nndsvd" / "nndsvda" computed on the device or
+sklearn's "random" draws.  Parity claim, against `NMF(solver="cd")` in fp64: from the same init and at the same
+iteration count (tol=0), W H, VAF (overall and per muscle) and ||X - W H||_F / ||X||_F agree to 1e-9; run to
+convergence with the reference's defaults (tol=1e-6, max_iter=100 000) from the device's NNDSVD init, VAF agrees to
+1e-8 and n_iter to max(3, 0.5 %).  Deviation: the device's NNDSVD uses an exact SVD where sklearn uses a randomized
+one, so sklearn's random_state has no effect on it; the two inits agree to ~1e-13 relative where sklearn's randomized
+SVD is itself accurate (tests/test_nmf_cd_gpu.py).
 """
 import ctypes
 import functools
 import threading
+import warnings
 from collections import OrderedDict
 from dataclasses import dataclass, field
 from collections.abc import Sequence
@@ -30,8 +40,8 @@ from . import _native as nat
 class NMFBatchResult:
     ranks: np.ndarray          # (P,)
     seeds: np.ndarray          # (P,)
-    W: Sequence                # P arrays (n, k_p) float32 (views of one packed array, made on access)
-    H: Sequence                # P arrays (k_p, m) float32
+    W: Sequence                # P arrays (n, k_p) float32 (mu) / float64 (cd) (views of one packed array, made on access)
+    H: Sequence                # P arrays (k_p, m) float32 (mu) / float64 (cd)
     n_iter: np.ndarray         # (P,)
     err: np.ndarray            # (P,)  ||X - W H||_F
     vaf: np.ndarray            # (P, m + 1): overall, then per column
@@ -134,18 +144,24 @@ def _pinned_give(buf):
         free.append(buf)
 
 
+_NEGATIVE_X = "Negative values in data passed to NMF (input X)"
+_NNDSVD_DEGENERATE = ("NNDSVD initialisation divides by zero for this X: a singular value it needs is zero, or the "
+                      "chosen part of a singular vector pair is empty")
+
+
 class PendingNMF:
     """A batch whose kernel is queued and whose results are on their way to pinned host memory: `result()` waits
     for the copies and builds the NMFBatchResult.  Lets a caller queue the next trial's GPU work before it
     looks at this one's (pipeline.synergies_for_files)."""
 
-    def __init__(self, torch, stream, ranks, seeds, n, m, device_arrays, keep, negative=None):
+    def __init__(self, torch, stream, ranks, seeds, n, m, device_arrays, keep, negative=None, degenerate=None):
         self._ranks, self._seeds, self._n, self._m = ranks, seeds, n, m
         self._keep = keep  # inputs of the kernel: alive until the copies below have run
         self._bufs = []
-        self._negative = negative is not None  # a device flag "X has a negative entry" travels with the results
-        if negative is not None:
-            device_arrays = list(device_arrays) + [negative.to(torch.uint8).reshape(1)]
+        # device flags travel with the results: "X has a negative entry", "the NNDSVD init divided by zero"
+        self._flags = [msg for msg, flag in ((_NEGATIVE_X, negative), (_NNDSVD_DEGENERATE, degenerate)) if flag is not None]
+        device_arrays = list(device_arrays) + [(flag != 0).to(torch.uint8).reshape(1)
+                                               for flag in (negative, degenerate) if flag is not None]
         for t in device_arrays:
             t = t.contiguous()
             buf = _pinned_take(torch, int(t.numel()) * t.element_size())
@@ -164,8 +180,10 @@ class PendingNMF:
                 out.append(buf.view(dtype).numpy().reshape(shape).copy())  # own memory: the pinned buffer goes back
                 _pinned_give(buf)
             self._bufs, self._keep = [], []
-            if self._negative and out.pop()[0]:
-                raise ValueError("Negative values in data passed to NMF (input X)")
+            raised = [msg for msg, flag in zip(self._flags, out[len(out) - len(self._flags):]) if flag[0]]
+            del out[len(out) - len(self._flags):]
+            if raised:
+                raise ValueError(raised[0])
             self._result = _assemble(self._ranks, self._seeds, self._n, self._m, *out)
         return self._result
 
@@ -234,7 +252,7 @@ def nmf_mu_batched(X, ranks: Sequence[int], seeds: Sequence[int], max_iter: int 
     # the previous trial's factorisation included): the flag travels with the results and `.result()` raises
     negative = (dX64 < 0).any() if on_device and defer else None
     if negative is None and (bool((dX64 < 0).any()) if on_device else bool((Xh < 0).any())):
-        raise ValueError("Negative values in data passed to NMF (input X)")
+        raise ValueError(_NEGATIVE_X)
     B, n, m = shape
     ranks = np.ascontiguousarray(ranks, dtype=np.int32)
     seeds = np.ascontiguousarray(seeds, dtype=np.int64)
@@ -303,6 +321,102 @@ def nmf_mu_batched(X, ranks: Sequence[int], seeds: Sequence[int], max_iter: int 
     return _assemble(ranks, seeds, n, m, Wall, Hall, n_iter, err, vafs)
 
 
+def nmf_cd_batched(X, ranks: Sequence[int], init="nndsvda", seeds: Optional[Sequence[int]] = None, max_iter: int = 200,
+                   tol: float = 1e-4, x_index: Optional[Sequence[int]] = None, regime: Optional[str] = None,
+                   defer: bool = False) -> Union[NMFBatchResult, PendingNMF]:
+    """Runs len(ranks) factorisations with scikit-learn's coordinate-descent solver (`NMF(solver="cd")`, shuffle=False,
+    no regularisation) in fp64, all in one launch.  X, ranks, x_index, regime and defer as for `nmf_mu_batched`.
+
+    init: "nndsvd" / "nndsvda" (computed on the device from an exact SVD, one per matrix of the stack; `seeds` is not
+    needed and sklearn's random_state has no counterpart), "random" (sklearn's draws for seeds[p]), or one explicit
+    (W, H) pair per problem.  The factors of the result are fp64; its seeds are -1 where no seed was given."""
+    import torch
+
+    lib = nat.lib()
+    if not torch.cuda.is_available():
+        raise nat.NativeError("nmf_cd_batched needs a CUDA device; there is no CPU fallback")
+    if isinstance(X, torch.Tensor) and X.is_cuda:
+        dev = X.device
+        dX = X.detach().to(torch.float64)
+    else:
+        dev = torch.device(f"cuda:{torch.cuda.current_device()}")
+        Xh = X.detach().to("cpu", torch.float64).numpy() if isinstance(X, torch.Tensor) else np.asarray(X, dtype=np.float64)
+        dX = torch.from_numpy(np.ascontiguousarray(Xh)).to(dev)
+    if dX.ndim == 2:
+        dX = dX[None]
+    if dX.ndim != 3 or 0 in dX.shape:
+        raise ValueError("X must be a non-empty (n, m) matrix or a (B, n, m) stack")
+    dX = dX.contiguous()
+    B, n, m = dX.shape
+    # as for nmf_mu_batched: a deferred run does not wait here, the flag travels with the results
+    negative = (dX < 0).any()
+    if not defer and bool(negative):
+        raise ValueError(_NEGATIVE_X)
+    ranks = np.ascontiguousarray(ranks, dtype=np.int32)
+    P = len(ranks)
+    xi = np.zeros(P, dtype=np.int32) if x_index is None else np.ascontiguousarray(x_index, dtype=np.int32)
+    seeds = np.full(P, -1, dtype=np.int64) if seeds is None else np.ascontiguousarray(seeds, dtype=np.int64)
+    if P < 1 or len(xi) != P or len(seeds) != P or xi.min() < 0 or xi.max() >= B:
+        raise ValueError("ranks, seeds and x_index must have one entry per problem")
+    if ranks.min() < 1:
+        raise ValueError("ranks must be positive")
+    named = isinstance(init, str)
+    if named and init not in ("nndsvd", "nndsvda", "random"):
+        raise ValueError(f"init must be 'nndsvd', 'nndsvda', 'random' or (W, H) pairs, not {init!r}")
+    if init == "random" and (seeds < 0).any():
+        raise ValueError("init='random' needs a non-negative seed per problem")
+    if named and init != "random" and int(ranks.max()) > min(n, m):
+        raise ValueError(f"init = '{init}' can only be used when n_components <= min(n_samples, n_features)")
+    table, kmax, d_ranks, d_xi, w_problem, h_problem = _batch_plan(torch, lib, n, m, ranks, xi, dev)
+    stream = torch.cuda.current_stream(dev)
+    keep, status = [dX], None
+    with torch.cuda.device(dev):
+        if init == "random":
+            unit_w, unit_h = _batch_draws(torch, n, m, ranks, seeds, dev)
+            avg = torch.sqrt(dX.mean(dim=(1, 2))[d_xi] / d_ranks)
+            dW, dH = unit_w * avg[w_problem], unit_h * avg[h_problem]
+        elif named:
+            dW = torch.empty(int(ranks.astype(np.int64).sum()) * n, dtype=torch.float64, device=dev)
+            dH = torch.empty(int(ranks.astype(np.int64).sum()) * m, dtype=torch.float64, device=dev)
+            work = torch.empty(int(lib.ms_nndsvd_workspace_bytes(m, B)), dtype=torch.uint8, device=dev)
+            status = torch.empty(1, dtype=torch.int32, device=dev)
+            nat.check(lib.ms_nndsvd_init(dX.data_ptr(), n, m, B, table.data_ptr(), P, kmax, int(init == "nndsvda"),
+                                         work.data_ptr(), dW.data_ptr(), dH.data_ptr(), status.data_ptr(),
+                                         ctypes.c_void_p(stream.cuda_stream)), "ms_nndsvd_init")
+            keep.append(work)
+        else:
+            if len(init) != P:
+                raise ValueError("init must give one (W, H) pair per problem")
+            for p, (W0, H0) in enumerate(init):
+                if np.shape(W0) != (n, ranks[p]) or np.shape(H0) != (ranks[p], m):
+                    raise ValueError(f"init pair {p} must have shapes {(n, int(ranks[p]))} and {(int(ranks[p]), m)}")
+            dW = torch.from_numpy(np.concatenate([np.asarray(w, dtype=np.float64).ravel() for w, _ in init])).to(dev)
+            dH = torch.from_numpy(np.concatenate([np.asarray(h, dtype=np.float64).ravel() for _, h in init])).to(dev)
+        d_iter = torch.empty(P, dtype=torch.int32, device=dev)
+        d_err = torch.empty(P, dtype=torch.float64, device=dev)
+        d_vaf = torch.empty((P, m + 1), dtype=torch.float64, device=dev)
+        resident = (n <= int(lib.ms_nmf_cd_resident_max_rows(m, kmax))) if regime is None else (regime == "resident")
+        if resident:
+            nat.check(lib.ms_nmf_cd_batched_planned(
+                dX.data_ptr(), n, m, table.data_ptr(), P, kmax, dW.data_ptr(), dH.data_ptr(), int(max_iter), float(tol),
+                d_iter.data_ptr(), d_err.data_ptr(), d_vaf.data_ptr(), ctypes.c_void_p(stream.cuda_stream)),
+                "ms_nmf_cd_batched_planned")
+        else:
+            work = torch.empty(int(lib.ms_nmf_cd_stream_workspace_bytes(m, P)), dtype=torch.uint8, device=dev)
+            keep.append(work)
+            nat.check(lib.ms_nmf_cd_stream(
+                dX.data_ptr(), n, m, table.data_ptr(), P, kmax, dW.data_ptr(), dH.data_ptr(), int(max_iter), float(tol),
+                work.data_ptr(), d_iter.data_ptr(), d_err.data_ptr(), d_vaf.data_ptr(), ctypes.c_void_p(stream.cuda_stream)),
+                "ms_nmf_cd_stream")
+        if defer:
+            return PendingNMF(torch, stream, ranks, seeds, n, m, [dW, dH, d_iter, d_err, d_vaf], keep, negative, status)
+        if status is not None and int(status.item()) != 0:
+            raise ValueError(_NNDSVD_DEGENERATE)
+        Wall, Hall = dW.cpu().numpy(), dH.cpu().numpy()
+        n_iter, err, vafs = d_iter.cpu().numpy(), d_err.cpu().numpy(), d_vaf.cpu().numpy()
+    return _assemble(ranks, seeds, n, m, Wall, Hall, n_iter, err, vafs)
+
+
 # ---- reference API ------------------------------------------------------------------------------------
 def vaf(original_df: pandas.DataFrame, transformed_signal=None, components=None, reconstructed_signal=None) -> pandas.DataFrame:
     """Variance accounted for, overall and per muscle (analysis.py:597-667)."""
@@ -329,7 +443,7 @@ class NMFModel:
     n_iter_: int
     reconstruction_err_: float
     n_features_in_: int
-    random_state: int
+    random_state: Optional[int]  # None: a deterministic init (nndsvd*)
     solver: str = "mu"
     beta_loss: str = "frobenius"
     init: str = "random"
@@ -367,6 +481,10 @@ def _find_synergies_sklearn(processed_emg_df, n_components, max_components, **sk
                             {k: r.transformed for k, r in runs.items()})
 
 
+# keywords of sklearn.decomposition.NMF that engine="gpu" accepts at scikit-learn's default value only
+_SKLEARN_DEFAULTS = {"alpha_W": 0.0, "alpha_H": "same", "l1_ratio": 0.0, "shuffle": False, "verbose": 0}
+
+
 def find_synergies(
     processed_emg_df: pandas.DataFrame,
     n_components: int,
@@ -375,14 +493,20 @@ def find_synergies(
     max_iter: int = 100_000,
     tol: float = 1e-6,
     n_restarts: int = 1,
+    engine: str = "auto",
     **sklearn_kwargs,
 ) -> SynergyRunResult:
     """Find muscle synergies with NMF (analysis.py:713-914) - all ranks and restarts in one launch.
 
-    solver="mu", init="random", beta_loss="frobenius" (or 2), random_state=int run on the GPU, all ranks and
-    restarts in one launch; `n_restarts` (extension) runs seeds random_state .. random_state+R-1 per rank and keeps,
+    engine="auto": solver="mu", init="random", beta_loss="frobenius" (or 2), random_state=int run on the GPU, all ranks
+    and restarts in one launch; `n_restarts` (extension) runs seeds random_state .. random_state+R-1 per rank and keeps,
     per rank, the restart with the smallest reconstruction error.  Any other scikit-learn configuration (the
-    default solver="cd", nndsvd inits, regularisation ...) is forwarded to scikit-learn as the reference does."""
+    default solver="cd", nndsvd inits, regularisation ...) is forwarded to scikit-learn as the reference does.
+    engine="sklearn" always forwards.  engine="gpu" runs on the GPU solver="cd" (the default; fp64, `nmf_cd_batched`)
+    or "mu", with init None (resolved as scikit-learn does: "nndsvda" if k <= min(n_samples, n_features), else
+    "random"), "nndsvd", "nndsvda" or "random", and raises NotImplementedError for any other keyword or value."""
+    if engine not in ("auto", "sklearn", "gpu"):
+        raise ValueError(f"engine must be 'auto', 'sklearn' or 'gpu', not {engine!r}")
     if processed_emg_df.empty:
         raise ValueError("empty EMG DataFrame")
     num_features = len(processed_emg_df.columns)
@@ -390,16 +514,19 @@ def find_synergies(
         raise ValueError("invalid number of components")
     if max_components is not None and (max_components < n_components or max_components > num_features):
         raise ValueError("invalid number of components")
+    if engine == "gpu":
+        return _find_synergies_gpu(processed_emg_df, n_components, max_components, max_iter, tol, n_restarts,
+                                   sklearn_kwargs)
     kw = dict(sklearn_kwargs)
     solver = kw.pop("solver", "cd")
     init = kw.pop("init", None)
     beta_loss = kw.pop("beta_loss", "frobenius")
     seed = kw.pop("random_state", None)
-    if solver != "mu" or init != "random" or beta_loss not in ("frobenius", 2, 2.0) or kw:
+    if engine == "sklearn" or solver != "mu" or init != "random" or beta_loss not in ("frobenius", 2, 2.0) or kw:
         # Everything the batched kernels do not implement is what the reference itself does with it: the keywords go
         # to scikit-learn unchanged (analysis.py:848-864) - solver="cd" with an nndsvd* init is the tutorial's own call
         # (docs/source/tutorials/Finding muscle synergies.ipynb, cell 26).  This is the reference's code path, not a
-        # fallback of the accelerated one: solver="mu", init="random" never comes here.
+        # fallback of the accelerated one: solver="mu", init="random" never comes here (unless engine="sklearn").
         if n_restarts != 1:
             raise ValueError("n_restarts is an extension of the batched mu solver; scikit-learn runs one initialisation")
         return _find_synergies_sklearn(processed_emg_df, n_components, max_components, max_iter=max_iter, tol=tol,
@@ -411,25 +538,34 @@ def find_synergies(
     seeds = [int(seed) + r for _ in ranks_sweep for r in range(n_restarts)]
     X = processed_emg_df.to_numpy(dtype=np.float64)
     res = nmf_mu_batched(X, ranks, seeds, max_iter=max_iter, tol=tol)
+    return _synergy_result(processed_emg_df, max_components, ranks_sweep, n_restarts, {k: (res, i * n_restarts)
+                           for i, k in enumerate(ranks_sweep)}, "mu", {k: "random" for k in ranks_sweep})
 
+
+def _synergy_result(processed_emg_df, max_components, ranks_sweep, n_restarts, batches, solver, inits):
+    """The SynergyRunResult of a sweep whose rank k has n_restarts consecutive problems in batch batches[k][0],
+    starting at problem batches[k][1]: per rank, the restart with the smallest reconstruction error."""
+    num_features = len(processed_emg_df.columns)
     columns = processed_emg_df.columns
     labels = ["All signals"] + columns.tolist()
     per_rank = OrderedDict()
-    for i, k in enumerate(ranks_sweep):
-        sl = slice(i * n_restarts, (i + 1) * n_restarts)
-        best = i * n_restarts + int(np.argmin(res.err[sl]))
+    for k in ranks_sweep:
+        res, first = batches[k]
+        sl = slice(first, first + n_restarts)
+        best = first + int(np.argmin(res.err[sl]))
         table = pandas.DataFrame(res.vaf[sl].astype(np.float64), columns=labels)
         table.insert(0, "reconstruction_err", res.err[sl].astype(np.float64))
         table.insert(0, "n_iter", res.n_iter[sl])
         table.insert(0, "random_state", res.seeds[sl])
+        seed = int(res.seeds[best])
         model = NMFModel(k, res.H[best].astype(np.float64), int(res.n_iter[best]), float(res.err[best]),
-                         num_features, int(res.seeds[best]), restarts=table)
+                         num_features, seed if seed >= 0 else None, solver=solver, init=inits[k], restarts=table)
         transformed = res.W[best].astype(np.float64)
         comps = pandas.DataFrame(model.components_, columns=columns)
         vaf_values = vaf(processed_emg_df, components=model.components_, transformed_signal=transformed)
         per_rank[k] = SynergyRunResult(vaf_values, comps, model, transformed)
     if max_components is None:
-        return per_rank[n_components]
+        return per_rank[ranks_sweep[0]]
     vaf_values = pandas.concat([r.vaf_values for r in per_rank.values()])
     vaf_values.set_index(np.array(tuple(per_rank.keys())), inplace=True)
     return SynergyRunResult(
@@ -438,3 +574,53 @@ def find_synergies(
         {k: r.model for k, r in per_rank.items()},
         {k: r.transformed for k, r in per_rank.items()},
     )
+
+
+def _find_synergies_gpu(df, n_components, max_components, max_iter, tol, n_restarts, sklearn_kwargs):
+    """find_synergies(engine="gpu"): the configurations the kernels implement, every other one refused by name."""
+    kw = dict(sklearn_kwargs)
+    solver = kw.pop("solver", "cd")
+    init = kw.pop("init", None)
+    beta_loss = kw.pop("beta_loss", "frobenius")
+    seed = kw.pop("random_state", None)
+    for name, default in _SKLEARN_DEFAULTS.items():
+        if name in kw and kw[name] == default and type(kw[name]) is type(default):
+            del kw[name]
+    if kw:
+        raise NotImplementedError(f"find_synergies(engine='gpu') does not implement {', '.join(f'{k}={v!r}' for k, v in kw.items())}")
+    if solver not in ("cd", "mu"):
+        raise NotImplementedError(f"find_synergies(engine='gpu') does not implement solver={solver!r}")
+    if init not in (None, "nndsvd", "nndsvda", "random"):
+        raise NotImplementedError(f"find_synergies(engine='gpu') does not implement init={init!r}")
+    if beta_loss not in ("frobenius", 2, 2.0):
+        raise NotImplementedError(f"find_synergies(engine='gpu') does not implement beta_loss={beta_loss!r}")
+    n, m = df.shape
+    ranks_sweep = [n_components] if max_components is None else list(range(n_components, max_components + 1))
+    inits = {k: init if init is not None else ("nndsvda" if k <= min(n, m) else "random") for k in ranks_sweep}
+    if n_restarts < 1:
+        raise ValueError("n_restarts must be positive")
+    if n_restarts > 1 and any(v != "random" for v in inits.values()):
+        raise ValueError("n_restarts > 1 needs init='random': an nndsvd init is deterministic")
+    if any(v == "random" for v in inits.values()) and seed is None:
+        seed = int(np.random.randint(0, 2**31 - 1))
+    X = df.to_numpy(dtype=np.float64)
+    batches = {}
+    for how in sorted(set(inits.values())):  # one launch per init kind (a sweep mixes them only when n < k)
+        group = [k for k in ranks_sweep if inits[k] == how]
+        ranks = [k for k in group for _ in range(n_restarts)]
+        seeds = [int(seed) + r for _ in group for r in range(n_restarts)] if how == "random" else None
+        if solver == "cd":
+            res = nmf_cd_batched(X, ranks, init=how, seeds=seeds, max_iter=max_iter, tol=tol)
+        elif how == "random":
+            res = nmf_mu_batched(X, ranks, seeds, max_iter=max_iter, tol=tol)
+        else:  # mu from the device's NNDSVD init
+            start = nmf_cd_batched(X, ranks, init=how, max_iter=0, tol=0.0)
+            res = nmf_mu_batched(X, ranks, np.full(len(ranks), -1), max_iter=max_iter, tol=tol,
+                                 init=[(start.W[p], start.H[p]) for p in range(len(ranks))])
+        if tol > 0 and (res.n_iter == max_iter).any():
+            from sklearn.exceptions import ConvergenceWarning
+
+            warnings.warn("Maximum number of iterations %d reached. Increase it to improve convergence." % max_iter,
+                          ConvergenceWarning)
+        batches.update({k: (res, i * n_restarts) for i, k in enumerate(group)})
+    return _synergy_result(df, max_components, ranks_sweep, n_restarts, batches, solver, inits)

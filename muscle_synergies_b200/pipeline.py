@@ -22,7 +22,7 @@ from typing import Dict, Iterable, List, Optional, Sequence, Tuple, Union
 import numpy as np
 import pandas
 
-from .analysis import NMFBatchResult, nmf_mu_batched
+from .analysis import NMFBatchResult, nmf_cd_batched, nmf_mu_batched
 from .emg import envelope_windows
 from .segment import Cycle, Segmenter, Trecho
 from .vicon_data import ViconLoader, ViconNexusData
@@ -113,23 +113,45 @@ class PendingTrial:
         return self._done
 
 
-def trial_synergies(data: ViconNexusData, min_components: int = 1, max_components: int = 8, n_restarts: int = 20,
-                    random_state: int = 0, max_iter: int = 200, tol: float = 1e-4, window_size: float = 0.5,
-                    reduce_to: int = 200, segmenter: Optional[Segmenter] = None, keep_batch: bool = False,
-                    seeds: Optional[Sequence[int]] = None, defer: bool = False) -> Union[TrialSynergies, PendingTrial]:
+def _deterministic(solver: str, init: Optional[str]) -> bool:
+    """True when trial_synergies(solver, init) starts from the deterministic NNDSVD init (one run per problem)."""
+    if solver == "mu":
+        if init not in (None, "random"):
+            raise ValueError(f"solver='mu' runs from init='random', not {init!r}")
+        return False
+    if solver != "cd":
+        raise ValueError(f"solver must be 'mu' or 'cd', not {solver!r}")
+    if init not in (None, "nndsvd", "nndsvda", "random"):
+        raise ValueError(f"solver='cd' runs from init 'nndsvd', 'nndsvda' or 'random', not {init!r}")
+    return init != "random"
+
+
+def trial_synergies(data: ViconNexusData, min_components: int = 1, max_components: int = 8,
+                    n_restarts: Optional[int] = None, random_state: int = 0, max_iter: int = 200, tol: float = 1e-4,
+                    window_size: float = 0.5, reduce_to: int = 200, segmenter: Optional[Segmenter] = None,
+                    keep_batch: bool = False, seeds: Optional[Sequence[int]] = None, defer: bool = False,
+                    solver: str = "mu", init: Optional[str] = None) -> Union[TrialSynergies, PendingTrial]:
     """Segments a loaded trial and factorises the EMG envelope of each of its 8 gait cycles for
     every rank in [min_components, max_components] from `n_restarts` random initialisations
-    (seeds random_state .. random_state + n_restarts - 1, sklearn `init="random"` draws; `seeds` names
+    (default 20; seeds random_state .. random_state + n_restarts - 1, sklearn `init="random"` draws; `seeds` names
     them explicitly instead - the share of one GPU when the restarts of a trial are split over several).
+    solver="mu" (fp32 multiplicative updates, `nmf_mu_batched`) or "cd" (sklearn's default coordinate descent, fp64,
+    `nmf_cd_batched`); under "cd", init defaults to "nndsvda", and a deterministic init ("nndsvd", "nndsvda") runs
+    one problem per cycle and rank: it takes exactly one seed (n_restarts 1, the default there), which only labels it.
     defer=True queues the GPU work and returns a PendingTrial: the caller can queue the next trial before it
     asks this one to `finish()` (the host-side tables of one trial are then built while the GPU factorises the next)."""
     muscles = data.emg.columns
     if not 1 <= min_components <= max_components <= len(muscles):
         raise ValueError("invalid number of components")
+    deterministic = _deterministic(solver, init)
+    if n_restarts is None:
+        n_restarts = 1 if deterministic else 20
     seed_list = np.arange(random_state, random_state + n_restarts, dtype=np.int64) if seeds is None else np.asarray(list(seeds), dtype=np.int64)
     n_restarts = int(seed_list.shape[0])
     if n_restarts < 1:
         raise ValueError("n_restarts must be positive")
+    if deterministic and n_restarts != 1:
+        raise ValueError("a deterministic init (nndsvd, nndsvda) takes exactly one seed")
     seg = segmenter if segmenter is not None else Segmenter(data)
     wins = cycle_windows(seg)
     env = envelope_windows(data.emg, [w for (_, _, w) in wins], window_size=window_size, reduce_to=reduce_to)
@@ -139,7 +161,11 @@ def trial_synergies(data: ViconNexusData, min_components: int = 1, max_component
     ranks = np.tile(np.repeat(np.array(sweep, dtype=np.int32), n_restarts), n_cyc)
     seeds = np.tile(seed_list, n_cyc * n_k)
     x_index = np.repeat(np.arange(n_cyc, dtype=np.int32), n_k * n_restarts)
-    pending = nmf_mu_batched(env, ranks, seeds, max_iter=max_iter, tol=tol, x_index=x_index, defer=True)
+    if solver == "cd":
+        pending = nmf_cd_batched(env, ranks, init=init or "nndsvda", seeds=seeds, max_iter=max_iter, tol=tol,
+                                 x_index=x_index, defer=True)
+    else:
+        pending = nmf_mu_batched(env, ranks, seeds, max_iter=max_iter, tol=tol, x_index=x_index, defer=True)
 
     def finish() -> TrialSynergies:
         return _trial_tables(pending.result(), data, wins, sweep, n_restarts, ranks, seeds, muscles, env, keep_batch)
@@ -278,6 +304,10 @@ def synergies_for_files_sharded(paths: Sequence[str], rank: Optional[int] = None
             rank, world = 0, 1
     paths = [str(p) for p in paths]
     analyse = analyse if analyse is not None else synergies_for_files
+    if _deterministic(kwargs.get("solver", "mu"), kwargs.get("init")):
+        # one run per (cycle, rank) and no restarts to split: by file, and with fewer files than GPUs the ranks that
+        # get no seed below have nothing to do
+        n_restarts = 1
     if len(paths) >= world:
         sizes = [os.path.getsize(p) if os.path.exists(p) else 0 for p in paths]
         mine = shard(paths, rank, world, sizes)
