@@ -335,6 +335,24 @@ int64_t ms_nndsvd_workspace_bytes(int32_t m, int32_t n_matrices);
 int ms_nndsvd_init(const double* d_X, int64_t n, int32_t m, int32_t n_matrices, const void* d_table, int32_t n_problems,
                    int32_t kmax, int32_t variant, void* d_work, double* d_W, double* d_H, int32_t* d_status, void* stream);
 
+/* NMF with fixed synergies, what sklearn's NMF.transform does (update_H=False), for a batch of problems in fp64:
+ * problem p fits W_p >= 0 to the matrix x_off of its ms_nmf_plan table entry with H_p (d_H, packed, k_p x m) held fixed.
+ * solver 0 = "cd" (coordinate descent; d_W must hold zeros), 1 = "mu" (multiplicative updates, beta 2; d_W must hold
+ * sqrt(mean(X) / k_p)); d_W receives the result.  X element (i, j) of a matrix is at d_X[x_off + i * row_stride +
+ * j * col_stride]: a row-major [n][m] matrix (m, 1) and a channel-major [m][n] one (1, n) are read in place.  Outputs
+ * per problem as for ms_nmf_cd_batched_planned: d_n_iter, d_err = ||X - W H||_F, d_vaf [m + 1].
+ * regime 0 (n <= ms_nmf_fixed_h_resident_max_rows(m, kmax)): one CTA per problem, all of it in shared memory, d_work
+ * unused.  regime 1 (any n): X is read once to form X H^T, then rows iterate in registers in chunks; synchronises
+ * `stream` every 64 iterations to stop once every problem has stopped.  d_work: ms_nmf_fixed_h_workspace_bytes(n, m,
+ * n_problems, kmax), 256-byte aligned.  Ranks 1..16, m <= 64; reductions have a fixed order (results are reproducible
+ * bit for bit), and at tol = 0 both regimes give the same W bit for bit. */
+int32_t ms_nmf_fixed_h_resident_max_rows(int32_t m, int32_t kmax);
+int64_t ms_nmf_fixed_h_workspace_bytes(int64_t n, int32_t m, int32_t n_problems, int32_t kmax);
+int ms_nmf_fixed_h(const double* d_X, int64_t n, int32_t m, int64_t row_stride, int64_t col_stride, const void* d_table,
+                   int32_t n_problems, int32_t kmax, double* d_W, const double* d_H, int32_t solver, int32_t max_iter,
+                   double tol, int32_t regime, void* d_work, int32_t* d_n_iter, double* d_err, double* d_vaf,
+                   void* stream);
+
 /* ---- misc ------------------------------------------------------------------------------- */
 /* The used part of a channel-major block (rows channels of width_bytes each, src_pitch_bytes apart) to host
  * memory as one 2-D copy on the DMA engine; asynchronous when h_dst is page-locked. */

@@ -11,7 +11,7 @@ there is no CPU fallback.
 """
 __version__ = "0.1.0"
 
-from .analysis import SynergyRunResult, find_synergies, nmf_cd_batched, nmf_mu_batched, vaf  # noqa: F401
+from .analysis import SynergyRunResult, find_synergies, nmf_cd_batched, nmf_mu_batched, nmf_transform_batched, vaf  # noqa: F401
 from .cache import load_trial, load_vicon_file_cached, save_trial  # noqa: F401
 from .emg import (  # noqa: F401
     digital_filter,
@@ -22,7 +22,7 @@ from .emg import (  # noqa: F401
     time_normalize,
     zero_center,
 )
-from .pipeline import synergies_for_files, synergies_for_files_sharded, trial_synergies  # noqa: F401
+from .pipeline import cross_cycle_vaf, synergies_for_files, synergies_for_files_sharded, trial_synergies  # noqa: F401
 from .vicon_data import (  # noqa: F401
     DeviceData,
     DeviceType,
@@ -51,11 +51,13 @@ __all__ = (
     # extensions
     "nmf_cd_batched",
     "nmf_mu_batched",
+    "nmf_transform_batched",
     "envelope_windows",
     "save_trial",
     "load_trial",
     "load_vicon_file_cached",
     "trial_synergies",
+    "cross_cycle_vaf",
     "synergies_for_files",
     "synergies_for_files_sharded",
 )

@@ -19,6 +19,12 @@ convergence with the reference's defaults (tol=1e-6, max_iter=100 000) from the 
 1e-8 and n_iter to max(3, 0.5 %).  Deviation: the device's NNDSVD uses an exact SVD where sklearn uses a randomized
 one, so sklearn's random_state has no effect on it; the two inits agree to ~1e-13 relative where sklearn's randomized
 SVD is itself accurate (tests/test_nmf_cd_gpu.py).
+
+`NMFModel.transform` and `nmf_transform_batched` fit activations to fixed synergies - sklearn's `NMF.transform`, for
+solver "cd" and "mu" - on the GPU in fp64 (csrc/ms_nmf_fixed.cu).  Parity claim, against sklearn's transform of the same
+X with the same components_ in fp64: at the same iteration count (tol=0), W H and VAF agree to 1e-9; run to convergence
+(tol=1e-6, max_iter=100 000), VAF agrees to 1e-8 and n_iter to max(3, 0.5 %) for "cd" and to one check (10) for "mu"
+(tests/test_nmf_transform_gpu.py).  The result is fp64 whatever X's dtype; sklearn's is in X's dtype, fp64 for a DataFrame.
 """
 import ctypes
 import functools
@@ -154,14 +160,17 @@ class PendingNMF:
     for the copies and builds the NMFBatchResult.  Lets a caller queue the next trial's GPU work before it
     looks at this one's (pipeline.synergies_for_files)."""
 
-    def __init__(self, torch, stream, ranks, seeds, n, m, device_arrays, keep, negative=None, degenerate=None):
+    def __init__(self, torch, stream, ranks, seeds, n, m, device_arrays, keep, negative=None, degenerate=None,
+                 checks=()):
         self._ranks, self._seeds, self._n, self._m = ranks, seeds, n, m
         self._keep = keep  # inputs of the kernel: alive until the copies below have run
         self._bufs = []
-        # device flags travel with the results: "X has a negative entry", "the NNDSVD init divided by zero"
-        self._flags = [msg for msg, flag in ((_NEGATIVE_X, negative), (_NNDSVD_DEGENERATE, degenerate)) if flag is not None]
+        # device flags travel with the results: "X has a negative entry", "the NNDSVD init divided by zero", and any
+        # other (message, flag) of `checks`; the first one set is raised
+        pairs = [(_NEGATIVE_X, negative), (_NNDSVD_DEGENERATE, degenerate)] + list(checks)
+        self._flags = [msg for msg, flag in pairs if flag is not None]
         device_arrays = list(device_arrays) + [(flag != 0).to(torch.uint8).reshape(1)
-                                               for flag in (negative, degenerate) if flag is not None]
+                                               for _, flag in pairs if flag is not None]
         for t in device_arrays:
             t = t.contiguous()
             buf = _pinned_take(torch, int(t.numel()) * t.element_size())
@@ -417,6 +426,138 @@ def nmf_cd_batched(X, ranks: Sequence[int], init="nndsvda", seeds: Optional[Sequ
     return _assemble(ranks, seeds, n, m, Wall, Hall, n_iter, err, vafs)
 
 
+# sklearn's texts for the input checks of NMF.transform (sklearn.utils.validation)
+_TRANSFORM_NAN = "Input X contains NaN."
+_TRANSFORM_INF = "Input X contains infinity or a value too large for dtype('float64')."
+_TRANSFORM_NEGATIVE = "Negative values in data passed to X in NMF."
+_SOLVER_CODES = {"cd": 0, "mu": 1}
+
+
+def _check_transform_host(Xh: np.ndarray):
+    """The input checks of sklearn's transform, in its order: NaN, infinity, negative values."""
+    if not np.isfinite(Xh).all():
+        raise ValueError(_TRANSFORM_NAN if np.isnan(Xh).any() else _TRANSFORM_INF)
+    if (Xh < 0).any():
+        raise ValueError(_TRANSFORM_NEGATIVE)
+
+
+def _transform_args(X, H, x_index, solver, max_iter, tol, regime):
+    """Validates what nmf_transform_batched is given, without touching a device; returns (H list, m, x_index)."""
+    if solver not in _SOLVER_CODES:
+        raise ValueError(f"solver must be 'cd' or 'mu', not {solver!r}")
+    if regime not in (None, "resident", "stream"):
+        raise ValueError(f"regime must be None, 'resident' or 'stream', not {regime!r}")
+    if int(max_iter) < 0 or not float(tol) >= 0:
+        raise ValueError("max_iter and tol must be non-negative")
+    Hs = [np.ascontiguousarray(h, dtype=np.float64) for h in H]
+    if not Hs:
+        raise ValueError("H must give one (k, m) matrix per problem")
+    m = Hs[0].shape[-1] if Hs[0].ndim == 2 else -1
+    for p, h in enumerate(Hs):
+        if h.ndim != 2 or h.shape[1] != m or not 1 <= h.shape[0] <= 16 or m > 64:
+            raise ValueError(f"H[{p}] must be a (k, m) matrix with 1 <= k <= 16 and m <= 64 columns shared by every "
+                             f"problem, not {h.shape}")
+        if not np.isfinite(h).all() or (h < 0).any():
+            raise ValueError(f"H[{p}] must be finite and non-negative")
+    xi = np.zeros(len(Hs), dtype=np.int32) if x_index is None else np.ascontiguousarray(x_index, dtype=np.int32)
+    if xi.shape != (len(Hs),) or xi.min() < 0:
+        raise ValueError("x_index must have one non-negative entry per matrix of H")
+    shape = tuple(X.shape)
+    if len(shape) not in (2, 3) or 0 in shape:
+        raise ValueError("X must be a non-empty (n, m) matrix or a (B, n, m) stack")
+    if shape[-1] != m:
+        raise ValueError(f"X has {shape[-1]} features, but H has {m}")
+    if xi.max() >= (shape[0] if len(shape) == 3 else 1):
+        raise ValueError("x_index names a matrix X does not have")
+    return Hs, m, xi
+
+
+def nmf_transform_batched(X, H: Sequence, x_index: Optional[Sequence[int]] = None, solver: str = "cd",
+                          max_iter: int = 200, tol: float = 1e-4, regime: Optional[str] = None,
+                          defer: bool = False) -> Union[NMFBatchResult, PendingNMF]:
+    """Fits activations to fixed synergies - scikit-learn's `NMF.transform` (update_H=False, no regularisation) - for a
+    batch of problems in one launch, in fp64: problem p fits W_p >= 0 to X[x_index[p]] with H[p] (k_p x m) fixed.
+
+    solver "cd" starts from W = 0, "mu" from sqrt(X.mean() / k_p), as sklearn does; max_iter and tol are sklearn's.
+    X: a non-negative (n, m) matrix or a (B, n, m) stack, as a numpy array or a CUDA tensor (which never leaves the
+    device; a strided view such as the (samples, channels) `env.T` of a channel-major envelope is read in place).
+    A negative or non-finite X raises ValueError (under defer, from `.result()`).  regime: None (by size),
+    "resident" or "stream".  Returns an NMFBatchResult whose H are the given matrices and whose seeds are -1, or a
+    PendingNMF when defer=True."""
+    return _nmf_transform(X, H, x_index, solver, max_iter, tol, regime, defer)
+
+
+def _nmf_transform(X, H, x_index, solver, max_iter, tol, regime, defer, device_w=False):
+    import torch
+
+    on_device = isinstance(X, torch.Tensor) and X.is_cuda
+    if not on_device:
+        Xh = X.detach().to("cpu", torch.float64).numpy() if isinstance(X, torch.Tensor) else np.asarray(X, dtype=np.float64)
+        X = Xh
+    Hs, m, xi = _transform_args(X, H, x_index, solver, max_iter, tol, regime)
+    if not on_device:
+        _check_transform_host(X)
+    lib = nat.lib()
+    if not torch.cuda.is_available():
+        raise nat.NativeError("nmf_transform_batched needs a CUDA device; there is no CPU fallback")
+    ranks = np.array([h.shape[0] for h in Hs], dtype=np.int32)
+    P = len(ranks)
+    seeds = np.full(P, -1, dtype=np.int64)
+    checks = ()
+    if on_device:
+        dev = X.device
+        dX = X.detach().to(torch.float64)
+        if dX.ndim == 2:
+            dX = dX[None]
+        B, n, _ = dX.shape
+        if B > 1 and dX.stride(0) != n * m:  # the problem table addresses matrix b at b * n * m
+            dX = dX.contiguous()
+        flags = (torch.isnan(dX).any(), torch.isinf(dX).any(), (dX < 0).any())
+        checks = tuple(zip((_TRANSFORM_NAN, _TRANSFORM_INF, _TRANSFORM_NEGATIVE), flags))
+        if not defer:
+            for msg, flag in checks:
+                if bool(flag):
+                    raise ValueError(msg)
+            checks = ()
+    else:
+        dev = torch.device(f"cuda:{torch.cuda.current_device()}")
+        Xh = X[None] if X.ndim == 2 else X
+        B, n, _ = Xh.shape
+        means = np.array([Xh[b].mean() for b in range(B)])  # sklearn's X.mean(), on the host as sklearn computes it
+        dX = torch.from_numpy(np.ascontiguousarray(Xh)).to(dev)
+    kmax = int(ranks.max())
+    resident = (n <= int(lib.ms_nmf_fixed_h_resident_max_rows(m, kmax))) if regime is None else (regime == "resident")
+    table, kmax, d_ranks, d_xi, w_problem, _ = _batch_plan(torch, lib, n, m, ranks, xi, dev)
+    stream = torch.cuda.current_stream(dev)
+    keep = [dX]
+    with torch.cuda.device(dev):
+        if solver == "cd":
+            dW = torch.zeros(int(ranks.astype(np.int64).sum()) * n, dtype=torch.float64, device=dev)
+        elif on_device:
+            # the mean of the row-major copy: the same W0, bit for bit, whatever the layout X comes in
+            dW = torch.sqrt(dX.contiguous().mean(dim=(1, 2))[d_xi] / d_ranks)[w_problem]
+        else:
+            dW = torch.from_numpy(np.sqrt(means[xi] / ranks)).to(dev)[w_problem]
+        dH = torch.from_numpy(np.concatenate([h.ravel() for h in Hs])).to(dev)
+        d_iter = torch.empty(P, dtype=torch.int32, device=dev)
+        d_err = torch.empty(P, dtype=torch.float64, device=dev)
+        d_vaf = torch.empty((P, m + 1), dtype=torch.float64, device=dev)
+        work = torch.empty(0 if resident else int(lib.ms_nmf_fixed_h_workspace_bytes(n, m, P, kmax)), dtype=torch.uint8,
+                           device=dev)
+        keep.append(work)
+        nat.check(lib.ms_nmf_fixed_h(
+            dX.data_ptr(), n, m, dX.stride(1), dX.stride(2), table.data_ptr(), P, kmax, dW.data_ptr(), dH.data_ptr(),
+            _SOLVER_CODES[solver], int(max_iter), float(tol), 0 if resident else 1, work.data_ptr() if not resident else None,
+            d_iter.data_ptr(), d_err.data_ptr(), d_vaf.data_ptr(), ctypes.c_void_p(stream.cuda_stream)), "ms_nmf_fixed_h")
+        if device_w:
+            return dW, d_iter
+        if defer:
+            return PendingNMF(torch, stream, ranks, seeds, n, m, [dW, dH, d_iter, d_err, d_vaf], keep, checks=checks)
+        Wall = dW.cpu().numpy()
+        n_iter, err, vafs = d_iter.cpu().numpy(), d_err.cpu().numpy(), d_vaf.cpu().numpy()
+    return _assemble(ranks, seeds, n, m, Wall, np.concatenate([h.ravel() for h in Hs]), n_iter, err, vafs)
+
+
 # ---- reference API ------------------------------------------------------------------------------------
 def vaf(original_df: pandas.DataFrame, transformed_signal=None, components=None, reconstructed_signal=None) -> pandas.DataFrame:
     """Variance accounted for, overall and per muscle (analysis.py:597-667)."""
@@ -448,9 +589,48 @@ class NMFModel:
     beta_loss: str = "frobenius"
     init: str = "random"
     restarts: Optional[pandas.DataFrame] = None  # extension: one row per restart (seed, n_iter, err, VAF)
+    max_iter: int = 100_000
+    tol: float = 1e-6
 
-    def transform(self, X):  # pragma: no cover - kept for API familiarity
-        raise NotImplementedError("transform of new data is not part of the accelerated path")
+    def transform(self, X):
+        """sklearn's `NMF.transform`: the activations W >= 0 that fit X with these components fixed, by the model's
+        solver, max_iter and tol, on the GPU in fp64 (`nmf_transform_batched`).  X: a DataFrame, an ndarray or a CUDA
+        tensor (n, n_features_in_); returns an (n, n_components) ndarray, or a CUDA tensor for a CUDA input.  Raises
+        sklearn's ValueErrors for non-finite or negative X and a wrong feature count, and emits its ConvergenceWarning
+        when max_iter is reached with tol > 0."""
+        import torch
+
+        if isinstance(X, torch.Tensor) and X.is_cuda:
+            if X.ndim != 2:
+                raise ValueError(f"Expected 2D array, got {X.ndim}D array instead")
+            for msg, flag in zip((_TRANSFORM_NAN, _TRANSFORM_INF, _TRANSFORM_NEGATIVE),
+                                 (torch.isnan(X).any(), torch.isinf(X).any(), (X < 0).any())):
+                if bool(flag):
+                    raise ValueError(msg)
+        else:
+            X = np.asarray(X.to_numpy() if isinstance(X, pandas.DataFrame) else X, dtype=np.float64)
+            if X.ndim != 2:
+                raise ValueError(f"Expected 2D array, got {X.ndim}D array instead")
+            _check_transform_host(X)
+        if X.shape[1] != self.n_features_in_:
+            raise ValueError(f"X has {X.shape[1]} features, but NMF is expecting {self.n_features_in_} features as input.")
+        W, n_iter = _nmf_transform(X, [self.components_], None, self.solver, self.max_iter, self.tol, None, False,
+                                   device_w=True)
+        if self.tol > 0 and int(n_iter[0]) == self.max_iter:
+            from sklearn.exceptions import ConvergenceWarning
+
+            warnings.warn("Maximum number of iterations %d reached. Increase it to improve convergence." % self.max_iter,
+                          ConvergenceWarning)
+        W = W.reshape(X.shape[0], self.components_.shape[0])
+        return W if isinstance(X, torch.Tensor) else W.cpu().numpy()
+
+    def inverse_transform(self, W):
+        """sklearn's `NMF.inverse_transform`: W @ components_ (a CUDA tensor for a CUDA W)."""
+        import torch
+
+        if isinstance(W, torch.Tensor):
+            return W @ torch.as_tensor(self.components_, dtype=W.dtype, device=W.device)
+        return np.asarray(W) @ self.components_
 
 
 @dataclass
@@ -539,10 +719,10 @@ def find_synergies(
     X = processed_emg_df.to_numpy(dtype=np.float64)
     res = nmf_mu_batched(X, ranks, seeds, max_iter=max_iter, tol=tol)
     return _synergy_result(processed_emg_df, max_components, ranks_sweep, n_restarts, {k: (res, i * n_restarts)
-                           for i, k in enumerate(ranks_sweep)}, "mu", {k: "random" for k in ranks_sweep})
+                           for i, k in enumerate(ranks_sweep)}, "mu", {k: "random" for k in ranks_sweep}, max_iter, tol)
 
 
-def _synergy_result(processed_emg_df, max_components, ranks_sweep, n_restarts, batches, solver, inits):
+def _synergy_result(processed_emg_df, max_components, ranks_sweep, n_restarts, batches, solver, inits, max_iter, tol):
     """The SynergyRunResult of a sweep whose rank k has n_restarts consecutive problems in batch batches[k][0],
     starting at problem batches[k][1]: per rank, the restart with the smallest reconstruction error."""
     num_features = len(processed_emg_df.columns)
@@ -559,7 +739,8 @@ def _synergy_result(processed_emg_df, max_components, ranks_sweep, n_restarts, b
         table.insert(0, "random_state", res.seeds[sl])
         seed = int(res.seeds[best])
         model = NMFModel(k, res.H[best].astype(np.float64), int(res.n_iter[best]), float(res.err[best]),
-                         num_features, seed if seed >= 0 else None, solver=solver, init=inits[k], restarts=table)
+                         num_features, seed if seed >= 0 else None, solver=solver, init=inits[k], restarts=table,
+                         max_iter=max_iter, tol=tol)
         transformed = res.W[best].astype(np.float64)
         comps = pandas.DataFrame(model.components_, columns=columns)
         vaf_values = vaf(processed_emg_df, components=model.components_, transformed_signal=transformed)
@@ -623,4 +804,4 @@ def _find_synergies_gpu(df, n_components, max_components, max_iter, tol, n_resta
             warnings.warn("Maximum number of iterations %d reached. Increase it to improve convergence." % max_iter,
                           ConvergenceWarning)
         batches.update({k: (res, i * n_restarts) for i, k in enumerate(group)})
-    return _synergy_result(df, max_components, ranks_sweep, n_restarts, batches, solver, inits)
+    return _synergy_result(df, max_components, ranks_sweep, n_restarts, batches, solver, inits, max_iter, tol)

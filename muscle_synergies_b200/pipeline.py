@@ -22,7 +22,7 @@ from typing import Dict, Iterable, List, Optional, Sequence, Tuple, Union
 import numpy as np
 import pandas
 
-from .analysis import NMFBatchResult, nmf_cd_batched, nmf_mu_batched
+from .analysis import NMFBatchResult, nmf_cd_batched, nmf_mu_batched, nmf_transform_batched
 from .emg import envelope_windows
 from .segment import Cycle, Segmenter, Trecho
 from .vicon_data import ViconLoader, ViconNexusData
@@ -199,6 +199,24 @@ def _trial_tables(res, data, wins, sweep, n_restarts, ranks, seeds, muscles, env
         "All signals": res.vaf[:, 0].astype(np.float64),
     }
     return TrialSynergies(cycles, env, res if keep_batch else None, restart_columns)
+
+
+def cross_cycle_vaf(trial: TrialSynergies, ranks: Optional[Sequence[int]] = None, solver: str = "cd",
+                    max_iter: int = 100_000, tol: float = 1e-6) -> pandas.DataFrame:
+    """How well each cycle's synergies generalise to the other cycles of the trial: for every rank, every cycle's
+    envelope (`trial.envelopes`, on the device) is fitted with every cycle's synergies held fixed (sklearn's
+    `NMF.transform` with `solver`, `max_iter`, `tol`), all ranks x sources x targets in one launch.  Returns the overall
+    VAF; index (n_components, source trecho, source cycle), columns (target trecho, target cycle)."""
+    cycles = trial.cycles
+    ranks = list(cycles[0].components) if ranks is None else [int(k) for k in ranks]
+    n_cyc = len(cycles)
+    H = [cycles[s].components[k].to_numpy(dtype=np.float64) for k in ranks for s in range(n_cyc) for _ in range(n_cyc)]
+    x_index = np.tile(np.arange(n_cyc, dtype=np.int32), len(ranks) * n_cyc)
+    res = nmf_transform_batched(trial.envelopes, H, x_index=x_index, solver=solver, max_iter=max_iter, tol=tol)
+    index = pandas.MultiIndex.from_tuples([(k, c.trecho.value, c.cycle.value) for k in ranks for c in cycles],
+                                          names=["n_components", "trecho", "cycle"])
+    columns = pandas.MultiIndex.from_tuples([(c.trecho.value, c.cycle.value) for c in cycles], names=["trecho", "cycle"])
+    return pandas.DataFrame(res.vaf[:, 0].reshape(len(ranks) * n_cyc, n_cyc), index=index, columns=columns)
 
 
 def synergies_for_files(paths: Sequence[str], loader: Optional[ViconLoader] = None, **kwargs) -> Iterable[Tuple[str, TrialSynergies]]:
