@@ -353,6 +353,23 @@ int ms_nmf_fixed_h(const double* d_X, int64_t n, int32_t m, int64_t row_stride, 
                    double tol, int32_t regime, void* d_work, int32_t* d_n_iter, double* d_err, double* d_vaf,
                    void* stream);
 
+/* β-divergence NMF by multiplicative updates, fp64: scikit-learn's solver="mu" with beta_loss = beta != 2 (1: Kullback-
+ * Leibler, 0: Itakura-Saito, any other float), no regularisation.  update_H = 1: fit W (n x k_p) and H (k_p x m) from
+ * the given d_W / d_H (ms_nmf_plan's table, as for ms_nmf_cd_batched_planned); update_H = 0: sklearn's transform, H
+ * fixed, from the given W (sklearn starts it at sqrt(mean(X) / k_p)).  X as for ms_nmf_fixed_h (row_stride,
+ * col_stride).  Outputs per problem: d_n_iter, d_err = sqrt(2 D_beta(X | W H)) (sklearn's reconstruction_err_), d_vaf
+ * [m + 1] (Frobenius VAF, overall then per column).  regime 0 (n <= ms_nmf_beta_resident_max_rows(m, kmax)): one CTA
+ * per problem, d_work unused.  regime 1 (any n): one pass over X per iteration; synchronises `stream` every 64
+ * iterations when tol > 0 to stop once every problem has stopped.  d_work: ms_nmf_beta_workspace_bytes(n, m,
+ * n_problems, kmax), 256-byte aligned.  Ranks 1..16, m <= 64; beta = 2 is refused (MS_E_INVALID).  Reductions have a
+ * fixed order: results are reproducible bit for bit. */
+int32_t ms_nmf_beta_resident_max_rows(int32_t m, int32_t kmax);
+int64_t ms_nmf_beta_workspace_bytes(int64_t n, int32_t m, int32_t n_problems, int32_t kmax);
+int ms_nmf_beta(const double* d_X, int64_t n, int32_t m, int64_t row_stride, int64_t col_stride, const void* d_table,
+                int32_t n_problems, int32_t kmax, double* d_W, double* d_H, double beta, int32_t update_H,
+                int32_t max_iter, double tol, int32_t regime, void* d_work, int32_t* d_n_iter, double* d_err,
+                double* d_vaf, void* stream);
+
 /* ---- misc ------------------------------------------------------------------------------- */
 /* The used part of a channel-major block (rows channels of width_bytes each, src_pitch_bytes apart) to host
  * memory as one 2-D copy on the DMA engine; asynchronous when h_dst is page-locked. */

@@ -11,7 +11,8 @@ there is no CPU fallback.
 """
 __version__ = "0.1.0"
 
-from .analysis import SynergyRunResult, find_synergies, nmf_cd_batched, nmf_mu_batched, nmf_transform_batched, vaf  # noqa: F401
+from .analysis import (SynergyRunResult, find_synergies, nmf_beta_batched, nmf_cd_batched, nmf_mu_batched,  # noqa: F401
+                       nmf_transform_batched, vaf)
 from .cache import load_trial, load_vicon_file_cached, save_trial  # noqa: F401
 from .emg import (  # noqa: F401
     digital_filter,
@@ -49,6 +50,7 @@ __all__ = (
     "vaf",
     "find_synergies",
     # extensions
+    "nmf_beta_batched",
     "nmf_cd_batched",
     "nmf_mu_batched",
     "nmf_transform_batched",

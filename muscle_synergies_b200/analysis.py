@@ -25,6 +25,12 @@ solver "cd" and "mu" - on the GPU in fp64 (csrc/ms_nmf_fixed.cu).  Parity claim,
 X with the same components_ in fp64: at the same iteration count (tol=0), W H and VAF agree to 1e-9; run to convergence
 (tol=1e-6, max_iter=100 000), VAF agrees to 1e-8 and n_iter to max(3, 0.5 %) for "cd" and to one check (10) for "mu"
 (tests/test_nmf_transform_gpu.py).  The result is fp64 whatever X's dtype; sklearn's is in X's dtype, fp64 for a DataFrame.
+
+`nmf_beta_batched`, `find_synergies(engine="gpu", solver="mu", beta_loss=...)` and the transform of such a model run
+sklearn's multiplicative updates for the β-divergence (beta_loss "kullback-leibler" = 1, "itakura-saito" = 0, or any
+float other than 2) on the GPU in fp64 (csrc/ms_nmf_beta.cu).  Parity claim, against sklearn in fp64: from the same init
+at the same iteration count (tol=0), W H, VAF and err (sklearn's reconstruction_err_, the square-rooted divergence) agree
+to 1e-9; converged, VAF agrees to 1e-8 and n_iter to one check (10) (tests/test_nmf_beta_gpu.py).
 """
 import ctypes
 import functools
@@ -426,6 +432,178 @@ def nmf_cd_batched(X, ranks: Sequence[int], init="nndsvda", seeds: Optional[Sequ
     return _assemble(ranks, seeds, n, m, Wall, Hall, n_iter, err, vafs)
 
 
+_BETA_NAMES = {"frobenius": 2.0, "kullback-leibler": 1.0, "itakura-saito": 0.0}
+_BETA_ZEROS = ("When beta_loss <= 0 and X contains zeros, the solver may diverge. Please add small values to X, or use a "
+               "positive beta_loss.")
+
+
+def _beta_to_float(beta_loss) -> float:
+    """sklearn's _beta_loss_to_float, with its parameter check: a name of _BETA_NAMES or a finite real number."""
+    if isinstance(beta_loss, str):
+        if beta_loss not in _BETA_NAMES:
+            raise ValueError(f"beta_loss must be one of {sorted(_BETA_NAMES)} or a float, not {beta_loss!r}")
+        return _BETA_NAMES[beta_loss]
+    if isinstance(beta_loss, bool) or not isinstance(beta_loss, (int, float, np.integer, np.floating)) \
+            or not np.isfinite(beta_loss):
+        raise ValueError(f"beta_loss must be one of {sorted(_BETA_NAMES)} or a float, not {beta_loss!r}")
+    return float(beta_loss)
+
+
+class _BetaLossSolverError(ValueError, NotImplementedError):
+    """scikit-learn's ValueError for a solver other than "mu" with beta_loss != 2.  It is also the NotImplementedError
+    that find_synergies(engine="gpu") raised for beta_loss != 2 before the β kernels existed, so code that caught that
+    keeps working."""
+
+
+def _beta_solver_error(solver, beta_loss) -> ValueError:
+    return _BetaLossSolverError(f"Invalid beta_loss parameter: solver {solver!r} does not handle beta_loss = {beta_loss!r}")
+
+
+def nmf_beta_batched(X, ranks: Sequence[int], beta_loss, init="nndsvda", seeds: Optional[Sequence[int]] = None,
+                     max_iter: int = 200, tol: float = 1e-4, x_index: Optional[Sequence[int]] = None,
+                     regime: Optional[str] = None, defer: bool = False) -> Union[NMFBatchResult, PendingNMF]:
+    """Runs len(ranks) factorisations with scikit-learn's multiplicative updates for the β-divergence
+    (`NMF(solver="mu", beta_loss=beta_loss)`, no regularisation) in fp64, all in one launch.
+
+    beta_loss: "kullback-leibler" (1), "itakura-saito" (0) or any float other than 2 (Frobenius runs on
+    `nmf_mu_batched` / `nmf_cd_batched`).  X, ranks, init, seeds, x_index, regime and defer as for `nmf_cd_batched`; X
+    may also be a strided CUDA view (a channel-major `env.T`), read in place.  A negative X, and a zero in X with
+    beta_loss <= 0, raise sklearn's ValueError (under defer, from `.result()` for a CUDA X).  The result's err is
+    sklearn's reconstruction_err_, sqrt(2 D_beta(X | W H)); its VAF is the Frobenius one, as `vaf` computes it."""
+    import torch
+
+    beta = _beta_to_float(beta_loss)
+    if beta == 2.0:
+        raise ValueError("beta_loss = 2 (Frobenius) runs on nmf_mu_batched or nmf_cd_batched")
+    if regime not in (None, "resident", "stream"):
+        raise ValueError(f"regime must be None, 'resident' or 'stream', not {regime!r}")
+    if int(max_iter) < 0 or not float(tol) >= 0:
+        raise ValueError("max_iter and tol must be non-negative")
+    on_device = isinstance(X, torch.Tensor) and X.is_cuda
+    if not on_device:
+        Xh = X.detach().to("cpu", torch.float64).numpy() if isinstance(X, torch.Tensor) else np.asarray(X, dtype=np.float64)
+        Xh = Xh[None] if Xh.ndim == 2 else Xh
+        shape = Xh.shape
+    else:
+        shape = tuple(X.shape) if X.ndim == 3 else (1,) + tuple(X.shape)
+    if len(shape) != 3 or 0 in shape:
+        raise ValueError("X must be a non-empty (n, m) matrix or a (B, n, m) stack")
+    B, n, m = shape
+    ranks = np.ascontiguousarray(ranks, dtype=np.int32)
+    P = len(ranks)
+    xi = np.zeros(P, dtype=np.int32) if x_index is None else np.ascontiguousarray(x_index, dtype=np.int32)
+    seeds = np.full(P, -1, dtype=np.int64) if seeds is None else np.ascontiguousarray(seeds, dtype=np.int64)
+    if P < 1 or len(xi) != P or len(seeds) != P or xi.min() < 0 or xi.max() >= B:
+        raise ValueError("ranks, seeds and x_index must have one entry per problem")
+    if ranks.min() < 1 or ranks.max() > 16 or m > 64:
+        raise ValueError(f"ranks must be in 1..16 and X may have at most 64 columns (ranks {ranks.min()}..{ranks.max()}, "
+                         f"{m} columns)")
+    named = isinstance(init, str)
+    if named and init not in ("nndsvd", "nndsvda", "random"):
+        raise ValueError(f"init must be 'nndsvd', 'nndsvda', 'random' or (W, H) pairs, not {init!r}")
+    if init == "random" and (seeds < 0).any():
+        raise ValueError("init='random' needs a non-negative seed per problem")
+    if named and init != "random" and int(ranks.max()) > min(n, m):
+        raise ValueError(f"init = '{init}' can only be used when n_components <= min(n_samples, n_features)")
+    if not named:
+        if len(init) != P:
+            raise ValueError("init must give one (W, H) pair per problem")
+        for p, (W0, H0) in enumerate(init):
+            if np.shape(W0) != (n, ranks[p]) or np.shape(H0) != (ranks[p], m):
+                raise ValueError(f"init pair {p} must have shapes {(n, int(ranks[p]))} and {(int(ranks[p]), m)}")
+            for A, whom in ((H0, "NMF (input H)"), (W0, "NMF (input W)")):  # sklearn's _check_init, H first
+                A = np.asarray(A, dtype=np.float64)
+                if not np.isfinite(A).all():
+                    raise ValueError(f"Input contains NaN or infinity (init pair {p}, {whom})")
+                if (A < 0).any():
+                    raise ValueError(f"Negative values in data passed to {whom}")
+                if A.max() == 0:
+                    raise ValueError(f"Array passed to {whom} is full of zeros.")
+    if not on_device:  # sklearn's order: negative values first, then zeros under beta_loss <= 0
+        if (Xh < 0).any():
+            raise ValueError(_NEGATIVE_X)
+        if beta <= 0 and Xh.min() == 0:
+            raise ValueError(_BETA_ZEROS)
+    lib = nat.lib()
+    if not torch.cuda.is_available():
+        raise nat.NativeError("nmf_beta_batched needs a CUDA device; there is no CPU fallback")
+    negative, checks = None, ()
+    if on_device:
+        dev = X.device
+        dX = X.detach().to(torch.float64)
+        dX = dX[None] if dX.ndim == 2 else dX
+        if B > 1 and dX.stride(0) != n * m:  # the problem table addresses matrix b at b * n * m
+            dX = dX.contiguous()
+        # as for nmf_mu_batched: a deferred run does not wait here, the flags travel with the results
+        negative = (dX < 0).any()
+        zeros = (dX == 0).any() if beta <= 0 else None
+        if not defer:
+            if bool(negative):
+                raise ValueError(_NEGATIVE_X)
+            if zeros is not None and bool(zeros):
+                raise ValueError(_BETA_ZEROS)
+            negative = None
+        elif zeros is not None:
+            checks = ((_BETA_ZEROS, zeros),)
+    else:
+        dev = torch.device(f"cuda:{torch.cuda.current_device()}")
+        dX = torch.from_numpy(np.ascontiguousarray(Xh)).to(dev)
+    table, kmax, d_ranks, d_xi, w_problem, h_problem = _batch_plan(torch, lib, n, m, ranks, xi, dev)
+    stream = torch.cuda.current_stream(dev)
+    keep, status = [dX], None
+    with torch.cuda.device(dev):
+        if init == "random":
+            unit_w, unit_h = _batch_draws(torch, n, m, ranks, seeds, dev)
+            if on_device:
+                means = dX.contiguous().mean(dim=(1, 2))
+            else:  # sklearn's X.mean(), on the host as sklearn computes it: the same init, bit for bit
+                means = torch.from_numpy(np.array([Xh[b].mean() for b in range(B)])).to(dev)
+            avg = torch.sqrt(means[d_xi] / d_ranks)
+            dW, dH = unit_w * avg[w_problem], unit_h * avg[h_problem]
+        elif named:
+            dXc = dX.contiguous()  # the SVD reads row-major matrices
+            dW = torch.empty(int(ranks.astype(np.int64).sum()) * n, dtype=torch.float64, device=dev)
+            dH = torch.empty(int(ranks.astype(np.int64).sum()) * m, dtype=torch.float64, device=dev)
+            work = torch.empty(int(lib.ms_nndsvd_workspace_bytes(m, B)), dtype=torch.uint8, device=dev)
+            status = torch.empty(1, dtype=torch.int32, device=dev)
+            nat.check(lib.ms_nndsvd_init(dXc.data_ptr(), n, m, B, table.data_ptr(), P, kmax, int(init == "nndsvda"),
+                                         work.data_ptr(), dW.data_ptr(), dH.data_ptr(), status.data_ptr(),
+                                         ctypes.c_void_p(stream.cuda_stream)), "ms_nndsvd_init")
+            keep += [dXc, work]
+        else:
+            dW = torch.from_numpy(np.concatenate([np.asarray(w, dtype=np.float64).ravel() for w, _ in init])).to(dev)
+            dH = torch.from_numpy(np.concatenate([np.asarray(h, dtype=np.float64).ravel() for _, h in init])).to(dev)
+        d_iter, d_err, d_vaf, work = _beta_launch(torch, lib, dX, n, m, table, P, kmax, dW, dH, beta, 1, max_iter, tol,
+                                                  regime, stream)
+        keep.append(work)
+        if defer:
+            return PendingNMF(torch, stream, ranks, seeds, n, m, [dW, dH, d_iter, d_err, d_vaf], keep, negative, status,
+                              checks=checks)
+        if status is not None and int(status.item()) != 0:
+            raise ValueError(_NNDSVD_DEGENERATE)
+        Wall, Hall = dW.cpu().numpy(), dH.cpu().numpy()
+        n_iter, err, vafs = d_iter.cpu().numpy(), d_err.cpu().numpy(), d_vaf.cpu().numpy()
+    return _assemble(ranks, seeds, n, m, Wall, Hall, n_iter, err, vafs)
+
+
+def _beta_launch(torch, lib, dX, n, m, table, P, kmax, dW, dH, beta, update_H, max_iter, tol, regime, stream):
+    """Queues ms_nmf_beta on `stream` (regime None: resident when n fits shared memory); returns the device outputs
+    and the workspace, which must outlive the launch."""
+    dev = dX.device
+    resident = (n <= int(lib.ms_nmf_beta_resident_max_rows(m, kmax))) if regime is None else (regime == "resident")
+    d_iter = torch.empty(P, dtype=torch.int32, device=dev)
+    d_err = torch.empty(P, dtype=torch.float64, device=dev)
+    d_vaf = torch.empty((P, m + 1), dtype=torch.float64, device=dev)
+    work = torch.empty(0 if resident else int(lib.ms_nmf_beta_workspace_bytes(n, m, P, kmax)), dtype=torch.uint8,
+                       device=dev)
+    nat.check(lib.ms_nmf_beta(
+        dX.data_ptr(), n, m, dX.stride(1), dX.stride(2), table.data_ptr(), P, kmax, dW.data_ptr(), dH.data_ptr(),
+        float(beta), int(update_H), int(max_iter), float(tol), 0 if resident else 1,
+        work.data_ptr() if not resident else None, d_iter.data_ptr(), d_err.data_ptr(), d_vaf.data_ptr(),
+        ctypes.c_void_p(stream.cuda_stream)), "ms_nmf_beta")
+    return d_iter, d_err, d_vaf, work
+
+
 # sklearn's texts for the input checks of NMF.transform (sklearn.utils.validation)
 _TRANSFORM_NAN = "Input X contains NaN."
 _TRANSFORM_INF = "Input X contains infinity or a value too large for dtype('float64')."
@@ -441,10 +619,12 @@ def _check_transform_host(Xh: np.ndarray):
         raise ValueError(_TRANSFORM_NEGATIVE)
 
 
-def _transform_args(X, H, x_index, solver, max_iter, tol, regime):
+def _transform_args(X, H, x_index, solver, max_iter, tol, regime, beta_loss="frobenius"):
     """Validates what nmf_transform_batched is given, without touching a device; returns (H list, m, x_index)."""
     if solver not in _SOLVER_CODES:
         raise ValueError(f"solver must be 'cd' or 'mu', not {solver!r}")
+    if _beta_to_float(beta_loss) != 2.0 and solver != "mu":
+        raise _beta_solver_error(solver, beta_loss)
     if regime not in (None, "resident", "stream"):
         raise ValueError(f"regime must be None, 'resident' or 'stream', not {regime!r}")
     if int(max_iter) < 0 or not float(tol) >= 0:
@@ -474,7 +654,7 @@ def _transform_args(X, H, x_index, solver, max_iter, tol, regime):
 
 def nmf_transform_batched(X, H: Sequence, x_index: Optional[Sequence[int]] = None, solver: str = "cd",
                           max_iter: int = 200, tol: float = 1e-4, regime: Optional[str] = None,
-                          defer: bool = False) -> Union[NMFBatchResult, PendingNMF]:
+                          defer: bool = False, beta_loss="frobenius") -> Union[NMFBatchResult, PendingNMF]:
     """Fits activations to fixed synergies - scikit-learn's `NMF.transform` (update_H=False, no regularisation) - for a
     batch of problems in one launch, in fp64: problem p fits W_p >= 0 to X[x_index[p]] with H[p] (k_p x m) fixed.
 
@@ -482,21 +662,26 @@ def nmf_transform_batched(X, H: Sequence, x_index: Optional[Sequence[int]] = Non
     X: a non-negative (n, m) matrix or a (B, n, m) stack, as a numpy array or a CUDA tensor (which never leaves the
     device; a strided view such as the (samples, channels) `env.T` of a channel-major envelope is read in place).
     A negative or non-finite X raises ValueError (under defer, from `.result()`).  regime: None (by size),
-    "resident" or "stream".  Returns an NMFBatchResult whose H are the given matrices and whose seeds are -1, or a
+    "resident" or "stream".  beta_loss: "frobenius" (2), or with solver "mu" "kullback-leibler" (1), "itakura-saito"
+    (0) or any other float - then err is sklearn's square-rooted β-divergence, and a zero in X with beta_loss <= 0
+    raises sklearn's ValueError.  Returns an NMFBatchResult whose H are the given matrices and whose seeds are -1, or a
     PendingNMF when defer=True."""
-    return _nmf_transform(X, H, x_index, solver, max_iter, tol, regime, defer)
+    return _nmf_transform(X, H, x_index, solver, max_iter, tol, regime, defer, beta_loss=beta_loss)
 
 
-def _nmf_transform(X, H, x_index, solver, max_iter, tol, regime, defer, device_w=False):
+def _nmf_transform(X, H, x_index, solver, max_iter, tol, regime, defer, device_w=False, beta_loss="frobenius"):
     import torch
 
     on_device = isinstance(X, torch.Tensor) and X.is_cuda
     if not on_device:
         Xh = X.detach().to("cpu", torch.float64).numpy() if isinstance(X, torch.Tensor) else np.asarray(X, dtype=np.float64)
         X = Xh
-    Hs, m, xi = _transform_args(X, H, x_index, solver, max_iter, tol, regime)
+    Hs, m, xi = _transform_args(X, H, x_index, solver, max_iter, tol, regime, beta_loss)
+    beta = _beta_to_float(beta_loss)
     if not on_device:
         _check_transform_host(X)
+        if beta <= 0 and X.min() == 0:
+            raise ValueError(_BETA_ZEROS)
     lib = nat.lib()
     if not torch.cuda.is_available():
         raise nat.NativeError("nmf_transform_batched needs a CUDA device; there is no CPU fallback")
@@ -514,6 +699,8 @@ def _nmf_transform(X, H, x_index, solver, max_iter, tol, regime, defer, device_w
             dX = dX.contiguous()
         flags = (torch.isnan(dX).any(), torch.isinf(dX).any(), (dX < 0).any())
         checks = tuple(zip((_TRANSFORM_NAN, _TRANSFORM_INF, _TRANSFORM_NEGATIVE), flags))
+        if beta <= 0:
+            checks += ((_BETA_ZEROS, (dX == 0).any()),)
         if not defer:
             for msg, flag in checks:
                 if bool(flag):
@@ -539,16 +726,22 @@ def _nmf_transform(X, H, x_index, solver, max_iter, tol, regime, defer, device_w
         else:
             dW = torch.from_numpy(np.sqrt(means[xi] / ranks)).to(dev)[w_problem]
         dH = torch.from_numpy(np.concatenate([h.ravel() for h in Hs])).to(dev)
-        d_iter = torch.empty(P, dtype=torch.int32, device=dev)
-        d_err = torch.empty(P, dtype=torch.float64, device=dev)
-        d_vaf = torch.empty((P, m + 1), dtype=torch.float64, device=dev)
-        work = torch.empty(0 if resident else int(lib.ms_nmf_fixed_h_workspace_bytes(n, m, P, kmax)), dtype=torch.uint8,
-                           device=dev)
-        keep.append(work)
-        nat.check(lib.ms_nmf_fixed_h(
-            dX.data_ptr(), n, m, dX.stride(1), dX.stride(2), table.data_ptr(), P, kmax, dW.data_ptr(), dH.data_ptr(),
-            _SOLVER_CODES[solver], int(max_iter), float(tol), 0 if resident else 1, work.data_ptr() if not resident else None,
-            d_iter.data_ptr(), d_err.data_ptr(), d_vaf.data_ptr(), ctypes.c_void_p(stream.cuda_stream)), "ms_nmf_fixed_h")
+        if beta != 2.0:  # the β-divergence: the same loop as the fit, H fixed
+            d_iter, d_err, d_vaf, work = _beta_launch(torch, lib, dX, n, m, table, P, kmax, dW, dH, beta, 0, max_iter,
+                                                      tol, regime, stream)
+            keep.append(work)
+        else:
+            d_iter = torch.empty(P, dtype=torch.int32, device=dev)
+            d_err = torch.empty(P, dtype=torch.float64, device=dev)
+            d_vaf = torch.empty((P, m + 1), dtype=torch.float64, device=dev)
+            work = torch.empty(0 if resident else int(lib.ms_nmf_fixed_h_workspace_bytes(n, m, P, kmax)),
+                               dtype=torch.uint8, device=dev)
+            keep.append(work)
+            nat.check(lib.ms_nmf_fixed_h(
+                dX.data_ptr(), n, m, dX.stride(1), dX.stride(2), table.data_ptr(), P, kmax, dW.data_ptr(), dH.data_ptr(),
+                _SOLVER_CODES[solver], int(max_iter), float(tol), 0 if resident else 1,
+                work.data_ptr() if not resident else None, d_iter.data_ptr(), d_err.data_ptr(), d_vaf.data_ptr(),
+                ctypes.c_void_p(stream.cuda_stream)), "ms_nmf_fixed_h")
         if device_w:
             return dW, d_iter
         if defer:
@@ -594,7 +787,7 @@ class NMFModel:
 
     def transform(self, X):
         """sklearn's `NMF.transform`: the activations W >= 0 that fit X with these components fixed, by the model's
-        solver, max_iter and tol, on the GPU in fp64 (`nmf_transform_batched`).  X: a DataFrame, an ndarray or a CUDA
+        solver, beta_loss, max_iter and tol, on the GPU in fp64 (`nmf_transform_batched`).  X: a DataFrame, an ndarray or a CUDA
         tensor (n, n_features_in_); returns an (n, n_components) ndarray, or a CUDA tensor for a CUDA input.  Raises
         sklearn's ValueErrors for non-finite or negative X and a wrong feature count, and emits its ConvergenceWarning
         when max_iter is reached with tol > 0."""
@@ -615,7 +808,7 @@ class NMFModel:
         if X.shape[1] != self.n_features_in_:
             raise ValueError(f"X has {X.shape[1]} features, but NMF is expecting {self.n_features_in_} features as input.")
         W, n_iter = _nmf_transform(X, [self.components_], None, self.solver, self.max_iter, self.tol, None, False,
-                                   device_w=True)
+                                   device_w=True, beta_loss=self.beta_loss)
         if self.tol > 0 and int(n_iter[0]) == self.max_iter:
             from sklearn.exceptions import ConvergenceWarning
 
@@ -684,7 +877,9 @@ def find_synergies(
     default solver="cd", nndsvd inits, regularisation ...) is forwarded to scikit-learn as the reference does.
     engine="sklearn" always forwards.  engine="gpu" runs on the GPU solver="cd" (the default; fp64, `nmf_cd_batched`)
     or "mu", with init None (resolved as scikit-learn does: "nndsvda" if k <= min(n_samples, n_features), else
-    "random"), "nndsvd", "nndsvda" or "random", and raises NotImplementedError for any other keyword or value."""
+    "random"), "nndsvd", "nndsvda" or "random", and raises NotImplementedError for any other keyword or value.  With
+    solver="mu" it also runs beta_loss "kullback-leibler", "itakura-saito" or any float (fp64, `nmf_beta_batched`);
+    solver="cd" with beta_loss != 2 raises scikit-learn's ValueError."""
     if engine not in ("auto", "sklearn", "gpu"):
         raise ValueError(f"engine must be 'auto', 'sklearn' or 'gpu', not {engine!r}")
     if processed_emg_df.empty:
@@ -722,9 +917,11 @@ def find_synergies(
                            for i, k in enumerate(ranks_sweep)}, "mu", {k: "random" for k in ranks_sweep}, max_iter, tol)
 
 
-def _synergy_result(processed_emg_df, max_components, ranks_sweep, n_restarts, batches, solver, inits, max_iter, tol):
+def _synergy_result(processed_emg_df, max_components, ranks_sweep, n_restarts, batches, solver, inits, max_iter, tol,
+                    beta_loss="frobenius"):
     """The SynergyRunResult of a sweep whose rank k has n_restarts consecutive problems in batch batches[k][0],
-    starting at problem batches[k][1]: per rank, the restart with the smallest reconstruction error."""
+    starting at problem batches[k][1]: per rank, the restart with the smallest reconstruction error (the
+    square-rooted β-divergence for beta_loss != "frobenius")."""
     num_features = len(processed_emg_df.columns)
     columns = processed_emg_df.columns
     labels = ["All signals"] + columns.tolist()
@@ -739,8 +936,8 @@ def _synergy_result(processed_emg_df, max_components, ranks_sweep, n_restarts, b
         table.insert(0, "random_state", res.seeds[sl])
         seed = int(res.seeds[best])
         model = NMFModel(k, res.H[best].astype(np.float64), int(res.n_iter[best]), float(res.err[best]),
-                         num_features, seed if seed >= 0 else None, solver=solver, init=inits[k], restarts=table,
-                         max_iter=max_iter, tol=tol)
+                         num_features, seed if seed >= 0 else None, solver=solver, beta_loss=beta_loss, init=inits[k],
+                         restarts=table, max_iter=max_iter, tol=tol)
         transformed = res.W[best].astype(np.float64)
         comps = pandas.DataFrame(model.components_, columns=columns)
         vaf_values = vaf(processed_emg_df, components=model.components_, transformed_signal=transformed)
@@ -773,8 +970,17 @@ def _find_synergies_gpu(df, n_components, max_components, max_iter, tol, n_resta
         raise NotImplementedError(f"find_synergies(engine='gpu') does not implement solver={solver!r}")
     if init not in (None, "nndsvd", "nndsvda", "random"):
         raise NotImplementedError(f"find_synergies(engine='gpu') does not implement init={init!r}")
-    if beta_loss not in ("frobenius", 2, 2.0):
-        raise NotImplementedError(f"find_synergies(engine='gpu') does not implement beta_loss={beta_loss!r}")
+    try:
+        beta = _beta_to_float(beta_loss)
+    except ValueError:
+        raise NotImplementedError(f"find_synergies(engine='gpu') does not implement beta_loss={beta_loss!r}") from None
+    if beta != 2.0:
+        if solver != "mu":
+            raise _beta_solver_error(solver, beta_loss)
+        if init == "nndsvd":
+            warnings.warn("The multiplicative update ('mu') solver cannot update zeros present in the initialization, "
+                          "and so leads to poorer results when used jointly with init='nndsvd'. You may try "
+                          "init='nndsvda' or init='nndsvdar' instead.", UserWarning)
     n, m = df.shape
     ranks_sweep = [n_components] if max_components is None else list(range(n_components, max_components + 1))
     inits = {k: init if init is not None else ("nndsvda" if k <= min(n, m) else "random") for k in ranks_sweep}
@@ -790,7 +996,9 @@ def _find_synergies_gpu(df, n_components, max_components, max_iter, tol, n_resta
         group = [k for k in ranks_sweep if inits[k] == how]
         ranks = [k for k in group for _ in range(n_restarts)]
         seeds = [int(seed) + r for _ in group for r in range(n_restarts)] if how == "random" else None
-        if solver == "cd":
+        if beta != 2.0:
+            res = nmf_beta_batched(X, ranks, beta_loss, init=how, seeds=seeds, max_iter=max_iter, tol=tol)
+        elif solver == "cd":
             res = nmf_cd_batched(X, ranks, init=how, seeds=seeds, max_iter=max_iter, tol=tol)
         elif how == "random":
             res = nmf_mu_batched(X, ranks, seeds, max_iter=max_iter, tol=tol)
@@ -804,4 +1012,5 @@ def _find_synergies_gpu(df, n_components, max_components, max_iter, tol, n_resta
             warnings.warn("Maximum number of iterations %d reached. Increase it to improve convergence." % max_iter,
                           ConvergenceWarning)
         batches.update({k: (res, i * n_restarts) for i, k in enumerate(group)})
-    return _synergy_result(df, max_components, ranks_sweep, n_restarts, batches, solver, inits, max_iter, tol)
+    return _synergy_result(df, max_components, ranks_sweep, n_restarts, batches, solver, inits, max_iter, tol,
+                           beta_loss if beta != 2.0 else "frobenius")

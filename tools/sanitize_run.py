@@ -33,6 +33,10 @@ analysis.nmf_cd_batched(x, [2, 3, 4], init="nndsvda", max_iter=10, regime="strea
 analysis.nmf_cd_batched(np.stack([x[:300], x[300:600]]), [1, 3, 6], init="nndsvd", x_index=[0, 1, 1], max_iter=10)
 analysis.nmf_transform_batched(x, [np.ones((2, 6)), np.ones((4, 6))], solver="cd", max_iter=10, regime="stream")
 analysis.nmf_transform_batched(x[:300], [np.ones((3, 6))], solver="mu", max_iter=30, regime="resident")
+analysis.nmf_beta_batched(x, [2, 3, 4], "kullback-leibler", max_iter=25, tol=1e-4, regime="stream")
+analysis.nmf_beta_batched(x[:300] + 0.01, [1, 3, 6], "itakura-saito", init="random", seeds=[0, 1, 2], max_iter=25)
+analysis.nmf_beta_batched(x[:300], [2, 5], 1.5, max_iter=25, tol=1e-4, regime="resident")
+analysis.nmf_transform_batched(x + 0.01, [np.ones((2, 6))], solver="mu", max_iter=25, regime="stream", beta_loss=0.5)
 res = trial_synergies(trial, 1, 3, max_iter=20, segmenter=seg, solver="cd")
 df = pd.DataFrame(x, columns=list("abcdef"))
 emg.linear_envelope(df, 6.0, 2000, 4); emg.rms(df, 100); emg.digital_filter(df, (20.0, 450.0), 2000, 2, band_type="bandpass", zero_lag=False)
