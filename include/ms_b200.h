@@ -370,6 +370,33 @@ int ms_nmf_beta(const double* d_X, int64_t n, int32_t m, int64_t row_stride, int
                 int32_t max_iter, double tol, int32_t regime, void* d_work, int32_t* d_n_iter, double* d_err,
                 double* d_vaf, void* stream);
 
+/* ---- synergy comparison (extension; fp64) --------------------------------------------------- */
+
+/* One synergy set of a packed array: rows [offset, offset + k * m) of d_H are its k synergy vectors (row-major). */
+typedef struct ms_synergy_set {
+    int64_t offset;   /* element offset of the set's first row in d_H */
+    int32_t k;        /* rank: rows of the set, 1..kmax */
+    int32_t reserved;
+} ms_synergy_set;
+
+/* Matched cosine similarity of pairs of synergy sets of equal rank, the standard comparison of synergies between
+ * cycles, trials or subjects.  For pair p = (a, b) = d_pairs[2p], d_pairs[2p + 1] (int32 indices into d_sets, device
+ * memory, 8-byte aligned): S[i][j] = <a_i, b_j> / (||a_i|| ||b_j||) (0 where a row's norm is 0 or its squared norm
+ * overflows), then the exact
+ * maximum-weight perfect matching on S that scipy.optimize.linear_sum_assignment(S, maximize=True) finds (shortest
+ * augmenting paths, O(k^3); among equal tentative distances the lowest column is taken).  Writes d_mean[p], the mean
+ * matched similarity; d_pairs NULL: every pair a < b of the table, in np.triu_indices(n_sets, 1) order (the kernel
+ * decodes p; n_pairs must be n_sets (n_sets - 1) / 2).  d_perm[p * kmax + i] (int8), the row of b paired with row i of a, and d_sim[p * kmax + i], that
+ * similarity, both for i < k and -1 / NaN for k <= i < kmax; d_perm and d_sim may be NULL.  kmax: the largest rank in
+ * the table, 1..16; m: 1..64.  d_work: ms_synergy_match_workspace_bytes(n_sets) bytes (the norms, once per set).  A
+ * set whose rank is outside 1..kmax, a pair index outside the table or a pair of unequal ranks is found on the device:
+ * the entry then returns MS_E_INVALID (that pair's outputs are NaN / -1).  Synchronises `stream` to read that check.
+ * No floating-point atomics: repeated calls are bit-identical. */
+int64_t ms_synergy_match_workspace_bytes(int32_t n_sets);
+int ms_synergy_match(const double* d_H, int32_t m, const ms_synergy_set* d_sets, int32_t n_sets, int32_t kmax,
+                     const int32_t* d_pairs, int64_t n_pairs, int8_t* d_perm, double* d_sim, double* d_mean,
+                     void* d_work, int64_t work_bytes, void* stream);
+
 /* ---- misc ------------------------------------------------------------------------------- */
 /* The used part of a channel-major block (rows channels of width_bytes each, src_pitch_bytes apart) to host
  * memory as one 2-D copy on the DMA engine; asynchronous when h_dst is page-locked. */

@@ -11,8 +11,8 @@ there is no CPU fallback.
 """
 __version__ = "0.1.0"
 
-from .analysis import (SynergyRunResult, find_synergies, nmf_beta_batched, nmf_cd_batched, nmf_mu_batched,  # noqa: F401
-                       nmf_transform_batched, vaf)
+from .analysis import (SynergyMatch, SynergyRunResult, find_synergies, match_synergies_batched,  # noqa: F401
+                       nmf_beta_batched, nmf_cd_batched, nmf_mu_batched, nmf_transform_batched, vaf)
 from .cache import load_trial, load_vicon_file_cached, save_trial  # noqa: F401
 from .emg import (  # noqa: F401
     digital_filter,
@@ -23,7 +23,8 @@ from .emg import (  # noqa: F401
     time_normalize,
     zero_center,
 )
-from .pipeline import cross_cycle_vaf, synergies_for_files, synergies_for_files_sharded, trial_synergies  # noqa: F401
+from .pipeline import (cross_cycle_vaf, synergies_for_files, synergies_for_files_sharded,  # noqa: F401
+                       synergy_similarity, trial_synergies)
 from .vicon_data import (  # noqa: F401
     DeviceData,
     DeviceType,
@@ -50,6 +51,7 @@ __all__ = (
     "vaf",
     "find_synergies",
     # extensions
+    "match_synergies_batched",
     "nmf_beta_batched",
     "nmf_cd_batched",
     "nmf_mu_batched",
@@ -60,6 +62,7 @@ __all__ = (
     "load_vicon_file_cached",
     "trial_synergies",
     "cross_cycle_vaf",
+    "synergy_similarity",
     "synergies_for_files",
     "synergies_for_files_sharded",
 )

@@ -152,6 +152,8 @@ def _declare(L):
         "ms_nmf_beta_workspace_bytes": (i64, [i64, i32, i32, i32]),
         "ms_nmf_beta": (ctypes.c_int, [vp, i64, i32, i64, i64, vp, i32, i32, vp, vp, ctypes.c_double, i32, i32,
                                        ctypes.c_double, i32, vp, vp, vp, vp, vp]),
+        "ms_synergy_match_workspace_bytes": (i64, [i32]),
+        "ms_synergy_match": (ctypes.c_int, [vp, i32, vp, i32, i32, vp, i64, vp, vp, vp, vp, i64, vp]),
         "ms_parse_long_workspace_bytes": (i64, [i64]),
         "ms_parse_long": (ctypes.c_int, [vp, i64, vp, ctypes.POINTER(Section), i32, i64, vp, vp, vp]),
         "ms_load_workspace_bytes": (i64, [i64, i32]),

@@ -31,6 +31,11 @@ sklearn's multiplicative updates for the β-divergence (beta_loss "kullback-leib
 float other than 2) on the GPU in fp64 (csrc/ms_nmf_beta.cu).  Parity claim, against sklearn in fp64: from the same init
 at the same iteration count (tol=0), W H, VAF and err (sklearn's reconstruction_err_, the square-rooted divergence) agree
 to 1e-9; converged, VAF agrees to 1e-8 and n_iter to one check (10) (tests/test_nmf_beta_gpu.py).
+
+`match_synergies_batched` compares synergy sets pair by pair - unit-length synergies, the optimal one-to-one pairing
+of `scipy.optimize.linear_sum_assignment(maximize=True)`, the mean matched similarity - on the GPU in fp64
+(csrc/ms_synmatch.cu); mean and per-synergy similarity agree with numpy + scipy to 1e-12
+(tests/test_synergy_match_gpu.py).
 """
 import ctypes
 import functools
@@ -749,6 +754,171 @@ def _nmf_transform(X, H, x_index, solver, max_iter, tol, regime, defer, device_w
         Wall = dW.cpu().numpy()
         n_iter, err, vafs = d_iter.cpu().numpy(), d_err.cpu().numpy(), d_vaf.cpu().numpy()
     return _assemble(ranks, seeds, n, m, Wall, np.concatenate([h.ravel() for h in Hs]), n_iter, err, vafs)
+
+
+# ---- synergy comparison -------------------------------------------------------------------------------
+@dataclass
+class SynergyMatch:
+    """What `match_synergies_batched` returns: numpy arrays, or CUDA tensors for a CUDA H.  kmax is the largest rank
+    among the sets; a pair of rank k < kmax has -1 (perm) and NaN (sim) in its columns k .. kmax - 1."""
+
+    mean: object          # (P,) float64: mean matched cosine similarity of each pair
+    sim: object = None    # (P, kmax) float64: sim[p, i] = similarity of row i of a and row perm[p, i] of b
+    perm: object = None   # (P, kmax) int8: the row of b paired with row i of a
+
+
+def _match_sets(H):
+    """(on_device, list of sets, m) after the shape checks of match_synergies_batched; a set is a 2-D numpy array or
+    a 2-D CUDA tensor.  Touches no device."""
+    import torch
+
+    if not isinstance(H, (list, tuple)):
+        if not (isinstance(H, torch.Tensor) and H.is_cuda):
+            H = H.detach().cpu().numpy() if isinstance(H, torch.Tensor) else np.asarray(H)
+        if H.ndim != 3:
+            raise ValueError(f"H must be a list of (k, m) synergy sets or an (S, k, m) stack, not shape {tuple(H.shape)}")
+        if isinstance(H, torch.Tensor):  # a CUDA stack stays one tensor: S can be large
+            S, k, m = H.shape
+            if S < 1 or not 1 <= k <= 16 or not 1 <= m <= 64:
+                raise ValueError(f"H is a stack of {S} sets of rank k = {k} with m = {m} muscles: a synergy set needs "
+                                 "1 <= k <= 16 and 1 <= m <= 64")
+            return True, H, m
+    sets = list(H)
+    on_device = any(isinstance(h, torch.Tensor) and h.is_cuda for h in sets)
+    out = []
+    for s, h in enumerate(sets):
+        if not (isinstance(h, torch.Tensor) and h.is_cuda):
+            h = h.detach().cpu().numpy() if isinstance(h, torch.Tensor) else np.asarray(h)
+        if h.ndim != 2:
+            raise ValueError(f"H[{s}] must be a (k, m) synergy set, not shape {tuple(h.shape)}")
+        out.append(h)
+    if not out:
+        raise ValueError("H holds no synergy set")
+    m = int(out[0].shape[1])
+    for s, h in enumerate(out):
+        k = int(h.shape[0])
+        if not 1 <= k <= 16:
+            raise ValueError(f"H[{s}] has rank k = {k}: a synergy set has 1 <= k <= 16 rows")
+        if int(h.shape[1]) != m:
+            raise ValueError(f"H[{s}] has m = {h.shape[1]} muscles, H[0] has {m}: every set must have the same m")
+    if not 1 <= m <= 64:
+        raise ValueError(f"the sets have m = {m} muscles: 1 <= m <= 64 is supported")
+    return on_device, out, m
+
+
+def _match_pairs(pairs, ranks, n_sets):
+    """Checks a host (P, 2) pair list against the sets' ranks (an array, or an int for a stack); returns it as int32."""
+    pairs = np.asarray(pairs)
+    if pairs.ndim != 2 or pairs.shape[1] != 2 or not (pairs.size == 0 or np.issubdtype(pairs.dtype, np.integer)):
+        raise ValueError(f"pairs must be a (P, 2) integer array of set indices, not {pairs.dtype} {pairs.shape}")
+    if pairs.size and (pairs.min() < 0 or pairs.max() >= n_sets):
+        bad = int(np.flatnonzero(((pairs < 0) | (pairs >= n_sets)).any(axis=1))[0])
+        raise ValueError(f"pair {bad} = {tuple(pairs[bad].tolist())} names a set H does not have ({n_sets} sets)")
+    if not isinstance(ranks, int) and pairs.size:
+        ka, kb = ranks[pairs[:, 0]], ranks[pairs[:, 1]]
+        if (ka != kb).any():
+            bad = int(np.flatnonzero(ka != kb)[0])
+            a, b = pairs[bad]
+            raise ValueError(f"pair {bad} compares H[{a}] (rank {ka[bad]}) with H[{b}] (rank {kb[bad]}): both sets of a "
+                             "pair must have the same rank")
+    return np.ascontiguousarray(pairs, dtype=np.int32)
+
+
+def match_synergies_batched(H, pairs=None, *, similarities: bool = False, permutations: bool = False) -> SynergyMatch:
+    """Compares synergy sets pair by pair in one launch, the standard comparison of synergies between gait cycles,
+    trials or subjects: each synergy vector (a row of `components_`) is scaled to unit length (a zero row has
+    similarity 0 with everything), the k x k matrix S of scalar products is formed, and the rows are paired one to one
+    so that the summed similarity is as large as possible - the optimum `scipy.optimize.linear_sum_assignment(S,
+    maximize=True)` finds.  fp64 (csrc/ms_synmatch.cu).
+
+    H: a list of (k, m) synergy sets or an (S, k, m) stack, as numpy arrays or CUDA tensors (which never leave the
+    device); 1 <= k <= 16, 1 <= m <= 64, finite.  pairs: a (P, 2) array of set indices, both sets of a pair of the same
+    rank; None compares every unordered pair a < b, in `np.triu_indices(S, 1)` order, generated on the device (the
+    kernel decodes the pair index: no pair list is built).
+    Returns a SynergyMatch with `mean` (P,) and, on request, `sim` and `perm` (P, kmax).  Argument errors raise
+    ValueError, naming the set or pair, before any native call."""
+    import torch
+
+    on_device, sets, m = _match_sets(H)
+    stack = isinstance(sets, torch.Tensor)
+    n_sets = int(sets.shape[0]) if stack else len(sets)
+    if stack:
+        ranks, kmax = int(sets.shape[1]), int(sets.shape[1])
+    else:
+        ranks = np.array([h.shape[0] for h in sets], dtype=np.int64)
+        kmax = int(ranks.max())
+    pairs_dev = None
+    if pairs is None:
+        if stack or (ranks == ranks[0]).all():
+            pass  # every pair of the triangle has equal ranks
+        else:
+            raise ValueError("pairs=None compares every pair of sets, but H mixes ranks "
+                             f"{sorted(set(ranks.tolist()))}: give the pairs of equal rank")
+    elif isinstance(pairs, torch.Tensor) and pairs.is_cuda:
+        if pairs.ndim != 2 or pairs.shape[1] != 2 or pairs.dtype.is_floating_point or pairs.dtype == torch.bool:
+            raise ValueError(f"pairs must be a (P, 2) integer array of set indices, not {pairs.dtype} {tuple(pairs.shape)}")
+        pairs_dev = pairs
+        if pairs.numel():
+            if int(pairs.min()) < 0 or int(pairs.max()) >= n_sets:
+                raise ValueError(f"pairs names a set H does not have ({n_sets} sets)")
+            if not stack:
+                r = torch.from_numpy(ranks).to(pairs.device)[pairs.long()]
+                differ = (r[:, 0] != r[:, 1]).nonzero()
+                if differ.numel():
+                    bad = int(differ[0, 0])
+                    a, b = pairs[bad].tolist()
+                    raise ValueError(f"pair {bad} compares H[{a}] (rank {ranks[a]}) with H[{b}] (rank {ranks[b]}): "
+                                     "both sets of a pair must have the same rank")
+    else:
+        pairs = _match_pairs(pairs, ranks, n_sets)
+    # the sets as one fp64 array (a CUDA one never leaves its device), checked for finiteness in one pass
+    if stack:
+        flat = sets.detach().to(torch.float64).contiguous().view(-1)
+    elif on_device:
+        dev = next(h.device for h in sets if isinstance(h, torch.Tensor))
+        flat = torch.cat([torch.as_tensor(h, device=dev).detach().to(torch.float64).reshape(-1) for h in sets])
+    else:
+        flat = np.concatenate([np.asarray(h, dtype=np.float64).ravel() for h in sets])
+    if not bool((torch.isfinite(flat) if on_device else np.isfinite(flat)).all()):
+        if stack:
+            raise ValueError("H contains a non-finite entry")
+        finite = [bool((torch.isfinite(h) if isinstance(h, torch.Tensor) else np.isfinite(h)).all()) for h in sets]
+        bad = finite.index(False)
+        raise ValueError(f"H[{bad}] contains a non-finite entry")
+
+    lib = nat.lib()
+    if not torch.cuda.is_available():
+        raise nat.NativeError("match_synergies_batched needs a CUDA device; there is no CPU fallback")
+    dev = flat.device if on_device else torch.device(f"cuda:{torch.cuda.current_device()}")
+    with torch.cuda.device(dev):
+        table = torch.zeros((n_sets, 2), dtype=torch.int64, device=dev)  # ms_synergy_set: offset, then k | reserved << 32
+        dH = flat if on_device else torch.from_numpy(flat).to(dev)
+        if stack:
+            table[:, 0] = torch.arange(n_sets, device=dev) * (kmax * m)
+            table[:, 1] = kmax
+        else:
+            offsets = np.concatenate([[0], np.cumsum(ranks * m)[:-1]])
+            table.copy_(torch.from_numpy(np.stack([offsets, ranks], axis=1)))
+        if pairs_dev is not None:
+            dP = pairs_dev.to(device=dev, dtype=torch.int32).contiguous()
+        elif pairs is not None:
+            dP = torch.from_numpy(pairs).to(dev)
+        else:
+            dP = None  # every pair a < b: the kernel decodes the pair index, no list is built
+        P = int(dP.shape[0]) if dP is not None else n_sets * (n_sets - 1) // 2
+        d_mean = torch.empty(P, dtype=torch.float64, device=dev)
+        d_sim = torch.empty((P, kmax), dtype=torch.float64, device=dev) if similarities else None
+        d_perm = torch.empty((P, kmax), dtype=torch.int8, device=dev) if permutations else None
+        work = torch.empty(int(lib.ms_synergy_match_workspace_bytes(n_sets)), dtype=torch.uint8, device=dev)
+        stream = torch.cuda.current_stream(dev)
+        nat.check(lib.ms_synergy_match(
+            dH.data_ptr(), m, table.data_ptr(), n_sets, kmax, dP.data_ptr() if dP is not None else None, P,
+            d_perm.data_ptr() if d_perm is not None else None, d_sim.data_ptr() if d_sim is not None else None,
+            d_mean.data_ptr(), work.data_ptr(), work.numel(), ctypes.c_void_p(stream.cuda_stream)), "ms_synergy_match")
+    if on_device:
+        return SynergyMatch(d_mean, d_sim, d_perm)
+    return SynergyMatch(d_mean.cpu().numpy(), d_sim.cpu().numpy() if similarities else None,
+                        d_perm.cpu().numpy() if permutations else None)
 
 
 # ---- reference API ------------------------------------------------------------------------------------

@@ -22,7 +22,7 @@ from typing import Dict, Iterable, List, Optional, Sequence, Tuple, Union
 import numpy as np
 import pandas
 
-from .analysis import NMFBatchResult, nmf_cd_batched, nmf_mu_batched, nmf_transform_batched
+from .analysis import NMFBatchResult, match_synergies_batched, nmf_cd_batched, nmf_mu_batched, nmf_transform_batched
 from .emg import envelope_windows
 from .segment import Cycle, Segmenter, Trecho
 from .vicon_data import ViconLoader, ViconNexusData
@@ -217,6 +217,29 @@ def cross_cycle_vaf(trial: TrialSynergies, ranks: Optional[Sequence[int]] = None
                                           names=["n_components", "trecho", "cycle"])
     columns = pandas.MultiIndex.from_tuples([(c.trecho.value, c.cycle.value) for c in cycles], names=["trecho", "cycle"])
     return pandas.DataFrame(res.vaf[:, 0].reshape(len(ranks) * n_cyc, n_cyc), index=index, columns=columns)
+
+
+def synergy_similarity(trial: TrialSynergies, ranks: Optional[Sequence[int]] = None) -> pandas.DataFrame:
+    """How alike the synergies of the trial's cycles are: for every rank, every pair of cycles' synergy sets (the best
+    restart's `components`) is compared by matched cosine similarity (`match_synergies_batched`: unit-length synergy
+    vectors, optimal one-to-one pairing, mean of the matched similarities), all ranks x pairs in one launch.  The
+    companion of `cross_cycle_vaf`, in its layout: index (n_components, source trecho, source cycle), columns (target
+    trecho, target cycle).  Pairs a < b are computed and mirrored, so the table is exactly symmetric; the diagonal is
+    computed too."""
+    cycles = trial.cycles
+    ranks = list(cycles[0].components) if ranks is None else [int(k) for k in ranks]
+    n_cyc = len(cycles)
+    H = [c.components[k].to_numpy(dtype=np.float64) for k in ranks for c in cycles]
+    a, b = np.triu_indices(n_cyc)
+    pairs = np.concatenate([np.stack([a, b], axis=1) + r * n_cyc for r in range(len(ranks))])
+    mean = match_synergies_batched(H, pairs).mean.reshape(len(ranks), -1)
+    table = np.empty((len(ranks), n_cyc, n_cyc))
+    table[:, a, b] = mean
+    table[:, b, a] = mean
+    index = pandas.MultiIndex.from_tuples([(k, c.trecho.value, c.cycle.value) for k in ranks for c in cycles],
+                                          names=["n_components", "trecho", "cycle"])
+    columns = pandas.MultiIndex.from_tuples([(c.trecho.value, c.cycle.value) for c in cycles], names=["trecho", "cycle"])
+    return pandas.DataFrame(table.reshape(len(ranks) * n_cyc, n_cyc), index=index, columns=columns)
 
 
 def synergies_for_files(paths: Sequence[str], loader: Optional[ViconLoader] = None, **kwargs) -> Iterable[Tuple[str, TrialSynergies]]:

@@ -38,6 +38,7 @@ analysis.nmf_beta_batched(x[:300] + 0.01, [1, 3, 6], "itakura-saito", init="rand
 analysis.nmf_beta_batched(x[:300], [2, 5], 1.5, max_iter=25, tol=1e-4, regime="resident")
 analysis.nmf_transform_batched(x + 0.01, [np.ones((2, 6))], solver="mu", max_iter=25, regime="stream", beta_loss=0.5)
 res = trial_synergies(trial, 1, 3, max_iter=20, segmenter=seg, solver="cd")
+analysis.match_synergies_batched([np.ones((3, 6)), x[:3, :], x[3:5, :], x[5:7, :]], [[0, 1], [2, 3], [1, 1]], similarities=True, permutations=True)
 df = pd.DataFrame(x, columns=list("abcdef"))
 emg.linear_envelope(df, 6.0, 2000, 4); emg.rms(df, 100); emg.digital_filter(df, (20.0, 450.0), 2000, 2, band_type="bandpass", zero_lag=False)
 torch.cuda.synchronize()
