@@ -147,7 +147,7 @@ def _batch_plan_locked(torch, lib, n, m, ranks, xi, dev):
     return hit
 
 
-_pinned_pool = {}  # nbytes -> pinned uint8 tensors not on loan (results of deferred runs travel through them)
+_pinned_pool = OrderedDict()  # nbytes -> pinned uint8 tensors not on loan (results travel through them), 32 sizes at most
 
 
 def _pinned_take(torch, nbytes: int):
@@ -157,8 +157,11 @@ def _pinned_take(torch, nbytes: int):
 
 def _pinned_give(buf):
     free = _pinned_pool.setdefault(int(buf.numel()), [])
+    _pinned_pool.move_to_end(int(buf.numel()))
     if len(free) < 4:
         free.append(buf)
+    while len(_pinned_pool) > 32:  # calls on ever new shapes must not keep pinned memory for each
+        _pinned_pool.popitem(last=False)
 
 
 _NEGATIVE_X = "Negative values in data passed to NMF (input X)"
@@ -171,17 +174,13 @@ class PendingNMF:
     for the copies and builds the NMFBatchResult.  Lets a caller queue the next trial's GPU work before it
     looks at this one's (pipeline.synergies_for_files)."""
 
-    def __init__(self, torch, stream, ranks, seeds, n, m, device_arrays, keep, negative=None, degenerate=None,
-                 checks=()):
+    def __init__(self, torch, stream, ranks, seeds, n, m, device_arrays, keep, checks=()):
         self._ranks, self._seeds, self._n, self._m = ranks, seeds, n, m
         self._keep = keep  # inputs of the kernel: alive until the copies below have run
         self._bufs = []
-        # device flags travel with the results: "X has a negative entry", "the NNDSVD init divided by zero", and any
-        # other (message, flag) of `checks`; the first one set is raised
-        pairs = [(_NEGATIVE_X, negative), (_NNDSVD_DEGENERATE, degenerate)] + list(checks)
-        self._flags = [msg for msg, flag in pairs if flag is not None]
-        device_arrays = list(device_arrays) + [(flag != 0).to(torch.uint8).reshape(1)
-                                               for _, flag in pairs if flag is not None]
+        # device flags travel with the results: each (message, flag) of `checks`; the first one set is raised
+        self._flags = [msg for msg, _ in checks]
+        device_arrays = list(device_arrays) + [(flag != 0).to(torch.uint8).reshape(1) for _, flag in checks]
         for t in device_arrays:
             t = t.contiguous()
             buf = _pinned_take(torch, int(t.numel()) * t.element_size())
@@ -237,6 +236,160 @@ def _assemble(ranks, seeds, n, m, Wall, Hall, n_iter, err, vafs) -> NMFBatchResu
     return NMFBatchResult(ranks, seeds, Ws, Hs, n_iter, err, vafs)
 
 
+# ---- what the NMF entries share: argument checks, X on the device, the initial factors, the launch outputs, the end
+def _host_x(X):
+    """(X as a float64 (B, n, m) numpy stack, or None for a CUDA X; the (B, n, m) shape).  Touches no device."""
+    import torch
+
+    if isinstance(X, torch.Tensor) and X.is_cuda:
+        Xh, shape = None, tuple(X.shape) if X.ndim == 3 else (1,) + tuple(X.shape)
+    else:
+        Xh = X.detach().to("cpu", torch.float64).numpy() if isinstance(X, torch.Tensor) else np.asarray(X, dtype=np.float64)
+        Xh = Xh[None] if Xh.ndim == 2 else Xh
+        shape = Xh.shape
+    if len(shape) != 3 or 0 in shape:
+        raise ValueError("X must be a non-empty (n, m) matrix or a (B, n, m) stack")
+    return Xh, shape
+
+
+def _problem_arrays(ranks, seeds, x_index, shape, regime, max_iter, tol):
+    """ranks (int32), seeds (int64, -1 where none is given) and x_index (int32) of a batch on an X of `shape` (B, n, m),
+    after the argument checks every NMF entry shares.  Touches no device."""
+    if regime not in (None, "resident", "stream"):
+        raise ValueError(f"regime must be None, 'resident' or 'stream', not {regime!r}")
+    if int(max_iter) < 0 or not float(tol) >= 0:
+        raise ValueError("max_iter and tol must be non-negative")
+    B, _, m = shape
+    ranks = np.ascontiguousarray(ranks, dtype=np.int32)
+    P = len(ranks)
+    xi = np.zeros(P, dtype=np.int32) if x_index is None else np.ascontiguousarray(x_index, dtype=np.int32)
+    seeds = np.full(P, -1, dtype=np.int64) if seeds is None else np.ascontiguousarray(seeds, dtype=np.int64)
+    if P < 1 or xi.shape != (P,) or len(seeds) != P or xi.min() < 0 or xi.max() >= B:
+        raise ValueError("ranks, seeds and x_index must have one entry per problem, and x_index must name a matrix of X")
+    if ranks.min() < 1 or ranks.max() > 16 or m > 64:
+        raise ValueError(f"ranks must be in 1..16 and X may have at most 64 columns (ranks {ranks.min()}..{ranks.max()}, "
+                         f"{m} columns)")
+    return ranks, seeds, xi
+
+
+def _check_init(init, ranks, seeds, shape, names=("nndsvd", "nndsvda", "random"), values=False):
+    """Checks `init`: a name of `names`, or one (W, H) pair per problem of the problem's shapes - with values, also
+    finite, non-negative and not all zero, as scikit-learn's _check_init.  Touches no device."""
+    _, n, m = shape
+    if isinstance(init, str):
+        if init not in names:
+            raise ValueError(f"init must be {', '.join(map(repr, names))} or (W, H) pairs, not {init!r}")
+        if init == "random" and (seeds < 0).any():
+            raise ValueError("init='random' needs a non-negative seed per problem")
+        if init != "random" and int(ranks.max()) > min(n, m):
+            raise ValueError(f"init = '{init}' can only be used when n_components <= min(n_samples, n_features)")
+        return
+    if len(init) != len(ranks):
+        raise ValueError("init must give one (W, H) pair per problem")
+    for p, (W0, H0) in enumerate(init):
+        if np.shape(W0) != (n, ranks[p]) or np.shape(H0) != (ranks[p], m):
+            raise ValueError(f"init pair {p} must have shapes {(n, int(ranks[p]))} and {(int(ranks[p]), m)}")
+        for A, whom in ((H0, "NMF (input H)"), (W0, "NMF (input W)")) if values else ():  # sklearn's order: H first
+            A = np.asarray(A, dtype=np.float64)
+            if not np.isfinite(A).all():
+                raise ValueError(f"Input contains NaN or infinity (init pair {p}, {whom})")
+            if (A < 0).any():
+                raise ValueError(f"Negative values in data passed to {whom}")
+            if A.max() == 0:
+                raise ValueError(f"Array passed to {whom} is full of zeros.")
+
+
+def _check_x(A, checks, defer=False):
+    """Raises the message of the first (message, test) of `checks` whose elementwise test holds somewhere in A (a numpy
+    or CUDA stack).  defer: returns the (message, device flag) pairs instead, for PendingNMF to raise - a deferred run
+    does not wait for the answer here (it would wait for everything queued before it, the previous trial's
+    factorisation included)."""
+    if defer:
+        return [(msg, test(A).any()) for msg, test in checks]
+    for msg, test in checks:
+        if bool(test(A).any()):
+            raise ValueError(msg)
+    return []
+
+
+def _cuda_lib(entry):
+    import torch
+
+    lib = nat.lib()
+    if not torch.cuda.is_available():
+        raise nat.NativeError(f"{entry} needs a CUDA device; there is no CPU fallback")
+    return lib
+
+
+def _device_x(torch, X, Xh, strided, device=None, host_dtype=np.float64):
+    """X as a (B, n, m) stack on the device.  A host X goes up row-major in host_dtype, to `device` (None: the current
+    one).  A CUDA X stays on its device, in float64: with `strided` (the kernel reads X through its strides) a view is
+    read in place - unless it is a stack whose matrices are not n * m apart, since the problem table addresses matrix b
+    at b * n * m - and otherwise it becomes row-major."""
+    if Xh is not None:
+        dev = torch.device(device if device is not None else f"cuda:{torch.cuda.current_device()}")
+        return torch.from_numpy(np.ascontiguousarray(Xh, dtype=host_dtype)).to(dev)
+    dX = X.detach().to(torch.float64)
+    dX = dX[None] if dX.ndim == 2 else dX
+    B, n, m = dX.shape
+    if not strided or (B > 1 and dX.stride(0) != n * m):
+        dX = dX.contiguous()
+    return dX
+
+
+def _init_scale(torch, dX, Xh, d_ranks, d_xi):
+    """sqrt(X.mean() / k) of every problem, on the device: the mean numpy takes on the host for a host X (what
+    scikit-learn computes), the mean of the row-major copy for a CUDA X (the same, bit for bit, whatever its layout)."""
+    if Xh is not None:
+        means = torch.from_numpy(np.array([Xh[b].mean() for b in range(len(Xh))])).to(dX.device)
+    else:
+        means = dX.contiguous().mean(dim=(1, 2))
+    return torch.sqrt(means[d_xi] / d_ranks)
+
+
+def _initial_factors(torch, lib, init, dX, Xh, ranks, seeds, xi, stream):
+    """The packed initial W and H (fp64, on X's device), the tensors that must outlive the launch and the (message,
+    device flag) checks of the init: "random" (scikit-learn's draws for seeds[p] times sqrt(X.mean() / k)), "nndsvd" /
+    "nndsvda" (computed on the device from an exact SVD, one per matrix of the stack) or one (W, H) pair per problem."""
+    _, n, m = dX.shape
+    dev = dX.device
+    if not isinstance(init, str):
+        dW = torch.from_numpy(np.concatenate([np.asarray(w, dtype=np.float64).ravel() for w, _ in init])).to(dev)
+        dH = torch.from_numpy(np.concatenate([np.asarray(h, dtype=np.float64).ravel() for _, h in init])).to(dev)
+        return dW, dH, [], []
+    table, kmax, d_ranks, d_xi, w_problem, h_problem = _batch_plan(torch, lib, n, m, ranks, xi, dev)
+    if init == "random":
+        unit_w, unit_h = _batch_draws(torch, n, m, ranks, seeds, dev)
+        avg = _init_scale(torch, dX, Xh, d_ranks, d_xi)
+        return unit_w * avg[w_problem], unit_h * avg[h_problem], [], []
+    dXc = dX.contiguous()  # the SVD reads row-major matrices
+    dW = torch.empty(int(ranks.astype(np.int64).sum()) * n, dtype=torch.float64, device=dev)
+    dH = torch.empty(int(ranks.astype(np.int64).sum()) * m, dtype=torch.float64, device=dev)
+    work = torch.empty(int(lib.ms_nndsvd_workspace_bytes(m, len(dX))), dtype=torch.uint8, device=dev)
+    status = torch.empty(1, dtype=torch.int32, device=dev)
+    nat.check(lib.ms_nndsvd_init(dXc.data_ptr(), n, m, len(dX), table.data_ptr(), len(ranks), kmax,
+                                 int(init == "nndsvda"), work.data_ptr(), dW.data_ptr(), dH.data_ptr(),
+                                 status.data_ptr(), ctypes.c_void_p(stream.cuda_stream)), "ms_nndsvd_init")
+    return dW, dH, [dXc, work], [(_NNDSVD_DEGENERATE, status)]
+
+
+def _launch_outputs(torch, dev, regime, n, max_rows, P, m, dtype):
+    """(resident, n_iter, err, vaf): the regime - resident when n fits the resident kernel's shared memory (regime None),
+    or as asked - and the per-problem outputs of the launch."""
+    resident = n <= max_rows if regime is None else regime == "resident"
+    return (resident, torch.empty(P, dtype=torch.int32, device=dev), torch.empty(P, dtype=dtype, device=dev),
+            torch.empty((P, m + 1), dtype=dtype, device=dev))
+
+
+def _finish(torch, stream, ranks, seeds, n, m, device_arrays, keep, checks, defer):
+    """The end of every entry: the PendingNMF of the queued launch under defer, else its result."""
+    pending = PendingNMF(torch, stream, ranks, seeds, n, m, device_arrays, keep, checks)
+    return pending if defer else pending.result()
+
+
+_NEGATIVE_CHECK = ((_NEGATIVE_X, lambda A: A < 0),)
+
+
 def nmf_mu_batched(X, ranks: Sequence[int], seeds: Sequence[int], max_iter: int = 200, tol: float = 1e-4,
                    check_every: int = 10, init=None, device=None, x_index: Optional[Sequence[int]] = None,
                    regime: Optional[str] = None, defer: bool = False) -> Union[NMFBatchResult, PendingNMF]:
@@ -250,66 +403,25 @@ def nmf_mu_batched(X, ranks: Sequence[int], seeds: Sequence[int], max_iter: int 
     instead of the seeds.  regime: None (by size), "resident" or "stream"."""
     import torch
 
-    lib = nat.lib()
-    if not torch.cuda.is_available():
-        raise nat.NativeError("nmf_mu_batched needs a CUDA device; there is no CPU fallback")
-    on_device = isinstance(X, torch.Tensor) and X.is_cuda
-    if on_device:
-        dev = X.device
-        dX64 = X.detach().to(torch.float64)
-        if dX64.ndim == 2:
-            dX64 = dX64[None]
-        shape = tuple(dX64.shape)
-    else:
-        dev = torch.device(device if device is not None else f"cuda:{torch.cuda.current_device()}")
-        Xh = X.detach().to("cpu", torch.float64).numpy() if isinstance(X, torch.Tensor) else np.asarray(X, dtype=np.float64)
-        if Xh.ndim == 2:
-            Xh = Xh[None]
-        shape = Xh.shape
-    if len(shape) != 3 or 0 in shape:
-        raise ValueError("X must be a non-empty (n, m) matrix or a (B, n, m) stack")
-    # a deferred run on device data does not wait for the answer here (it would wait for everything queued before it,
-    # the previous trial's factorisation included): the flag travels with the results and `.result()` raises
-    negative = (dX64 < 0).any() if on_device and defer else None
-    if negative is None and (bool((dX64 < 0).any()) if on_device else bool((Xh < 0).any())):
-        raise ValueError(_NEGATIVE_X)
-    B, n, m = shape
-    ranks = np.ascontiguousarray(ranks, dtype=np.int32)
-    seeds = np.ascontiguousarray(seeds, dtype=np.int64)
+    Xh, shape = _host_x(X)
+    ranks, seeds, xi = _problem_arrays(ranks, seeds, x_index, shape, regime, max_iter, tol)
+    how = "random" if init is None else init
+    _check_init(how, ranks, seeds, shape, names=("random",))
+    checks = _check_x(Xh, _NEGATIVE_CHECK) if Xh is not None else []
+    lib = _cuda_lib("nmf_mu_batched")
+    _, n, m = shape
     P = len(ranks)
-    xi = np.zeros(P, dtype=np.int32) if x_index is None else np.ascontiguousarray(x_index, dtype=np.int32)
-    if P < 1 or len(xi) != P or len(seeds) != P or xi.min() < 0 or xi.max() >= B:
-        raise ValueError("ranks, seeds and x_index must have one entry per problem")
-    if ranks.min() < 1:
-        raise ValueError("ranks must be positive")
-    kmax = int(ranks.max())
-    # short signals stay resident in shared memory; long ones stream from HBM every iteration
-    resident = (n <= int(lib.ms_nmf_resident_max_rows(m, kmax))) if regime is None else (regime == "resident")
+    dX = _device_x(torch, X, Xh, strided=False, device=device, host_dtype=np.float32)  # float64 for a CUDA X
+    dev = dX.device
     stream = torch.cuda.current_stream(dev)
     with torch.cuda.device(dev):
-        if on_device:
-            dX = dX64.to(torch.float32).contiguous()
-        else:
-            dX = torch.from_numpy(np.ascontiguousarray(Xh, dtype=np.float32)).to(dev)
-        if init is not None:
-            dW = torch.from_numpy(np.concatenate(
-                [np.ascontiguousarray(init[p][0], dtype=np.float32).ravel() for p in range(P)])).to(dev)
-            dH = torch.from_numpy(np.concatenate(
-                [np.ascontiguousarray(init[p][1], dtype=np.float32).ravel() for p in range(P)])).to(dev)
-        else:
-            # sklearn's init="random": float64 draws scaled by sqrt(X.mean() / k), then the kernel's fp32
-            unit_w, unit_h = _batch_draws(torch, n, m, ranks, seeds, dev)
-            if on_device:
-                means = dX64.mean(dim=(1, 2))
-            else:
-                means = torch.from_numpy(np.array([Xh[b].mean() for b in range(B)])).to(dev)
-            _, _, d_ranks, d_xi, w_problem, h_problem = _batch_plan(torch, lib, n, m, ranks, xi, dev)
-            avg = torch.sqrt(means[d_xi] / d_ranks)
-            dW = (unit_w * avg[w_problem]).to(torch.float32)
-            dH = (unit_h * avg[h_problem]).to(torch.float32)
-        d_iter = torch.empty(P, dtype=torch.int32, device=dev)
-        d_err = torch.empty(P, dtype=torch.float32, device=dev)
-        d_vaf = torch.empty((P, m + 1), dtype=torch.float32, device=dev)
+        if Xh is None:
+            checks = _check_x(dX, _NEGATIVE_CHECK, defer)
+        # sklearn's init in float64, then the kernel's fp32
+        dW, dH = (t.to(torch.float32) for t in _initial_factors(torch, lib, how, dX, Xh, ranks, seeds, xi, stream)[:2])
+        dX = dX.to(torch.float32)
+        max_rows = int(lib.ms_nmf_resident_max_rows(m, int(ranks.max())))
+        resident, d_iter, d_err, d_vaf = _launch_outputs(torch, dev, regime, n, max_rows, P, m, torch.float32)
         if resident:
             # the problem table lives on the device for as long as the sweep is repeated: the launch copies nothing
             # and waits for nothing
@@ -334,11 +446,7 @@ def nmf_mu_batched(X, ranks: Sequence[int], seeds: Sequence[int], max_iter: int 
                 ),
                 "ms_nmf_mu_stream",
             )
-        if defer:
-            return PendingNMF(torch, stream, ranks, seeds, n, m, [dW, dH, d_iter, d_err, d_vaf], [dX, work], negative)
-        Wall, Hall = dW.cpu().numpy(), dH.cpu().numpy()
-        n_iter, err, vafs = d_iter.cpu().numpy(), d_err.cpu().numpy(), d_vaf.cpu().numpy()
-    return _assemble(ranks, seeds, n, m, Wall, Hall, n_iter, err, vafs)
+        return _finish(torch, stream, ranks, seeds, n, m, [dW, dH, d_iter, d_err, d_vaf], [dX, work], checks, defer)
 
 
 def nmf_cd_batched(X, ranks: Sequence[int], init="nndsvda", seeds: Optional[Sequence[int]] = None, max_iter: int = 200,
@@ -352,70 +460,24 @@ def nmf_cd_batched(X, ranks: Sequence[int], init="nndsvda", seeds: Optional[Sequ
     (W, H) pair per problem.  The factors of the result are fp64; its seeds are -1 where no seed was given."""
     import torch
 
-    lib = nat.lib()
-    if not torch.cuda.is_available():
-        raise nat.NativeError("nmf_cd_batched needs a CUDA device; there is no CPU fallback")
-    if isinstance(X, torch.Tensor) and X.is_cuda:
-        dev = X.device
-        dX = X.detach().to(torch.float64)
-    else:
-        dev = torch.device(f"cuda:{torch.cuda.current_device()}")
-        Xh = X.detach().to("cpu", torch.float64).numpy() if isinstance(X, torch.Tensor) else np.asarray(X, dtype=np.float64)
-        dX = torch.from_numpy(np.ascontiguousarray(Xh)).to(dev)
-    if dX.ndim == 2:
-        dX = dX[None]
-    if dX.ndim != 3 or 0 in dX.shape:
-        raise ValueError("X must be a non-empty (n, m) matrix or a (B, n, m) stack")
-    dX = dX.contiguous()
-    B, n, m = dX.shape
-    # as for nmf_mu_batched: a deferred run does not wait here, the flag travels with the results
-    negative = (dX < 0).any()
-    if not defer and bool(negative):
-        raise ValueError(_NEGATIVE_X)
-    ranks = np.ascontiguousarray(ranks, dtype=np.int32)
+    Xh, shape = _host_x(X)
+    ranks, seeds, xi = _problem_arrays(ranks, seeds, x_index, shape, regime, max_iter, tol)
+    _check_init(init, ranks, seeds, shape)
+    checks = _check_x(Xh, _NEGATIVE_CHECK) if Xh is not None else []
+    lib = _cuda_lib("nmf_cd_batched")
+    _, n, m = shape
     P = len(ranks)
-    xi = np.zeros(P, dtype=np.int32) if x_index is None else np.ascontiguousarray(x_index, dtype=np.int32)
-    seeds = np.full(P, -1, dtype=np.int64) if seeds is None else np.ascontiguousarray(seeds, dtype=np.int64)
-    if P < 1 or len(xi) != P or len(seeds) != P or xi.min() < 0 or xi.max() >= B:
-        raise ValueError("ranks, seeds and x_index must have one entry per problem")
-    if ranks.min() < 1:
-        raise ValueError("ranks must be positive")
-    named = isinstance(init, str)
-    if named and init not in ("nndsvd", "nndsvda", "random"):
-        raise ValueError(f"init must be 'nndsvd', 'nndsvda', 'random' or (W, H) pairs, not {init!r}")
-    if init == "random" and (seeds < 0).any():
-        raise ValueError("init='random' needs a non-negative seed per problem")
-    if named and init != "random" and int(ranks.max()) > min(n, m):
-        raise ValueError(f"init = '{init}' can only be used when n_components <= min(n_samples, n_features)")
-    table, kmax, d_ranks, d_xi, w_problem, h_problem = _batch_plan(torch, lib, n, m, ranks, xi, dev)
+    dX = _device_x(torch, X, Xh, strided=False)
+    dev = dX.device
+    table, kmax = _batch_plan(torch, lib, n, m, ranks, xi, dev)[:2]
     stream = torch.cuda.current_stream(dev)
-    keep, status = [dX], None
     with torch.cuda.device(dev):
-        if init == "random":
-            unit_w, unit_h = _batch_draws(torch, n, m, ranks, seeds, dev)
-            avg = torch.sqrt(dX.mean(dim=(1, 2))[d_xi] / d_ranks)
-            dW, dH = unit_w * avg[w_problem], unit_h * avg[h_problem]
-        elif named:
-            dW = torch.empty(int(ranks.astype(np.int64).sum()) * n, dtype=torch.float64, device=dev)
-            dH = torch.empty(int(ranks.astype(np.int64).sum()) * m, dtype=torch.float64, device=dev)
-            work = torch.empty(int(lib.ms_nndsvd_workspace_bytes(m, B)), dtype=torch.uint8, device=dev)
-            status = torch.empty(1, dtype=torch.int32, device=dev)
-            nat.check(lib.ms_nndsvd_init(dX.data_ptr(), n, m, B, table.data_ptr(), P, kmax, int(init == "nndsvda"),
-                                         work.data_ptr(), dW.data_ptr(), dH.data_ptr(), status.data_ptr(),
-                                         ctypes.c_void_p(stream.cuda_stream)), "ms_nndsvd_init")
-            keep.append(work)
-        else:
-            if len(init) != P:
-                raise ValueError("init must give one (W, H) pair per problem")
-            for p, (W0, H0) in enumerate(init):
-                if np.shape(W0) != (n, ranks[p]) or np.shape(H0) != (ranks[p], m):
-                    raise ValueError(f"init pair {p} must have shapes {(n, int(ranks[p]))} and {(int(ranks[p]), m)}")
-            dW = torch.from_numpy(np.concatenate([np.asarray(w, dtype=np.float64).ravel() for w, _ in init])).to(dev)
-            dH = torch.from_numpy(np.concatenate([np.asarray(h, dtype=np.float64).ravel() for _, h in init])).to(dev)
-        d_iter = torch.empty(P, dtype=torch.int32, device=dev)
-        d_err = torch.empty(P, dtype=torch.float64, device=dev)
-        d_vaf = torch.empty((P, m + 1), dtype=torch.float64, device=dev)
-        resident = (n <= int(lib.ms_nmf_cd_resident_max_rows(m, kmax))) if regime is None else (regime == "resident")
+        if Xh is None:
+            checks = _check_x(dX, _NEGATIVE_CHECK, defer)
+        dW, dH, keep, init_checks = _initial_factors(torch, lib, init, dX, Xh, ranks, seeds, xi, stream)
+        max_rows = int(lib.ms_nmf_cd_resident_max_rows(m, kmax))
+        resident, d_iter, d_err, d_vaf = _launch_outputs(torch, dev, regime, n, max_rows, P, m, torch.float64)
+        keep.append(dX)
         if resident:
             nat.check(lib.ms_nmf_cd_batched_planned(
                 dX.data_ptr(), n, m, table.data_ptr(), P, kmax, dW.data_ptr(), dH.data_ptr(), int(max_iter), float(tol),
@@ -428,13 +490,8 @@ def nmf_cd_batched(X, ranks: Sequence[int], init="nndsvda", seeds: Optional[Sequ
                 dX.data_ptr(), n, m, table.data_ptr(), P, kmax, dW.data_ptr(), dH.data_ptr(), int(max_iter), float(tol),
                 work.data_ptr(), d_iter.data_ptr(), d_err.data_ptr(), d_vaf.data_ptr(), ctypes.c_void_p(stream.cuda_stream)),
                 "ms_nmf_cd_stream")
-        if defer:
-            return PendingNMF(torch, stream, ranks, seeds, n, m, [dW, dH, d_iter, d_err, d_vaf], keep, negative, status)
-        if status is not None and int(status.item()) != 0:
-            raise ValueError(_NNDSVD_DEGENERATE)
-        Wall, Hall = dW.cpu().numpy(), dH.cpu().numpy()
-        n_iter, err, vafs = d_iter.cpu().numpy(), d_err.cpu().numpy(), d_vaf.cpu().numpy()
-    return _assemble(ranks, seeds, n, m, Wall, Hall, n_iter, err, vafs)
+        return _finish(torch, stream, ranks, seeds, n, m, [dW, dH, d_iter, d_err, d_vaf], keep, checks + init_checks,
+                       defer)
 
 
 _BETA_NAMES = {"frobenius": 2.0, "kullback-leibler": 1.0, "itakura-saito": 0.0}
@@ -464,6 +521,11 @@ def _beta_solver_error(solver, beta_loss) -> ValueError:
     return _BetaLossSolverError(f"Invalid beta_loss parameter: solver {solver!r} does not handle beta_loss = {beta_loss!r}")
 
 
+def _zeros_check(beta):
+    """sklearn's refusal of zeros in X under beta_loss <= 0 (after its other checks of X)."""
+    return ((_BETA_ZEROS, lambda A: A == 0),) if beta <= 0 else ()
+
+
 def nmf_beta_batched(X, ranks: Sequence[int], beta_loss, init="nndsvda", seeds: Optional[Sequence[int]] = None,
                      max_iter: int = 200, tol: float = 1e-4, x_index: Optional[Sequence[int]] = None,
                      regime: Optional[str] = None, defer: bool = False) -> Union[NMFBatchResult, PendingNMF]:
@@ -480,125 +542,33 @@ def nmf_beta_batched(X, ranks: Sequence[int], beta_loss, init="nndsvda", seeds: 
     beta = _beta_to_float(beta_loss)
     if beta == 2.0:
         raise ValueError("beta_loss = 2 (Frobenius) runs on nmf_mu_batched or nmf_cd_batched")
-    if regime not in (None, "resident", "stream"):
-        raise ValueError(f"regime must be None, 'resident' or 'stream', not {regime!r}")
-    if int(max_iter) < 0 or not float(tol) >= 0:
-        raise ValueError("max_iter and tol must be non-negative")
-    on_device = isinstance(X, torch.Tensor) and X.is_cuda
-    if not on_device:
-        Xh = X.detach().to("cpu", torch.float64).numpy() if isinstance(X, torch.Tensor) else np.asarray(X, dtype=np.float64)
-        Xh = Xh[None] if Xh.ndim == 2 else Xh
-        shape = Xh.shape
-    else:
-        shape = tuple(X.shape) if X.ndim == 3 else (1,) + tuple(X.shape)
-    if len(shape) != 3 or 0 in shape:
-        raise ValueError("X must be a non-empty (n, m) matrix or a (B, n, m) stack")
-    B, n, m = shape
-    ranks = np.ascontiguousarray(ranks, dtype=np.int32)
-    P = len(ranks)
-    xi = np.zeros(P, dtype=np.int32) if x_index is None else np.ascontiguousarray(x_index, dtype=np.int32)
-    seeds = np.full(P, -1, dtype=np.int64) if seeds is None else np.ascontiguousarray(seeds, dtype=np.int64)
-    if P < 1 or len(xi) != P or len(seeds) != P or xi.min() < 0 or xi.max() >= B:
-        raise ValueError("ranks, seeds and x_index must have one entry per problem")
-    if ranks.min() < 1 or ranks.max() > 16 or m > 64:
-        raise ValueError(f"ranks must be in 1..16 and X may have at most 64 columns (ranks {ranks.min()}..{ranks.max()}, "
-                         f"{m} columns)")
-    named = isinstance(init, str)
-    if named and init not in ("nndsvd", "nndsvda", "random"):
-        raise ValueError(f"init must be 'nndsvd', 'nndsvda', 'random' or (W, H) pairs, not {init!r}")
-    if init == "random" and (seeds < 0).any():
-        raise ValueError("init='random' needs a non-negative seed per problem")
-    if named and init != "random" and int(ranks.max()) > min(n, m):
-        raise ValueError(f"init = '{init}' can only be used when n_components <= min(n_samples, n_features)")
-    if not named:
-        if len(init) != P:
-            raise ValueError("init must give one (W, H) pair per problem")
-        for p, (W0, H0) in enumerate(init):
-            if np.shape(W0) != (n, ranks[p]) or np.shape(H0) != (ranks[p], m):
-                raise ValueError(f"init pair {p} must have shapes {(n, int(ranks[p]))} and {(int(ranks[p]), m)}")
-            for A, whom in ((H0, "NMF (input H)"), (W0, "NMF (input W)")):  # sklearn's _check_init, H first
-                A = np.asarray(A, dtype=np.float64)
-                if not np.isfinite(A).all():
-                    raise ValueError(f"Input contains NaN or infinity (init pair {p}, {whom})")
-                if (A < 0).any():
-                    raise ValueError(f"Negative values in data passed to {whom}")
-                if A.max() == 0:
-                    raise ValueError(f"Array passed to {whom} is full of zeros.")
-    if not on_device:  # sklearn's order: negative values first, then zeros under beta_loss <= 0
-        if (Xh < 0).any():
-            raise ValueError(_NEGATIVE_X)
-        if beta <= 0 and Xh.min() == 0:
-            raise ValueError(_BETA_ZEROS)
-    lib = nat.lib()
-    if not torch.cuda.is_available():
-        raise nat.NativeError("nmf_beta_batched needs a CUDA device; there is no CPU fallback")
-    negative, checks = None, ()
-    if on_device:
-        dev = X.device
-        dX = X.detach().to(torch.float64)
-        dX = dX[None] if dX.ndim == 2 else dX
-        if B > 1 and dX.stride(0) != n * m:  # the problem table addresses matrix b at b * n * m
-            dX = dX.contiguous()
-        # as for nmf_mu_batched: a deferred run does not wait here, the flags travel with the results
-        negative = (dX < 0).any()
-        zeros = (dX == 0).any() if beta <= 0 else None
-        if not defer:
-            if bool(negative):
-                raise ValueError(_NEGATIVE_X)
-            if zeros is not None and bool(zeros):
-                raise ValueError(_BETA_ZEROS)
-            negative = None
-        elif zeros is not None:
-            checks = ((_BETA_ZEROS, zeros),)
-    else:
-        dev = torch.device(f"cuda:{torch.cuda.current_device()}")
-        dX = torch.from_numpy(np.ascontiguousarray(Xh)).to(dev)
-    table, kmax, d_ranks, d_xi, w_problem, h_problem = _batch_plan(torch, lib, n, m, ranks, xi, dev)
+    Xh, shape = _host_x(X)
+    ranks, seeds, xi = _problem_arrays(ranks, seeds, x_index, shape, regime, max_iter, tol)
+    _check_init(init, ranks, seeds, shape, values=True)
+    x_checks = _NEGATIVE_CHECK + _zeros_check(beta)
+    checks = _check_x(Xh, x_checks) if Xh is not None else []
+    lib = _cuda_lib("nmf_beta_batched")
+    _, n, m = shape
+    dX = _device_x(torch, X, Xh, strided=True)
+    dev = dX.device
+    table, kmax = _batch_plan(torch, lib, n, m, ranks, xi, dev)[:2]
     stream = torch.cuda.current_stream(dev)
-    keep, status = [dX], None
     with torch.cuda.device(dev):
-        if init == "random":
-            unit_w, unit_h = _batch_draws(torch, n, m, ranks, seeds, dev)
-            if on_device:
-                means = dX.contiguous().mean(dim=(1, 2))
-            else:  # sklearn's X.mean(), on the host as sklearn computes it: the same init, bit for bit
-                means = torch.from_numpy(np.array([Xh[b].mean() for b in range(B)])).to(dev)
-            avg = torch.sqrt(means[d_xi] / d_ranks)
-            dW, dH = unit_w * avg[w_problem], unit_h * avg[h_problem]
-        elif named:
-            dXc = dX.contiguous()  # the SVD reads row-major matrices
-            dW = torch.empty(int(ranks.astype(np.int64).sum()) * n, dtype=torch.float64, device=dev)
-            dH = torch.empty(int(ranks.astype(np.int64).sum()) * m, dtype=torch.float64, device=dev)
-            work = torch.empty(int(lib.ms_nndsvd_workspace_bytes(m, B)), dtype=torch.uint8, device=dev)
-            status = torch.empty(1, dtype=torch.int32, device=dev)
-            nat.check(lib.ms_nndsvd_init(dXc.data_ptr(), n, m, B, table.data_ptr(), P, kmax, int(init == "nndsvda"),
-                                         work.data_ptr(), dW.data_ptr(), dH.data_ptr(), status.data_ptr(),
-                                         ctypes.c_void_p(stream.cuda_stream)), "ms_nndsvd_init")
-            keep += [dXc, work]
-        else:
-            dW = torch.from_numpy(np.concatenate([np.asarray(w, dtype=np.float64).ravel() for w, _ in init])).to(dev)
-            dH = torch.from_numpy(np.concatenate([np.asarray(h, dtype=np.float64).ravel() for _, h in init])).to(dev)
-        d_iter, d_err, d_vaf, work = _beta_launch(torch, lib, dX, n, m, table, P, kmax, dW, dH, beta, 1, max_iter, tol,
-                                                  regime, stream)
-        keep.append(work)
-        if defer:
-            return PendingNMF(torch, stream, ranks, seeds, n, m, [dW, dH, d_iter, d_err, d_vaf], keep, negative, status,
-                              checks=checks)
-        if status is not None and int(status.item()) != 0:
-            raise ValueError(_NNDSVD_DEGENERATE)
-        Wall, Hall = dW.cpu().numpy(), dH.cpu().numpy()
-        n_iter, err, vafs = d_iter.cpu().numpy(), d_err.cpu().numpy(), d_vaf.cpu().numpy()
-    return _assemble(ranks, seeds, n, m, Wall, Hall, n_iter, err, vafs)
+        if Xh is None:
+            checks = _check_x(dX, x_checks, defer)
+        dW, dH, keep, init_checks = _initial_factors(torch, lib, init, dX, Xh, ranks, seeds, xi, stream)
+        d_iter, d_err, d_vaf, work = _beta_launch(torch, lib, dX, n, m, table, len(ranks), kmax, dW, dH, beta, 1,
+                                                  max_iter, tol, regime, stream)
+        return _finish(torch, stream, ranks, seeds, n, m, [dW, dH, d_iter, d_err, d_vaf], keep + [dX, work],
+                       checks + init_checks, defer)
 
 
 def _beta_launch(torch, lib, dX, n, m, table, P, kmax, dW, dH, beta, update_H, max_iter, tol, regime, stream):
     """Queues ms_nmf_beta on `stream` (regime None: resident when n fits shared memory); returns the device outputs
     and the workspace, which must outlive the launch."""
     dev = dX.device
-    resident = (n <= int(lib.ms_nmf_beta_resident_max_rows(m, kmax))) if regime is None else (regime == "resident")
-    d_iter = torch.empty(P, dtype=torch.int32, device=dev)
-    d_err = torch.empty(P, dtype=torch.float64, device=dev)
-    d_vaf = torch.empty((P, m + 1), dtype=torch.float64, device=dev)
+    max_rows = int(lib.ms_nmf_beta_resident_max_rows(m, kmax))
+    resident, d_iter, d_err, d_vaf = _launch_outputs(torch, dev, regime, n, max_rows, P, m, torch.float64)
     work = torch.empty(0 if resident else int(lib.ms_nmf_beta_workspace_bytes(n, m, P, kmax)), dtype=torch.uint8,
                        device=dev)
     nat.check(lib.ms_nmf_beta(
@@ -614,26 +584,18 @@ _TRANSFORM_NAN = "Input X contains NaN."
 _TRANSFORM_INF = "Input X contains infinity or a value too large for dtype('float64')."
 _TRANSFORM_NEGATIVE = "Negative values in data passed to X in NMF."
 _SOLVER_CODES = {"cd": 0, "mu": 1}
+# the input checks of sklearn's transform, in its order: NaN, infinity, negative values
+_TRANSFORM_CHECKS = ((_TRANSFORM_NAN, lambda A: A != A), (_TRANSFORM_INF, lambda A: abs(A) == np.inf),
+                     (_TRANSFORM_NEGATIVE, lambda A: A < 0))
 
 
-def _check_transform_host(Xh: np.ndarray):
-    """The input checks of sklearn's transform, in its order: NaN, infinity, negative values."""
-    if not np.isfinite(Xh).all():
-        raise ValueError(_TRANSFORM_NAN if np.isnan(Xh).any() else _TRANSFORM_INF)
-    if (Xh < 0).any():
-        raise ValueError(_TRANSFORM_NEGATIVE)
-
-
-def _transform_args(X, H, x_index, solver, max_iter, tol, regime, beta_loss="frobenius"):
-    """Validates what nmf_transform_batched is given, without touching a device; returns (H list, m, x_index)."""
+def _transform_args(shape, H, solver, beta_loss="frobenius"):
+    """Validates the synergies nmf_transform_batched is given for an X of `shape` (B, n, m), without touching a device;
+    returns (H list, ranks)."""
     if solver not in _SOLVER_CODES:
         raise ValueError(f"solver must be 'cd' or 'mu', not {solver!r}")
     if _beta_to_float(beta_loss) != 2.0 and solver != "mu":
         raise _beta_solver_error(solver, beta_loss)
-    if regime not in (None, "resident", "stream"):
-        raise ValueError(f"regime must be None, 'resident' or 'stream', not {regime!r}")
-    if int(max_iter) < 0 or not float(tol) >= 0:
-        raise ValueError("max_iter and tol must be non-negative")
     Hs = [np.ascontiguousarray(h, dtype=np.float64) for h in H]
     if not Hs:
         raise ValueError("H must give one (k, m) matrix per problem")
@@ -644,17 +606,9 @@ def _transform_args(X, H, x_index, solver, max_iter, tol, regime, beta_loss="fro
                              f"problem, not {h.shape}")
         if not np.isfinite(h).all() or (h < 0).any():
             raise ValueError(f"H[{p}] must be finite and non-negative")
-    xi = np.zeros(len(Hs), dtype=np.int32) if x_index is None else np.ascontiguousarray(x_index, dtype=np.int32)
-    if xi.shape != (len(Hs),) or xi.min() < 0:
-        raise ValueError("x_index must have one non-negative entry per matrix of H")
-    shape = tuple(X.shape)
-    if len(shape) not in (2, 3) or 0 in shape:
-        raise ValueError("X must be a non-empty (n, m) matrix or a (B, n, m) stack")
     if shape[-1] != m:
         raise ValueError(f"X has {shape[-1]} features, but H has {m}")
-    if xi.max() >= (shape[0] if len(shape) == 3 else 1):
-        raise ValueError("x_index names a matrix X does not have")
-    return Hs, m, xi
+    return Hs, [h.shape[0] for h in Hs]
 
 
 def nmf_transform_batched(X, H: Sequence, x_index: Optional[Sequence[int]] = None, solver: str = "cd",
@@ -677,71 +631,35 @@ def nmf_transform_batched(X, H: Sequence, x_index: Optional[Sequence[int]] = Non
 def _nmf_transform(X, H, x_index, solver, max_iter, tol, regime, defer, device_w=False, beta_loss="frobenius"):
     import torch
 
-    on_device = isinstance(X, torch.Tensor) and X.is_cuda
-    if not on_device:
-        Xh = X.detach().to("cpu", torch.float64).numpy() if isinstance(X, torch.Tensor) else np.asarray(X, dtype=np.float64)
-        X = Xh
-    Hs, m, xi = _transform_args(X, H, x_index, solver, max_iter, tol, regime, beta_loss)
+    Xh, shape = _host_x(X)
+    Hs, ranks = _transform_args(shape, H, solver, beta_loss)
+    ranks, seeds, xi = _problem_arrays(ranks, None, x_index, shape, regime, max_iter, tol)
     beta = _beta_to_float(beta_loss)
-    if not on_device:
-        _check_transform_host(X)
-        if beta <= 0 and X.min() == 0:
-            raise ValueError(_BETA_ZEROS)
-    lib = nat.lib()
-    if not torch.cuda.is_available():
-        raise nat.NativeError("nmf_transform_batched needs a CUDA device; there is no CPU fallback")
-    ranks = np.array([h.shape[0] for h in Hs], dtype=np.int32)
+    x_checks = _TRANSFORM_CHECKS + _zeros_check(beta)
+    checks = _check_x(Xh, x_checks) if Xh is not None else []
+    lib = _cuda_lib("nmf_transform_batched")
+    _, n, m = shape
     P = len(ranks)
-    seeds = np.full(P, -1, dtype=np.int64)
-    checks = ()
-    if on_device:
-        dev = X.device
-        dX = X.detach().to(torch.float64)
-        if dX.ndim == 2:
-            dX = dX[None]
-        B, n, _ = dX.shape
-        if B > 1 and dX.stride(0) != n * m:  # the problem table addresses matrix b at b * n * m
-            dX = dX.contiguous()
-        flags = (torch.isnan(dX).any(), torch.isinf(dX).any(), (dX < 0).any())
-        checks = tuple(zip((_TRANSFORM_NAN, _TRANSFORM_INF, _TRANSFORM_NEGATIVE), flags))
-        if beta <= 0:
-            checks += ((_BETA_ZEROS, (dX == 0).any()),)
-        if not defer:
-            for msg, flag in checks:
-                if bool(flag):
-                    raise ValueError(msg)
-            checks = ()
-    else:
-        dev = torch.device(f"cuda:{torch.cuda.current_device()}")
-        Xh = X[None] if X.ndim == 2 else X
-        B, n, _ = Xh.shape
-        means = np.array([Xh[b].mean() for b in range(B)])  # sklearn's X.mean(), on the host as sklearn computes it
-        dX = torch.from_numpy(np.ascontiguousarray(Xh)).to(dev)
-    kmax = int(ranks.max())
-    resident = (n <= int(lib.ms_nmf_fixed_h_resident_max_rows(m, kmax))) if regime is None else (regime == "resident")
+    dX = _device_x(torch, X, Xh, strided=True)
+    dev = dX.device
     table, kmax, d_ranks, d_xi, w_problem, _ = _batch_plan(torch, lib, n, m, ranks, xi, dev)
     stream = torch.cuda.current_stream(dev)
-    keep = [dX]
     with torch.cuda.device(dev):
+        if Xh is None:
+            checks = _check_x(dX, x_checks, defer)
         if solver == "cd":
             dW = torch.zeros(int(ranks.astype(np.int64).sum()) * n, dtype=torch.float64, device=dev)
-        elif on_device:
-            # the mean of the row-major copy: the same W0, bit for bit, whatever the layout X comes in
-            dW = torch.sqrt(dX.contiguous().mean(dim=(1, 2))[d_xi] / d_ranks)[w_problem]
         else:
-            dW = torch.from_numpy(np.sqrt(means[xi] / ranks)).to(dev)[w_problem]
+            dW = _init_scale(torch, dX, Xh, d_ranks, d_xi)[w_problem]
         dH = torch.from_numpy(np.concatenate([h.ravel() for h in Hs])).to(dev)
         if beta != 2.0:  # the β-divergence: the same loop as the fit, H fixed
             d_iter, d_err, d_vaf, work = _beta_launch(torch, lib, dX, n, m, table, P, kmax, dW, dH, beta, 0, max_iter,
                                                       tol, regime, stream)
-            keep.append(work)
         else:
-            d_iter = torch.empty(P, dtype=torch.int32, device=dev)
-            d_err = torch.empty(P, dtype=torch.float64, device=dev)
-            d_vaf = torch.empty((P, m + 1), dtype=torch.float64, device=dev)
+            max_rows = int(lib.ms_nmf_fixed_h_resident_max_rows(m, kmax))
+            resident, d_iter, d_err, d_vaf = _launch_outputs(torch, dev, regime, n, max_rows, P, m, torch.float64)
             work = torch.empty(0 if resident else int(lib.ms_nmf_fixed_h_workspace_bytes(n, m, P, kmax)),
                                dtype=torch.uint8, device=dev)
-            keep.append(work)
             nat.check(lib.ms_nmf_fixed_h(
                 dX.data_ptr(), n, m, dX.stride(1), dX.stride(2), table.data_ptr(), P, kmax, dW.data_ptr(), dH.data_ptr(),
                 _SOLVER_CODES[solver], int(max_iter), float(tol), 0 if resident else 1,
@@ -749,11 +667,7 @@ def _nmf_transform(X, H, x_index, solver, max_iter, tol, regime, defer, device_w
                 ctypes.c_void_p(stream.cuda_stream)), "ms_nmf_fixed_h")
         if device_w:
             return dW, d_iter
-        if defer:
-            return PendingNMF(torch, stream, ranks, seeds, n, m, [dW, dH, d_iter, d_err, d_vaf], keep, checks=checks)
-        Wall = dW.cpu().numpy()
-        n_iter, err, vafs = d_iter.cpu().numpy(), d_err.cpu().numpy(), d_vaf.cpu().numpy()
-    return _assemble(ranks, seeds, n, m, Wall, np.concatenate([h.ravel() for h in Hs]), n_iter, err, vafs)
+        return _finish(torch, stream, ranks, seeds, n, m, [dW, dH, d_iter, d_err, d_vaf], [dX, work], checks, defer)
 
 
 # ---- synergy comparison -------------------------------------------------------------------------------
@@ -966,15 +880,11 @@ class NMFModel:
         if isinstance(X, torch.Tensor) and X.is_cuda:
             if X.ndim != 2:
                 raise ValueError(f"Expected 2D array, got {X.ndim}D array instead")
-            for msg, flag in zip((_TRANSFORM_NAN, _TRANSFORM_INF, _TRANSFORM_NEGATIVE),
-                                 (torch.isnan(X).any(), torch.isinf(X).any(), (X < 0).any())):
-                if bool(flag):
-                    raise ValueError(msg)
         else:
             X = np.asarray(X.to_numpy() if isinstance(X, pandas.DataFrame) else X, dtype=np.float64)
             if X.ndim != 2:
                 raise ValueError(f"Expected 2D array, got {X.ndim}D array instead")
-            _check_transform_host(X)
+        _check_x(X, _TRANSFORM_CHECKS)
         if X.shape[1] != self.n_features_in_:
             raise ValueError(f"X has {X.shape[1]} features, but NMF is expecting {self.n_features_in_} features as input.")
         W, n_iter = _nmf_transform(X, [self.components_], None, self.solver, self.max_iter, self.tol, None, False,

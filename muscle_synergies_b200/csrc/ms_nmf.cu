@@ -18,9 +18,7 @@
 //                            no HBM traffic between iterations, bound by SM issue + shared memory
 //   ms_nmf_stream_*          long signals: X and W stream from HBM once per iteration, W^T X and
 //                            W^T W reduced per CTA and accumulated with atomics (HBM-bound)
-#include <stdio.h>
-
-#include "ms_common.cuh"
+#include "ms_nmf_common.cuh"
 
 #define NMF_EPS 1.1920929e-07f
 // The quotient of an update step: one reciprocal approximation and a multiply (2 ulp) instead of the ~10 instructions of
@@ -36,15 +34,6 @@
 #ifndef NMF_MIN_CTAS
 #define NMF_MIN_CTAS 3
 #endif
-#define NMF_MAX_K 16
-#define NMF_MAX_M 64
-
-struct MsNmfProblem {
-    int k;
-    long long w_off;  // floats from d_W to this problem's W [n][k]
-    long long h_off;  // floats from d_H to this problem's H [k][m]
-    long long x_off;  // floats from d_X to this problem's X [n][m]
-};
 
 __device__ __forceinline__ float ms_block_sum(float v, float* s_red) {
     for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
@@ -54,20 +43,6 @@ __device__ __forceinline__ float ms_block_sum(float v, float* s_red) {
     __syncthreads();
     float t = 0.f;
     for (int w = 0; w < (int)(blockDim.x >> 5); w++) t += s_red[w];
-    return t;
-}
-
-// the same in double: the stop test compares residuals that differ in the sixth digit (tol = 1e-6 is the reference's
-// default, analysis.py:718-719); float sums over n*m terms carry roundoff of that order
-__device__ __forceinline__ double ms_block_sum_d(double v, float* s_red) {
-    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    double* s_d = reinterpret_cast<double*>(s_red);
-    __syncthreads();
-    if (lane == 0) s_d[warp] = v;
-    __syncthreads();
-    double t = 0.0;
-    for (int w = 0; w < (int)(blockDim.x >> 5); w++) t += s_d[w];
     return t;
 }
 
@@ -171,7 +146,9 @@ __device__ __forceinline__ void ms_nmf_resident_body(const MsNmfArgs& A, float* 
                 acc += (double)r * (double)r;
             }
         }
-        return ms_block_sum_d(acc, s_red);
+        // summed in double: the stop test compares residuals that differ in the sixth digit (tol = 1e-6 is the
+        // reference's default, analysis.py:718-719); float sums over n*m terms carry roundoff of that order
+        return ms_block_sum_d(acc, reinterpret_cast<double*>(s_red));
     };
     auto compute_hht = [&]() {
         for (int e = tid; e < K * K; e += NMF_THREADS) {
@@ -312,7 +289,7 @@ __device__ __forceinline__ void ms_nmf_resident_body(const MsNmfArgs& A, float* 
         __syncthreads();
         // ---- H <- H * (W^T X) / ((W^T W) H)
         {
-            float newh[(NMF_MAX_K * NMF_MAX_M + NMF_THREADS - 1) / NMF_THREADS];
+            float newh[(MS_NMF_MAX_K * MS_NMF_MAX_M + NMF_THREADS - 1) / NMF_THREADS];
             int q = 0;
             for (int e = tid; e < K * m; e += NMF_THREADS, q++) {
                 const int a = e / m, j = e - a * m;
@@ -388,18 +365,9 @@ __global__ void __launch_bounds__(NMF_THREADS, NMF_MIN_CTAS)
     A.n_iter_out = n_iter_out + blockIdx.x;
     A.err_out = err_out + blockIdx.x;
     A.vaf_out = vaf_out + (long long)blockIdx.x * (m + 1);
-    switch (pb.k) {
-#define MS_NMF_CASE(KK) \
-    case KK:            \
-        ms_nmf_resident_body<KK>(A, sm); \
-        break;
-        MS_NMF_CASE(1) MS_NMF_CASE(2) MS_NMF_CASE(3) MS_NMF_CASE(4) MS_NMF_CASE(5) MS_NMF_CASE(6) MS_NMF_CASE(7)
-        MS_NMF_CASE(8) MS_NMF_CASE(9) MS_NMF_CASE(10) MS_NMF_CASE(11) MS_NMF_CASE(12) MS_NMF_CASE(13)
-        MS_NMF_CASE(14) MS_NMF_CASE(15) MS_NMF_CASE(16)
-#undef MS_NMF_CASE
-        default:
-            break;
-    }
+#define NMF_RESIDENT(KK) ms_nmf_resident_body<KK>(A, sm)
+    MS_NMF_K_SWITCH(pb.k, NMF_RESIDENT)
+#undef NMF_RESIDENT
 }
 
 static size_t ms_nmf_resident_fixed_floats(int m, int kmax) {
@@ -416,11 +384,7 @@ static size_t ms_nmf_resident_smem(int n, int m, int kmax) {
 
 // Largest n the resident kernel takes for (m, kmax); 0 if the shape is unsupported.
 extern "C" int32_t ms_nmf_resident_max_rows(int32_t m, int32_t kmax) {
-    if (m < 1 || m > NMF_MAX_M || kmax < 1 || kmax > NMF_MAX_K) return 0;
-    const size_t budget = 227 * 1024 - 1024;
-    const size_t fixed = sizeof(float) * ms_nmf_resident_fixed_floats(m, kmax);
-    const size_t per_row = sizeof(float) * ms_nmf_resident_row_floats(m, kmax);
-    return (int32_t)((budget - fixed) / per_row);
+    return ms_nmf_max_rows(m, kmax, sizeof(float), ms_nmf_resident_fixed_floats, ms_nmf_resident_row_floats);
 }
 
 // The problem table of a batch (32 bytes per problem: rank, offsets of its W, H and X), written to HOST memory the
@@ -429,22 +393,23 @@ extern "C" int32_t ms_nmf_resident_max_rows(int32_t m, int32_t kmax) {
 // copies nor waits.
 extern "C" int32_t ms_nmf_plan(int32_t n, int32_t m, const int32_t* h_ranks, const int32_t* h_x_index, int32_t n_problems,
                                void* h_table) {
-    if (!h_ranks || !h_table || n < 1 || m < 1 || m > NMF_MAX_M || n_problems < 0) return MS_E_INVALID;
-    MsNmfProblem* h = (MsNmfProblem*)h_table;
-    long long wo = 0, ho = 0;
-    int kmax = 0;
-    for (int p = 0; p < n_problems; p++) {
-        const int k = h_ranks[p];
-        if (k < 1 || k > NMF_MAX_K) return MS_E_INVALID;
-        h[p].k = k;
-        h[p].w_off = wo;
-        h[p].h_off = ho;
-        h[p].x_off = h_x_index ? (long long)h_x_index[p] * n * m : 0;
-        if (h[p].x_off < 0) return MS_E_INVALID;
-        wo += (long long)n * k;
-        ho += (long long)k * m;
-        if (k > kmax) kmax = k;
+    if (!h_ranks || !h_table || n < 1 || m < 1 || m > MS_NMF_MAX_M || n_problems < 0) return MS_E_INVALID;
+    return ms_nmf_fill_table(n, m, h_ranks, h_x_index, n_problems, (MsNmfProblem*)h_table);
+}
+
+// The table of ms_nmf_plan, copied to d_table (and waited for); returns the largest rank or a negative MS_E_* code.
+static int ms_nmf_upload_table(long long n, int m, const int32_t* h_ranks, const int32_t* h_x_index, int n_problems,
+                               void* d_table, cudaStream_t st) {
+    MsNmfProblem* h = (MsNmfProblem*)malloc(sizeof(MsNmfProblem) * n_problems);
+    if (!h) return MS_E_INVALID;
+    const int kmax = ms_nmf_fill_table(n, m, h_ranks, h_x_index, n_problems, h);
+    cudaError_t e = cudaSuccess;
+    if (kmax > 0) {
+        e = cudaMemcpyAsync(d_table, h, sizeof(MsNmfProblem) * n_problems, cudaMemcpyHostToDevice, st);
+        if (e == cudaSuccess) e = cudaStreamSynchronize(st);  // h is pageable: do not free it under the copy
     }
+    free(h);
+    MS_CUDA_CHECK(e);
     return kmax;
 }
 
@@ -453,7 +418,7 @@ extern "C" int ms_nmf_mu_batched_planned(const float* d_X, int32_t n, int32_t m,
                                          int32_t kmax, float* d_W, float* d_H, int32_t max_iter, float tol,
                                          int32_t check_every, int32_t* d_n_iter, float* d_err, float* d_vaf, void* stream) {
     if (!d_X || !d_table || !d_W || !d_H || !d_n_iter || !d_err || !d_vaf) return MS_E_INVALID;
-    if (n < 1 || m < 1 || m > NMF_MAX_M || kmax < 1 || kmax > NMF_MAX_K || n_problems < 0 || max_iter < 0 || check_every < 1)
+    if (n < 1 || m < 1 || m > MS_NMF_MAX_M || kmax < 1 || kmax > MS_NMF_MAX_K || n_problems < 0 || max_iter < 0 || check_every < 1)
         return MS_E_INVALID;
     if (n_problems == 0) return MS_OK;
     if (n > ms_nmf_resident_max_rows(m, kmax)) return MS_E_INVALID;  // too long for the resident kernel: use ms_nmf_mu_stream
@@ -476,46 +441,12 @@ extern "C" int ms_nmf_mu_batched(const float* d_X, int32_t n, int32_t m, const i
                                  float* d_W, float* d_H, int32_t max_iter, float tol, int32_t check_every, void* d_work,
                                  int32_t* d_n_iter, float* d_err, float* d_vaf, void* stream) {
     if (!d_X || !h_ranks || !d_W || !d_H || !d_work || !d_n_iter || !d_err || !d_vaf) return MS_E_INVALID;
-    if (n < 1 || m < 1 || m > NMF_MAX_M || n_problems < 0 || max_iter < 0 || check_every < 1) return MS_E_INVALID;
+    if (n < 1 || m < 1 || m > MS_NMF_MAX_M || n_problems < 0 || max_iter < 0 || check_every < 1) return MS_E_INVALID;
     if (n_problems == 0) return MS_OK;
-    cudaStream_t st = (cudaStream_t)stream;
-    int kmax = 0;
-    MsNmfProblem* h = (MsNmfProblem*)malloc(sizeof(MsNmfProblem) * n_problems);
-    if (!h) return MS_E_INVALID;
-    long long wo = 0, ho = 0;
-    for (int p = 0; p < n_problems; p++) {
-        const int k = h_ranks[p];
-        if (k < 1 || k > NMF_MAX_K) {
-            free(h);
-            return MS_E_INVALID;
-        }
-        h[p].k = k;
-        h[p].w_off = wo;
-        h[p].h_off = ho;
-        h[p].x_off = h_x_index ? (long long)h_x_index[p] * n * m : 0;
-        if (h[p].x_off < 0) {
-            free(h);
-            return MS_E_INVALID;
-        }
-        wo += (long long)n * k;
-        ho += (long long)k * m;
-        if (k > kmax) kmax = k;
-    }
-    if (n > ms_nmf_resident_max_rows(m, kmax)) {
-        free(h);
-        return MS_E_INVALID;  // too long for the resident kernel: use ms_nmf_mu_stream
-    }
-    cudaError_t e = cudaMemcpyAsync(d_work, h, sizeof(MsNmfProblem) * n_problems, cudaMemcpyHostToDevice, st);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(st);  // h is pageable: do not free it under the copy
-    free(h);
-    MS_CUDA_CHECK(e);
-    const size_t smem = ms_nmf_resident_smem(n, m, kmax);
-    MS_CUDA_CHECK(cudaFuncSetAttribute(ms_nmf_resident_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    ms_nmf_resident_kernel<<<n_problems, NMF_THREADS, smem, st>>>(d_X, n, m, (const MsNmfProblem*)d_work, d_W, d_H,
-                                                                  max_iter, tol, check_every, d_n_iter, d_err, d_vaf);
-    MS_COUNT_LAUNCH();
-    MS_CUDA_CHECK(cudaGetLastError());
-    return MS_OK;
+    const int kmax = ms_nmf_upload_table(n, m, h_ranks, h_x_index, n_problems, d_work, (cudaStream_t)stream);
+    if (kmax < 0) return kmax;
+    return ms_nmf_mu_batched_planned(d_X, n, m, d_work, n_problems, kmax, d_W, d_H, max_iter, tol, check_every, d_n_iter,
+                                     d_err, d_vaf, stream);
 }
 
 // ---------------------------------------------------------------------------------------------------
@@ -532,8 +463,8 @@ extern "C" int ms_nmf_mu_batched(const float* d_X, int32_t n, int32_t m, const i
 #define NMFS_ROWS 256
 
 struct MsNmfStreamState {  // per problem, device memory
-    float HHt[NMF_MAX_K * NMF_MAX_K];
-    float acc[NMF_MAX_K * NMF_MAX_K + NMF_MAX_K * NMF_MAX_M];  // W^T W then W^T X
+    float HHt[MS_NMF_MAX_K * MS_NMF_MAX_K];
+    float acc[MS_NMF_MAX_K * MS_NMF_MAX_K + MS_NMF_MAX_K * MS_NMF_MAX_M];  // W^T W then W^T X
     float err0, prev, err;
     int n_iter, done;
 };
@@ -738,18 +669,9 @@ __global__ void __launch_bounds__(NMFS_ROWS, 3)
     float* Wp = Wg + pb.w_off;
     const float* Hp = Hg + pb.h_off;
     const float* Xp = X + pb.x_off;
-    switch (pb.k) {
-#define MS_NMF_CASE(KK) \
-    case KK:            \
-        ms_nmf_stream_w_body<KK>(Xp, n, m, Wp, Hp, stt, sm); \
-        break;
-        MS_NMF_CASE(1) MS_NMF_CASE(2) MS_NMF_CASE(3) MS_NMF_CASE(4) MS_NMF_CASE(5) MS_NMF_CASE(6) MS_NMF_CASE(7)
-        MS_NMF_CASE(8) MS_NMF_CASE(9) MS_NMF_CASE(10) MS_NMF_CASE(11) MS_NMF_CASE(12) MS_NMF_CASE(13)
-        MS_NMF_CASE(14) MS_NMF_CASE(15) MS_NMF_CASE(16)
-#undef MS_NMF_CASE
-        default:
-            break;
-    }
+#define NMF_STREAM_W(KK) ms_nmf_stream_w_body<KK>(Xp, n, m, Wp, Hp, stt, sm)
+    MS_NMF_K_SWITCH(pb.k, NMF_STREAM_W)
+#undef NMF_STREAM_W
 }
 
 // mode 0: prepare (H H^T of the initial H, clear accumulators); mode 1: H update after a W pass
@@ -757,7 +679,7 @@ __global__ void __launch_bounds__(128)
     ms_nmf_stream_h_kernel(int m, const MsNmfProblem* __restrict__ problems, float* __restrict__ Hg,
                            MsNmfStreamState* __restrict__ states, const float* __restrict__ xx, int mode, int iteration,
                            float tol, int check_every) {
-    __shared__ float sH[NMF_MAX_K * NMF_MAX_M];
+    __shared__ float sH[MS_NMF_MAX_K * MS_NMF_MAX_M];
     const MsNmfProblem pb = problems[blockIdx.x];
     MsNmfStreamState* stt = states + blockIdx.x;
     const int k = pb.k, tid = threadIdx.x;
@@ -822,7 +744,7 @@ __global__ void __launch_bounds__(256)
     ms_nmf_stream_vaf_kernel(const float* __restrict__ X, long long n, int m, const MsNmfProblem* __restrict__ problems,
                              const float* __restrict__ Wg, const float* __restrict__ Hg, double* __restrict__ sums) {
     // sums: [P][2][m]  (residual, total)
-    __shared__ float sH[NMF_MAX_K * NMF_MAX_M];
+    __shared__ float sH[MS_NMF_MAX_K * MS_NMF_MAX_M];
     const MsNmfProblem pb = problems[blockIdx.y];
     const int k = pb.k;
     const float* Xp = X + pb.x_off;
@@ -886,39 +808,19 @@ extern "C" int ms_nmf_mu_stream(const float* d_X, int64_t n, int32_t m, const in
                                 int32_t check_every, void* d_work, int32_t* d_n_iter, float* d_err, float* d_vaf,
                                 void* stream) {
     if (!d_X || !h_ranks || !d_W || !d_H || !d_work || !d_n_iter || !d_err || !d_vaf) return MS_E_INVALID;
-    if (n < 1 || m < 1 || m > NMF_MAX_M || n_problems < 0 || max_iter < 0 || check_every < 1) return MS_E_INVALID;
+    if (n < 1 || m < 1 || m > MS_NMF_MAX_M || n_problems < 0 || max_iter < 0 || check_every < 1) return MS_E_INVALID;
     if (n_problems == 0) return MS_OK;
     cudaStream_t st = (cudaStream_t)stream;
-    MsNmfProblem* h = (MsNmfProblem*)malloc(sizeof(MsNmfProblem) * n_problems);
-    if (!h) return MS_E_INVALID;
-    long long wo = 0, ho = 0;
-    int kmax = 0;
-    for (int p = 0; p < n_problems; p++) {
-        const int k = h_ranks[p];
-        if (k < 1 || k > NMF_MAX_K) {
-            free(h);
-            return MS_E_INVALID;
-        }
-        h[p].k = k;
-        h[p].w_off = wo;
-        h[p].h_off = ho;
-        h[p].x_off = h_x_index ? (long long)h_x_index[p] * n * m : 0;
-        wo += (long long)n * k;
-        ho += (long long)k * m;
-        if (k > kmax) kmax = k;
-    }
     char* wsp = (char*)d_work;
     MsNmfProblem* d_problems = (MsNmfProblem*)wsp;
-    wsp += ((sizeof(MsNmfProblem) * n_problems + 255) / 256) * 256;
+    wsp += ms_align256(sizeof(MsNmfProblem) * n_problems);
     MsNmfStreamState* d_states = (MsNmfStreamState*)wsp;
-    wsp += ((sizeof(MsNmfStreamState) * n_problems + 255) / 256) * 256;
+    wsp += ms_align256(sizeof(MsNmfStreamState) * n_problems);
     double* d_sums = (double*)wsp;
     wsp += (size_t)n_problems * 2 * m * 8;
     float* d_xx = (float*)wsp;
-    cudaError_t e = cudaMemcpyAsync(d_problems, h, sizeof(MsNmfProblem) * n_problems, cudaMemcpyHostToDevice, st);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(st);
-    free(h);
-    MS_CUDA_CHECK(e);
+    const int kmax = ms_nmf_upload_table(n, m, h_ranks, h_x_index, n_problems, d_problems, st);
+    if (kmax < 0) return kmax;
 
     const long long n_tiles = (n + NMFS_ROWS - 1) / NMFS_ROWS;
     int ctas = (148 * 3 + n_problems - 1) / n_problems;  // three CTAs of the W pass fit an SM: one wave
@@ -948,18 +850,10 @@ extern "C" int ms_nmf_mu_stream(const float* d_X, int64_t n, int32_t m, const in
         MS_COUNT_LAUNCH();
         ms_nmf_stream_h_kernel<<<n_problems, 128, 0, st>>>(m, d_problems, d_H, d_states, d_xx, 1, it, tol, check_every);
         MS_COUNT_LAUNCH();
-        if (tol > 0.f && it % 64 == 0) {
-            // stop early when every problem has converged
-            int all_done = 1;
-            MsNmfStreamState* hs = (MsNmfStreamState*)malloc(sizeof(MsNmfStreamState) * n_problems);
-            if (hs) {
-                cudaMemcpyAsync(hs, d_states, sizeof(MsNmfStreamState) * n_problems, cudaMemcpyDeviceToHost, st);
-                cudaStreamSynchronize(st);
-                for (int p = 0; p < n_problems; p++)
-                    if (!hs[p].done) all_done = 0;
-                free(hs);
-                if (all_done) break;
-            }
+        if (tol > 0.f && it % 64 == 0) {  // stop early when every problem has converged
+            const int done = ms_nmf_all_done(d_states, n_problems, st);
+            if (done < 0) return done;
+            if (done) break;
         }
     }
     MS_CUDA_CHECK(cudaMemsetAsync(d_sums, 0, (size_t)n_problems * 2 * m * 8, st));

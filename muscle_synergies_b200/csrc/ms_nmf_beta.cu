@@ -31,28 +31,15 @@
 //
 // No floating-point atomics: two identical calls give bit-identical W, H, n_iter, err and VAF.  The two regimes sum the
 // H-step terms in different orders, so they agree to rounding, not bit for bit.
-#include <stdio.h>
-
-#include "ms_common.cuh"
+#include "ms_nmf_common.cuh"
 
 #define BT_THREADS 256
-#define BT_MAX_K 16
-#define BT_MAX_M 64
 #define BT_EPS 1.1920928955078125e-07        // np.finfo(np.float32).eps, sklearn's EPSILON
 #define BT_DBL_EPS 2.220446049250313e-16     // np.finfo(np.float64).eps
 #define BT_IS 0
 #define BT_KL 1
 #define BT_GEN 2
-#define BT_Q(K) (((K) * BT_MAX_M + BT_THREADS - 1) / BT_THREADS)  // H entries per thread in bt_hacc
-
-struct MsNmfProblem {  // ms_nmf_plan's table (csrc/ms_nmf.cu)
-    int k;
-    long long w_off;
-    long long h_off;
-    long long x_off;
-};
-
-__host__ __device__ inline int bt_odd(int v) { return v | 1; }
+#define BT_Q(K) (((K) * MS_NMF_MAX_M + BT_THREADS - 1) / BT_THREADS)  // H entries per thread in bt_hacc
 
 // numpy's x ** e for a scalar e: the fast paths first, pow otherwise
 __device__ __forceinline__ double bt_pow(double x, double e) {
@@ -212,37 +199,17 @@ __device__ __forceinline__ void bt_hsum(const double* sH, int k, int m, double* 
     }
 }
 
-// fixed-order sum over the CTA (warp trees, then the warps in order); every thread gets the total
-__device__ __forceinline__ double bt_block_sum(double v, double* s_red) {
-    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-    __syncthreads();
-    if ((threadIdx.x & 31) == 0) s_red[threadIdx.x >> 5] = v;
-    __syncthreads();
-    double total = 0.0;
-    for (int w = 0; w < (int)(blockDim.x >> 5); w++) total += s_red[w];
-    return total;
-}
-
-#define BT_K_SWITCH(KEXPR, CALL)                                                                                      \
-    switch (KEXPR) {                                                                                                  \
-        case 1: CALL(1); break;   case 2: CALL(2); break;   case 3: CALL(3); break;   case 4: CALL(4); break;         \
-        case 5: CALL(5); break;   case 6: CALL(6); break;   case 7: CALL(7); break;   case 8: CALL(8); break;         \
-        case 9: CALL(9); break;   case 10: CALL(10); break; case 11: CALL(11); break; case 12: CALL(12); break;       \
-        case 13: CALL(13); break; case 14: CALL(14); break; case 15: CALL(15); break; case 16: CALL(16); break;       \
-        default: break;                                                                                               \
-    }
-
 // ---------------------------------------------------------------------------------------------------
 // resident regime
 // ---------------------------------------------------------------------------------------------------
-// Shared memory (doubles): sX [n][XS], sF [n][XS], sG [n][XS], sW [n][WS], sH [K][m], sHs [K], sPart [2][BT_MAX_M],
+// Shared memory (doubles): sX [n][XS], sF [n][XS], sG [n][XS], sW [n][WS], sH [K][m], sHs [K], sPart [2][MS_NMF_MAX_M],
 // s_red [32]
 template <int MODE, int K>
 __device__ __forceinline__ void bt_resident_body(const double* __restrict__ X, int n, int m, long long rs, long long cs,
                                                  double* __restrict__ Wp, double* __restrict__ Hp, double beta,
                                                  double gamma, int update_H, int max_iter, double tol,
                                                  int32_t* n_iter_out, double* err_out, double* vaf_out, double* sm) {
-    const int XS = bt_odd(m), WS = bt_odd(K);
+    const int XS = ms_odd(m), WS = ms_odd(K);
     double* sX = sm;
     double* sF = sX + (size_t)n * XS;
     double* sG = sF + (size_t)n * XS;
@@ -250,7 +217,7 @@ __device__ __forceinline__ void bt_resident_body(const double* __restrict__ X, i
     double* sH = sW + (size_t)n * WS;
     double* sHs = sH + K * m;
     double* sPart = sHs + K;
-    double* s_red = sPart + 2 * BT_MAX_M;
+    double* s_red = sPart + 2 * MS_NMF_MAX_M;
     const int tid = threadIdx.x;
 
     for (int i = tid; i < n * m; i += BT_THREADS) sX[(i / m) * XS + i % m] = X[(i / m) * rs + (i % m) * cs];
@@ -261,7 +228,7 @@ __device__ __forceinline__ void bt_resident_body(const double* __restrict__ X, i
     __syncthreads();
 
     double stop_ref = 0.0, prev = 0.0, unused = 0.0;
-    if (tol > 0.0) stop_ref = prev = bt_err(MODE, bt_block_sum(bt_div_rows<MODE, K>(sX, XS, sW, WS, n, m, sH, beta), s_red), beta);
+    if (tol > 0.0) stop_ref = prev = bt_err(MODE, ms_block_sum_d(bt_div_rows<MODE, K>(sX, XS, sW, WS, n, m, sH, beta), s_red), beta);
     int it = 0;
     for (it = 1; it <= max_iter; it++) {
         for (int i = tid; i < n; i += BT_THREADS) {
@@ -292,7 +259,7 @@ __device__ __forceinline__ void bt_resident_body(const double* __restrict__ X, i
         }
         if (tol > 0.0 && it % 10 == 0) {
             const double err =
-                bt_err(MODE, bt_block_sum(bt_div_rows<MODE, K>(sX, XS, sW, WS, n, m, sH, beta), s_red), beta);
+                bt_err(MODE, ms_block_sum_d(bt_div_rows<MODE, K>(sX, XS, sW, WS, n, m, sH, beta), s_red), beta);
             if ((prev - err) / stop_ref < tol) break;
             prev = err;
         }
@@ -304,7 +271,7 @@ __device__ __forceinline__ void bt_resident_body(const double* __restrict__ X, i
     for (int i = tid; i < n * K; i += BT_THREADS) Wp[i] = sW[(i / K) * WS + i % K];
     if (update_H)
         for (int i = tid; i < K * m; i += BT_THREADS) Hp[i] = sH[i];
-    const double err = bt_err(MODE, bt_block_sum(bt_div_rows<MODE, K>(sX, XS, sW, WS, n, m, sH, beta), s_red), beta);
+    const double err = bt_err(MODE, ms_block_sum_d(bt_div_rows<MODE, K>(sX, XS, sW, WS, n, m, sH, beta), s_red), beta);
     for (int j = tid; j < m; j += BT_THREADS) {
         double r2 = 0.0, c2 = 0.0;
         for (int i = 0; i < n; i++) {
@@ -315,13 +282,13 @@ __device__ __forceinline__ void bt_resident_body(const double* __restrict__ X, i
             r2 = fma(r, r, r2);
         }
         sPart[j] = r2;
-        sPart[BT_MAX_M + j] = c2;
+        sPart[MS_NMF_MAX_M + j] = c2;
         vaf_out[1 + j] = 1.0 - r2 / c2;
     }
     __syncthreads();
     if (tid == 0) {
         double r2 = 0.0, c2 = 0.0;
-        for (int j = 0; j < m; j++) r2 += sPart[j], c2 += sPart[BT_MAX_M + j];
+        for (int j = 0; j < m; j++) r2 += sPart[j], c2 += sPart[MS_NMF_MAX_M + j];
         *n_iter_out = it;
         *err_out = err;
         vaf_out[0] = 1.0 - r2 / c2;
@@ -341,19 +308,16 @@ __global__ void __maxnreg__(255)
 #define BT_RESIDENT(KK)                                                                                               \
     bt_resident_body<MODE, KK>(X + pb.x_off, n, m, rs, cs, Wg + pb.w_off, Hg + pb.h_off, beta, gamma, update_H,       \
                                max_iter, tol, n_iter_out + p, err_out + p, vaf_out + (long long)p * (m + 1), bt_sm)
-    BT_K_SWITCH(pb.k, BT_RESIDENT)
+    MS_NMF_K_SWITCH(pb.k, BT_RESIDENT)
 #undef BT_RESIDENT
 }
 
-static size_t bt_resident_fixed(int m, int kmax) { return (size_t)kmax * m + kmax + 2 * BT_MAX_M + 32; }
-static size_t bt_resident_row(int m, int kmax) { return 3 * (size_t)bt_odd(m) + bt_odd(kmax); }
-static const size_t BT_SMEM_BUDGET = 227 * 1024 - 1024;
+static size_t bt_resident_fixed(int m, int kmax) { return (size_t)kmax * m + kmax + 2 * MS_NMF_MAX_M + 32; }
+static size_t bt_resident_row(int m, int kmax) { return 3 * (size_t)ms_odd(m) + ms_odd(kmax); }
 
 // Largest n the resident β kernel takes for (m, kmax); 0 if the shape is unsupported.
 extern "C" int32_t ms_nmf_beta_resident_max_rows(int32_t m, int32_t kmax) {
-    if (m < 1 || m > BT_MAX_M || kmax < 1 || kmax > BT_MAX_K) return 0;
-    return (int32_t)((BT_SMEM_BUDGET - sizeof(double) * bt_resident_fixed(m, kmax)) /
-                     (sizeof(double) * bt_resident_row(m, kmax)));
+    return ms_nmf_max_rows(m, kmax, sizeof(double), bt_resident_fixed, bt_resident_row);
 }
 
 // ---------------------------------------------------------------------------------------------------
@@ -375,17 +339,15 @@ struct BtLayout {  // the workspace, carved by bt_layout
     double* vparts;     // [P][vctas][2 m + 1]: per-CTA residual / total sums of squares per column, then the divergence
 };
 
-static size_t bt_align(size_t b) { return (b + 255) / 256 * 256; }
-
 // rows per tile of the pass kernel: one per thread, fewer where the H-step terms of 256 rows do not fit
 static int bt_tile_rows(int m, int kmax) {
-    const size_t fixed = (size_t)kmax * m + kmax + 32, row = 2 * (size_t)bt_odd(m) + bt_odd(kmax);
-    const size_t fit = (BT_SMEM_BUDGET / sizeof(double) - fixed) / row;
+    const size_t fixed = (size_t)kmax * m + kmax + 32, row = 2 * (size_t)ms_odd(m) + ms_odd(kmax);
+    const size_t fit = (MS_NMF_SMEM_BUDGET / sizeof(double) - fixed) / row;
     return (int)(fit < BT_THREADS ? fit : BT_THREADS);
 }
 static size_t bt_pass_smem(int m, int kmax) {
     return sizeof(double) * ((size_t)kmax * m + kmax + 32 +
-                             (size_t)bt_tile_rows(m, kmax) * (2 * (size_t)bt_odd(m) + bt_odd(kmax)));
+                             (size_t)bt_tile_rows(m, kmax) * (2 * (size_t)ms_odd(m) + ms_odd(kmax)));
 }
 static long long bt_ctas(long long n, int m, int kmax, int n_problems) {  // pass-kernel CTAs per problem
     const long long tr = bt_tile_rows(m, kmax);
@@ -408,7 +370,7 @@ static size_t bt_layout(long long n, int m, int n_problems, int kmax, char* base
     size_t off = 0;
     for (int s = 0; s < 4; s++) {
         ptrs[s] = base ? base + off : nullptr;
-        off += bt_align(sizes[s]);
+        off += ms_align256(sizes[s]);
     }
     if (L) {
         L->states = (MsBtState*)ptrs[0];
@@ -438,7 +400,7 @@ __device__ __forceinline__ void bt_pass_body(const double* __restrict__ X, long 
                                              double* __restrict__ Wp, const double* __restrict__ Hp, double beta,
                                              double gamma, int update_H, bool do_div, int TR,
                                              double* __restrict__ wsavep, double* __restrict__ part, double* sm) {
-    const int XS = bt_odd(m), WS = bt_odd(K);
+    const int XS = ms_odd(m), WS = ms_odd(K);
     double* sH = sm;
     double* sHs = sH + K * m;
     double* s_red = sHs + K;
@@ -483,7 +445,7 @@ __device__ __forceinline__ void bt_pass_body(const double* __restrict__ X, long 
         }
     }
     if (do_div) {
-        const double total = bt_block_sum(div, s_red);
+        const double total = ms_block_sum_d(div, s_red);
         if (tid == 0) part[2 * K * m] = total;
     }
 }
@@ -502,7 +464,7 @@ __global__ void __launch_bounds__(BT_THREADS)
 #define BT_PASS(KK)                                                                                                   \
     bt_pass_body<MODE, KK>(X + pb.x_off, n, m, rs, cs, Wg + pb.w_off, Hg + pb.h_off, beta, gamma, update_H,           \
                            st.pending >= 0, TR, L.wsave + (long long)p * n * kmax, part, bt_sm)
-    BT_K_SWITCH(pb.k, BT_PASS)
+    MS_NMF_K_SWITCH(pb.k, BT_PASS)
 #undef BT_PASS
 }
 
@@ -574,7 +536,7 @@ __global__ void __launch_bounds__(BT_THREADS)
     ms_bt_final_kernel(const double* __restrict__ X, long long n, int m, long long rs, long long cs,
                        const MsNmfProblem* __restrict__ problems, const double* __restrict__ Wg,
                        const double* __restrict__ Hg, double beta, BtLayout L) {
-    __shared__ double sH[BT_MAX_K * BT_MAX_M];
+    __shared__ double sH[MS_NMF_MAX_K * MS_NMF_MAX_M];
     __shared__ double sR[3][BT_THREADS];
     const MsNmfProblem pb = problems[blockIdx.y];
     const int k = pb.k;
@@ -614,7 +576,7 @@ __global__ void __launch_bounds__(BT_THREADS)
 
 __global__ void ms_bt_finish_kernel(int m, int mode, double beta, int vctas, BtLayout L, int32_t* __restrict__ n_iter,
                                     double* __restrict__ err, double* __restrict__ vaf) {
-    __shared__ double s_cols[2 * BT_MAX_M + 1];
+    __shared__ double s_cols[2 * MS_NMF_MAX_M + 1];
     const int p = blockIdx.x;
     const double* vp = L.vparts + (long long)p * vctas * (2 * m + 1);
     for (int e = threadIdx.x; e < 2 * m + 1; e += blockDim.x) {
@@ -637,7 +599,7 @@ __global__ void ms_bt_finish_kernel(int m, int mode, double beta, int vctas, BtL
 // C ABI
 // ---------------------------------------------------------------------------------------------------
 extern "C" int64_t ms_nmf_beta_workspace_bytes(int64_t n, int32_t m, int32_t n_problems, int32_t kmax) {
-    if (n < 1 || m < 1 || m > BT_MAX_M || n_problems < 0 || kmax < 1 || kmax > BT_MAX_K) return 0;
+    if (n < 1 || m < 1 || m > MS_NMF_MAX_M || n_problems < 0 || kmax < 1 || kmax > MS_NMF_MAX_K) return 0;
     if (n_problems == 0) return 256;
     return (int64_t)bt_layout(n, m, n_problems, kmax, nullptr, nullptr) + 256;
 }
@@ -654,7 +616,7 @@ extern "C" int ms_nmf_beta(const double* d_X, int64_t n, int32_t m, int64_t row_
                            int32_t update_H, int32_t max_iter, double tol, int32_t regime, void* d_work,
                            int32_t* d_n_iter, double* d_err, double* d_vaf, void* stream) {
     if (!d_X || !d_table || !d_W || !d_H || !d_n_iter || !d_err || !d_vaf) return MS_E_INVALID;
-    if (n < 1 || m < 1 || m > BT_MAX_M || kmax < 1 || kmax > BT_MAX_K || n_problems < 0 || max_iter < 0 ||
+    if (n < 1 || m < 1 || m > MS_NMF_MAX_M || kmax < 1 || kmax > MS_NMF_MAX_K || n_problems < 0 || max_iter < 0 ||
         !(tol >= 0.0) || !(beta == beta) || beta == 2.0 || (regime != 0 && regime != 1) || row_stride < 0 ||
         col_stride < 0 || (update_H != 0 && update_H != 1))
         return MS_E_INVALID;  // beta = 2 (Frobenius) is the job of ms_nmf_mu_* / ms_nmf_fixed_h
@@ -688,8 +650,6 @@ extern "C" int ms_nmf_beta(const double* d_X, int64_t n, int32_t m, int64_t row_
 #undef BT_SET_SMEM
     ms_bt_init_kernel<<<(n_problems + 127) / 128, 128, 0, st>>>(n_problems, max_iter, tol, L);
     MS_COUNT_LAUNCH();
-    MsBtState* h_states = (MsBtState*)malloc(sizeof(MsBtState) * (size_t)n_problems);
-    if (!h_states) return MS_E_INVALID;
     for (int it = 1; it <= max_iter; it++) {
 #define BT_LAUNCH_PASS(MM)                                                                                            \
     ms_bt_pass_kernel<MM><<<dim3(ctas, n_problems), BT_THREADS, smem, st>>>(d_X, n, m, row_stride, col_stride,        \
@@ -701,21 +661,12 @@ extern "C" int ms_nmf_beta(const double* d_X, int64_t n, int32_t m, int64_t row_
         ms_bt_update_kernel<<<n_problems, BT_THREADS, 0, st>>>(d_problems, d_H, m, mode, beta, gamma, update_H, it,
                                                                max_iter, tol, ctas, L, kmax);
         MS_COUNT_LAUNCH();
-        if (tol > 0.0 && it % 64 == 0 && it < max_iter) {
-            // stop early once every problem is done (pageable copy: waits for the stream)
-            cudaError_t e = cudaMemcpyAsync(h_states, L.states, sizeof(MsBtState) * (size_t)n_problems,
-                                            cudaMemcpyDeviceToHost, st);
-            if (e == cudaSuccess) e = cudaStreamSynchronize(st);
-            if (e != cudaSuccess) {
-                free(h_states);
-                MS_CUDA_CHECK(e);
-            }
-            int all_done = 1;
-            for (int p = 0; p < n_problems; p++) all_done &= h_states[p].done != 0;
-            if (all_done) break;
+        if (tol > 0.0 && it % 64 == 0 && it < max_iter) {  // stop early once every problem is done
+            const int done = ms_nmf_all_done(L.states, n_problems, st);
+            if (done < 0) return done;
+            if (done) break;
         }
     }
-    free(h_states);
     ms_bt_restore_kernel<<<dim3(ctas, n_problems), BT_THREADS, 0, st>>>(n, d_problems, d_W, L, kmax);
     MS_COUNT_LAUNCH();
 #define BT_LAUNCH_FINAL(MM)                                                                                           \

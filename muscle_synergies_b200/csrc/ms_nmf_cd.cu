@@ -19,29 +19,11 @@
 //                            violation), then one small CTA per problem for the H step and the stop test
 //   ms_nndsvd_*              _initialize_nmf(init="nndsvd" / "nndsvda") from an exact SVD: X^T X, cyclic Jacobi,
 //                            U = X V S^-1; one SVD per distinct matrix of the stack serves every rank on it
-#include <stdio.h>
-
-#include "ms_common.cuh"
+#include "ms_nmf_common.cuh"
 
 #define CD_THREADS 256
-#define CD_MAX_K 16
-#define CD_MAX_M 64
-#define CD_ITEMS ((CD_MAX_K * CD_MAX_K + CD_MAX_K * CD_MAX_M + CD_THREADS - 1) / CD_THREADS)  // reduction items a thread owns
-
-// ms_nmf_plan's table (csrc/ms_nmf.cu): offsets are element counts, so they serve fp64 factors unchanged
-struct MsNmfProblem {
-    int k;
-    long long w_off;
-    long long h_off;
-    long long x_off;
-};
-
-__host__ __device__ inline int cd_odd(int v) { return v | 1; }  // row stride in doubles: an odd stride is free of bank conflicts
-
-__device__ __forceinline__ double cd_warp_sum(double v) {
-    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-    return v;
-}
+// reduction items a thread owns
+#define CD_ITEMS ((MS_NMF_MAX_K * MS_NMF_MAX_K + MS_NMF_MAX_K * MS_NMF_MAX_M + CD_THREADS - 1) / CD_THREADS)
 
 // One coordinate-descent sweep over the K entries of one row w (of W, or of H^T): G = the K x K Gram matrix (row
 // stride gs), b = the K right-hand sides (XHt row, or X^T W row).  Returns the row's share of the violation.
@@ -102,7 +84,7 @@ template <int K>
 __device__ __forceinline__ void cd_resident_body(const double* __restrict__ X, int n, int m, double* __restrict__ Wp,
                                                  double* __restrict__ Hp, int max_iter, double tol, int32_t* n_iter_out,
                                                  double* err_out, double* vaf_out, double* sm) {
-    const int XS = cd_odd(m), WS = cd_odd(K);
+    const int XS = ms_odd(m), WS = ms_odd(K);
     const int n_out = K * K + K * m, slices = cd_slices(n_out, n), n_items = n_out * slices;
     double* sX = sm;
     double* sW = sX + n * XS;
@@ -145,7 +127,7 @@ __device__ __forceinline__ void cd_resident_body(const double* __restrict__ X, i
 #pragma unroll
             for (int t = 0; t < K; t++) sW[i * WS + t] = w[t];
         }
-        vw = cd_warp_sum(vw);
+        vw = ms_warp_sum_d(vw);
         if (lane == 0) s_red[warp] = vw;
         __syncthreads();
         // ---- W^T W and W^T X of the updated W: row slices side by side, then one sum per output
@@ -172,7 +154,7 @@ __device__ __forceinline__ void cd_resident_body(const double* __restrict__ X, i
             for (int t = 0; t < K; t++) sH[t * m + tid] = h[t];
         }
         if (tid < 64) {  // m <= 64: the violation of the H step lives in the first two warps
-            vh = cd_warp_sum(vh);
+            vh = ms_warp_sum_d(vh);
             if (lane == 0) s_red[32 + warp] = vh;
         }
         __syncthreads();
@@ -196,27 +178,18 @@ __device__ __forceinline__ void cd_resident_body(const double* __restrict__ X, i
             rs = fma(r, r, rs);
         }
         sPart[j] = rs;
-        sPart[CD_MAX_M + j] = cs;
+        sPart[MS_NMF_MAX_M + j] = cs;
         vaf_out[1 + j] = 1.0 - rs / cs;
     }
     __syncthreads();
     if (tid == 0) {
         double rs = 0.0, cs = 0.0;
-        for (int j = 0; j < m; j++) rs += sPart[j], cs += sPart[CD_MAX_M + j];
+        for (int j = 0; j < m; j++) rs += sPart[j], cs += sPart[MS_NMF_MAX_M + j];
         *n_iter_out = it;
         *err_out = sqrt(rs);
         vaf_out[0] = 1.0 - rs / cs;
     }
 }
-
-#define CD_K_SWITCH(KEXPR, CALL)                                                                                      \
-    switch (KEXPR) {                                                                                                  \
-        case 1: CALL(1); break;   case 2: CALL(2); break;   case 3: CALL(3); break;   case 4: CALL(4); break;         \
-        case 5: CALL(5); break;   case 6: CALL(6); break;   case 7: CALL(7); break;   case 8: CALL(8); break;         \
-        case 9: CALL(9); break;   case 10: CALL(10); break; case 11: CALL(11); break; case 12: CALL(12); break;       \
-        case 13: CALL(13); break; case 14: CALL(14); break; case 15: CALL(15); break; case 16: CALL(16); break;       \
-        default: break;                                                                                               \
-    }
 
 __global__ void __launch_bounds__(CD_THREADS)
     ms_cd_resident_kernel(const double* __restrict__ X, int n, int m, const MsNmfProblem* __restrict__ problems,
@@ -228,7 +201,7 @@ __global__ void __launch_bounds__(CD_THREADS)
 #define CD_RESIDENT(KK)                                                                                               \
     cd_resident_body<KK>(X + pb.x_off, n, m, Wg + pb.w_off, Hg + pb.h_off, max_iter, tol, n_iter_out + p, err_out + p, \
                          vaf_out + (long long)p * (m + 1), cd_sm)
-    CD_K_SWITCH(pb.k, CD_RESIDENT)
+    MS_NMF_K_SWITCH(pb.k, CD_RESIDENT)
 #undef CD_RESIDENT
 }
 
@@ -236,23 +209,20 @@ static size_t cd_resident_fixed(int m, int kmax) {
     const int n_out = kmax * kmax + kmax * m;
     return (size_t)kmax * m * 2 + (size_t)kmax * kmax * 2 + (size_t)(n_out > CD_THREADS ? n_out : CD_THREADS) + 64;
 }
-static size_t cd_resident_row(int m, int kmax) { return (size_t)cd_odd(m) + (size_t)cd_odd(kmax); }
+static size_t cd_resident_row(int m, int kmax) { return (size_t)ms_odd(m) + (size_t)ms_odd(kmax); }
 
 // Largest n the resident CD kernel takes for (m, kmax); 0 if the shape is unsupported.
 extern "C" int32_t ms_nmf_cd_resident_max_rows(int32_t m, int32_t kmax) {
-    if (m < 1 || m > CD_MAX_M || kmax < 1 || kmax > CD_MAX_K) return 0;
-    const size_t budget = 227 * 1024 - 1024;
-    const size_t fixed = sizeof(double) * cd_resident_fixed(m, kmax);
     // the row slices of the Gram reduction (<= n_out * slices partials) must fit the partial buffer: n_out * slices <=
     // max(CD_THREADS, n_out) holds for every n by construction of cd_slices
-    return (int32_t)((budget - fixed) / (sizeof(double) * cd_resident_row(m, kmax)));
+    return ms_nmf_max_rows(m, kmax, sizeof(double), cd_resident_fixed, cd_resident_row);
 }
 
 extern "C" int ms_nmf_cd_batched_planned(const double* d_X, int32_t n, int32_t m, const void* d_table, int32_t n_problems,
                                          int32_t kmax, double* d_W, double* d_H, int32_t max_iter, double tol,
                                          int32_t* d_n_iter, double* d_err, double* d_vaf, void* stream) {
     if (!d_X || !d_table || !d_W || !d_H || !d_n_iter || !d_err || !d_vaf) return MS_E_INVALID;
-    if (n < 1 || m < 1 || m > CD_MAX_M || kmax < 1 || kmax > CD_MAX_K || n_problems < 0 || max_iter < 0 || !(tol >= 0.0))
+    if (n < 1 || m < 1 || m > MS_NMF_MAX_M || kmax < 1 || kmax > MS_NMF_MAX_K || n_problems < 0 || max_iter < 0 || !(tol >= 0.0))
         return MS_E_INVALID;
     if (n_problems == 0) return MS_OK;
     if (n > ms_nmf_cd_resident_max_rows(m, kmax)) return MS_E_INVALID;  // too long for shared memory: ms_nmf_cd_stream
@@ -271,8 +241,8 @@ extern "C" int ms_nmf_cd_batched_planned(const double* d_X, int32_t n, int32_t m
 #define CDS_ROWS CD_THREADS
 
 struct MsCdStreamState {  // per problem, device memory
-    double HHt[CD_MAX_K * CD_MAX_K];
-    double acc[CD_MAX_K * CD_MAX_K + CD_MAX_K * CD_MAX_M];  // W^T W [K][K], then W^T X [K][m]
+    double HHt[MS_NMF_MAX_K * MS_NMF_MAX_K];
+    double acc[MS_NMF_MAX_K * MS_NMF_MAX_K + MS_NMF_MAX_K * MS_NMF_MAX_M];  // W^T W [K][K], then W^T X [K][m]
     double viol_w;                                          // violation of the W step (atomics of the W pass)
     double viol_init;
     int n_iter, done;
@@ -285,7 +255,7 @@ template <int K>
 __device__ __forceinline__ void cd_stream_w_body(const double* __restrict__ X, long long n, int m, double* __restrict__ Wp,
                                                  const double* __restrict__ Hp, MsCdStreamState* __restrict__ st,
                                                  double* sm) {
-    const int XS = cd_odd(m), WS = cd_odd(K);
+    const int XS = ms_odd(m), WS = ms_odd(K);
     const int n_out = K * K + K * m, slices = cd_slices(n_out, CDS_ROWS), n_items = n_out * slices;
     double* sX = sm;                     // [CDS_ROWS][XS]
     double* sW = sX + CDS_ROWS * XS;     // [CDS_ROWS][WS]
@@ -337,7 +307,7 @@ __device__ __forceinline__ void cd_stream_w_body(const double* __restrict__ X, l
         const int item = tid + q * CDS_ROWS;
         if (item < n_items) atomicAdd(&st->acc[item % n_out], acc[q]);
     }
-    vw = cd_warp_sum(vw);
+    vw = ms_warp_sum_d(vw);
     if ((tid & 31) == 0) s_red[tid >> 5] = vw;
     __syncthreads();
     if (tid == 0) {
@@ -355,7 +325,7 @@ __global__ void __launch_bounds__(CDS_ROWS)
     MsCdStreamState* st = states + blockIdx.y;
     if (st->done) return;
 #define CD_STREAM_W(KK) cd_stream_w_body<KK>(X + pb.x_off, n, m, Wg + pb.w_off, Hg + pb.h_off, st, cd_sm)
-    CD_K_SWITCH(pb.k, CD_STREAM_W)
+    MS_NMF_K_SWITCH(pb.k, CD_STREAM_W)
 #undef CD_STREAM_W
 }
 
@@ -363,7 +333,7 @@ __global__ void __launch_bounds__(CDS_ROWS)
 __global__ void __launch_bounds__(64)
     ms_cd_stream_h_kernel(int m, const MsNmfProblem* __restrict__ problems, double* __restrict__ Hg,
                           MsCdStreamState* __restrict__ states, int mode, int iteration, double tol) {
-    __shared__ double sH[CD_MAX_K * CD_MAX_M];
+    __shared__ double sH[MS_NMF_MAX_K * MS_NMF_MAX_M];
     __shared__ double s_red[2];
     const MsNmfProblem pb = problems[blockIdx.x];
     MsCdStreamState* st = states + blockIdx.x;
@@ -389,7 +359,7 @@ __global__ void __launch_bounds__(64)
                 if (hess != 0.0) sH[t * m + tid] = fmax(h - grad / hess, 0.0);
             }
         }
-        vh = cd_warp_sum(vh);
+        vh = ms_warp_sum_d(vh);
         if ((tid & 31) == 0) s_red[tid >> 5] = vh;
         __syncthreads();
         for (int e = tid; e < k * m; e += 64) Hp[e] = sH[e];
@@ -415,7 +385,7 @@ __global__ void __launch_bounds__(64)
 __global__ void __launch_bounds__(256)
     ms_cd_stream_vaf_kernel(const double* __restrict__ X, long long n, int m, const MsNmfProblem* __restrict__ problems,
                             const double* __restrict__ Wg, const double* __restrict__ Hg, double* __restrict__ sums) {
-    __shared__ double sH[CD_MAX_K * CD_MAX_M];
+    __shared__ double sH[MS_NMF_MAX_K * MS_NMF_MAX_M];
     const MsNmfProblem pb = problems[blockIdx.y];
     const int k = pb.k;
     const double* Xp = X + pb.x_off;
@@ -450,11 +420,9 @@ __global__ void ms_cd_stream_finish_kernel(int m, const MsCdStreamState* __restr
     }
 }
 
-static size_t cd_align256(size_t b) { return (b + 255) / 256 * 256; }
-
 extern "C" int64_t ms_nmf_cd_stream_workspace_bytes(int32_t m, int32_t n_problems) {
     if (m < 1 || n_problems < 0) return 0;
-    return (int64_t)(cd_align256(sizeof(MsCdStreamState) * (size_t)n_problems) + sizeof(double) * 2 * (size_t)m * n_problems +
+    return (int64_t)(ms_align256(sizeof(MsCdStreamState) * (size_t)n_problems) + sizeof(double) * 2 * (size_t)m * n_problems +
                      256);
 }
 
@@ -462,45 +430,33 @@ extern "C" int ms_nmf_cd_stream(const double* d_X, int64_t n, int32_t m, const v
                                 int32_t kmax, double* d_W, double* d_H, int32_t max_iter, double tol, void* d_work,
                                 int32_t* d_n_iter, double* d_err, double* d_vaf, void* stream) {
     if (!d_X || !d_table || !d_W || !d_H || !d_work || !d_n_iter || !d_err || !d_vaf) return MS_E_INVALID;
-    if (n < 1 || m < 1 || m > CD_MAX_M || kmax < 1 || kmax > CD_MAX_K || n_problems < 0 || max_iter < 0 || !(tol >= 0.0))
+    if (n < 1 || m < 1 || m > MS_NMF_MAX_M || kmax < 1 || kmax > MS_NMF_MAX_K || n_problems < 0 || max_iter < 0 || !(tol >= 0.0))
         return MS_E_INVALID;
     if (n_problems == 0) return MS_OK;
     cudaStream_t st = (cudaStream_t)stream;
     const MsNmfProblem* d_problems = (const MsNmfProblem*)d_table;
     MsCdStreamState* d_states = (MsCdStreamState*)d_work;
-    double* d_sums = (double*)((char*)d_work + cd_align256(sizeof(MsCdStreamState) * (size_t)n_problems));
+    double* d_sums = (double*)((char*)d_work + ms_align256(sizeof(MsCdStreamState) * (size_t)n_problems));
     MS_CUDA_CHECK(cudaMemsetAsync(d_states, 0, sizeof(MsCdStreamState) * (size_t)n_problems, st));
 
     const long long n_tiles = (n + CDS_ROWS - 1) / CDS_ROWS;
     long long ctas = (148LL * 4 + n_problems - 1) / n_problems;  // about one wave of the W pass over all problems
     if (ctas > n_tiles) ctas = n_tiles;
-    const size_t smem = sizeof(double) * ((size_t)CDS_ROWS * (cd_odd(m) + cd_odd(kmax)) + (size_t)kmax * m + kmax * kmax + 32);
+    const size_t smem = sizeof(double) * ((size_t)CDS_ROWS * (ms_odd(m) + ms_odd(kmax)) + (size_t)kmax * m + kmax * kmax + 32);
     MS_CUDA_CHECK(cudaFuncSetAttribute(ms_cd_stream_w_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     ms_cd_stream_h_kernel<<<n_problems, 64, 0, st>>>(m, d_problems, d_H, d_states, 0, 0, tol);
     MS_COUNT_LAUNCH();
-    int32_t* h_done = (int32_t*)malloc(sizeof(MsCdStreamState) * (size_t)n_problems);
-    if (!h_done) return MS_E_INVALID;
     for (int it = 1; it <= max_iter; it++) {
         ms_cd_stream_w_kernel<<<dim3((unsigned)ctas, n_problems), CDS_ROWS, smem, st>>>(d_X, n, m, d_problems, d_W, d_H, d_states);
         MS_COUNT_LAUNCH();
         ms_cd_stream_h_kernel<<<n_problems, 64, 0, st>>>(m, d_problems, d_H, d_states, 1, it, tol);
         MS_COUNT_LAUNCH();
-        if (it % 64 == 0 && it < max_iter) {
-            // stop early once every problem has converged (pageable copy: waits for the stream)
-            cudaError_t e = cudaMemcpyAsync(h_done, d_states, sizeof(MsCdStreamState) * (size_t)n_problems,
-                                            cudaMemcpyDeviceToHost, st);
-            if (e == cudaSuccess) e = cudaStreamSynchronize(st);
-            if (e != cudaSuccess) {
-                free(h_done);
-                MS_CUDA_CHECK(e);
-            }
-            const MsCdStreamState* hs = (const MsCdStreamState*)h_done;
-            int all_done = 1;
-            for (int p = 0; p < n_problems; p++) all_done &= hs[p].done != 0;
-            if (all_done) break;
+        if (it % 64 == 0 && it < max_iter) {  // stop early once every problem has converged
+            const int done = ms_nmf_all_done(d_states, n_problems, st);
+            if (done < 0) return done;
+            if (done) break;
         }
     }
-    free(h_done);
     const int vaf_rows = 256 / m;
     long long vaf_ctas = (148LL * 8 + n_problems - 1) / n_problems, vaf_cap = (n + vaf_rows - 1) / vaf_rows;
     if (vaf_ctas > vaf_cap) vaf_ctas = vaf_cap;
@@ -518,12 +474,12 @@ extern "C" int ms_nmf_cd_stream(const double* d_X, int64_t n, int32_t m, const v
 // ---------------------------------------------------------------------------------------------------
 // Workspace per distinct matrix b of the stack (doubles): G [m][m] (X^T X), V [m][m] (right singular vectors,
 // column j = j-th largest), S [m] (singular values; 0 where the matrix is numerically rank deficient),
-// U2 [2][CD_MAX_K] (squared norms of the positive / negative parts of U[:, j] = X V[:, j] / S[j]), sum (of X).
+// U2 [2][MS_NMF_MAX_K] (squared norms of the positive / negative parts of U[:, j] = X V[:, j] / S[j]), sum (of X).
 struct MsNndsvdMatrix {
-    double G[CD_MAX_M * CD_MAX_M];
-    double V[CD_MAX_M * CD_MAX_M];
-    double S[CD_MAX_M];
-    double U2[2][CD_MAX_K];
+    double G[MS_NMF_MAX_M * MS_NMF_MAX_M];
+    double V[MS_NMF_MAX_M * MS_NMF_MAX_M];
+    double S[MS_NMF_MAX_M];
+    double U2[2][MS_NMF_MAX_K];
     double sum;
 };
 
@@ -531,14 +487,14 @@ struct MsNndsvdMatrix {
 __global__ void __launch_bounds__(CDS_ROWS)
     ms_nndsvd_gram_kernel(const double* __restrict__ X, long long n, int m, MsNndsvdMatrix* __restrict__ mats) {
     extern __shared__ double cd_sm[];
-    const int XS = cd_odd(m), n_out = m * m, tid = threadIdx.x;
+    const int XS = ms_odd(m), n_out = m * m, tid = threadIdx.x;
     const double* Xb = X + (long long)blockIdx.y * n * m;
     MsNndsvdMatrix* mt = mats + blockIdx.y;
     double* sX = cd_sm;                  // [CDS_ROWS][XS]
     double* s_red = sX + CDS_ROWS * XS;  // [32]
-    double acc[CD_MAX_M * CD_MAX_M / CD_THREADS];
+    double acc[MS_NMF_MAX_M * MS_NMF_MAX_M / CD_THREADS];
 #pragma unroll
-    for (int q = 0; q < CD_MAX_M * CD_MAX_M / CD_THREADS; q++) acc[q] = 0.0;
+    for (int q = 0; q < MS_NMF_MAX_M * MS_NMF_MAX_M / CD_THREADS; q++) acc[q] = 0.0;
     const int slices = cd_slices(n_out, CDS_ROWS), n_items = n_out * slices;
     double total = 0.0;
     const long long n_tiles = (n + CDS_ROWS - 1) / CDS_ROWS;
@@ -554,17 +510,17 @@ __global__ void __launch_bounds__(CDS_ROWS)
         __syncthreads();
         const int sl = cd_slices(n_out, rows);
 #pragma unroll
-        for (int q = 0; q < CD_MAX_M * CD_MAX_M / CD_THREADS; q++) {
+        for (int q = 0; q < MS_NMF_MAX_M * MS_NMF_MAX_M / CD_THREADS; q++) {
             const int item = tid + q * CDS_ROWS;
             if (item < n_items && item / n_out < sl) acc[q] += cd_gram_item(item % n_out, item / n_out, sl, rows, sX, XS, m, sX, XS, m);
         }
     }
 #pragma unroll
-    for (int q = 0; q < CD_MAX_M * CD_MAX_M / CD_THREADS; q++) {
+    for (int q = 0; q < MS_NMF_MAX_M * MS_NMF_MAX_M / CD_THREADS; q++) {
         const int item = tid + q * CDS_ROWS;
         if (item < n_items) atomicAdd(&mt->G[item % n_out], acc[q]);
     }
-    total = cd_warp_sum(total);
+    total = ms_warp_sum_d(total);
     if ((tid & 31) == 0) s_red[tid >> 5] = total;
     __syncthreads();
     if (tid == 0) {
@@ -577,10 +533,10 @@ __global__ void __launch_bounds__(CDS_ROWS)
 // Eigen-decomposition of G = X^T X by cyclic Jacobi rotations, one warp per matrix; S = sqrt of the eigenvalues in
 // descending order, V their eigenvectors.  An eigenvalue at or below m * eps * the largest one is treated as zero.
 __global__ void __launch_bounds__(32) ms_nndsvd_eig_kernel(int m, MsNndsvdMatrix* __restrict__ mats) {
-    __shared__ double A[CD_MAX_M * (CD_MAX_M + 1)];
-    __shared__ int order[CD_MAX_M];
+    __shared__ double A[MS_NMF_MAX_M * (MS_NMF_MAX_M + 1)];
+    __shared__ int order[MS_NMF_MAX_M];
     MsNndsvdMatrix* mt = mats + blockIdx.x;
-    const int lane = threadIdx.x, AS = CD_MAX_M + 1, VS = m;
+    const int lane = threadIdx.x, AS = MS_NMF_MAX_M + 1, VS = m;
     double* V = mt->G;  // G is read into A first; its storage then accumulates the rotations
     for (int e = lane; e < m * m; e += 32) {
         const int r = e / m, c = e % m;
@@ -643,50 +599,50 @@ __global__ void __launch_bounds__(32) ms_nndsvd_eig_kernel(int m, MsNndsvdMatrix
         const int r = e / m, j = e % m;
         mt->V[r * m + j] = V[r * VS + order[j]];
     }
-    for (int e = lane; e < 2 * CD_MAX_K; e += 32) mt->U2[e / CD_MAX_K][e % CD_MAX_K] = 0.0;
+    for (int e = lane; e < 2 * MS_NMF_MAX_K; e += 32) mt->U2[e / MS_NMF_MAX_K][e % MS_NMF_MAX_K] = 0.0;
 }
 
 // u_ij = X[i, :] . V[:, j] / S[j] for j < kk (S[j] == 0: 0, flagged by the fill kernel)
 __device__ __forceinline__ void nndsvd_u_row(const double* __restrict__ xrow, int m, const double* sV, const double* sInvS,
-                                             int kk, double (&u)[CD_MAX_K]) {
+                                             int kk, double (&u)[MS_NMF_MAX_K]) {
 #pragma unroll
-    for (int j = 0; j < CD_MAX_K; j++) u[j] = 0.0;
+    for (int j = 0; j < MS_NMF_MAX_K; j++) u[j] = 0.0;
     for (int c = 0; c < m; c++) {
         const double x = xrow[c];
 #pragma unroll
-        for (int j = 0; j < CD_MAX_K; j++)
-            if (j < kk) u[j] = fma(x, sV[c * CD_MAX_K + j], u[j]);
+        for (int j = 0; j < MS_NMF_MAX_K; j++)
+            if (j < kk) u[j] = fma(x, sV[c * MS_NMF_MAX_K + j], u[j]);
     }
 #pragma unroll
-    for (int j = 0; j < CD_MAX_K; j++) u[j] *= sInvS[j];
+    for (int j = 0; j < MS_NMF_MAX_K; j++) u[j] *= sInvS[j];
 }
 
 // pass 2 over X: squared norms of the positive and negative parts of the first kk left singular vectors
 __global__ void __launch_bounds__(256)
     ms_nndsvd_norms_kernel(const double* __restrict__ X, long long n, int m, int kk, MsNndsvdMatrix* __restrict__ mats) {
-    __shared__ double sV[CD_MAX_M * CD_MAX_K];
-    __shared__ double sInvS[CD_MAX_K];
+    __shared__ double sV[MS_NMF_MAX_M * MS_NMF_MAX_K];
+    __shared__ double sInvS[MS_NMF_MAX_K];
     MsNndsvdMatrix* mt = mats + blockIdx.y;
     const double* Xb = X + (long long)blockIdx.y * n * m;
-    for (int e = threadIdx.x; e < m * CD_MAX_K; e += 256) sV[e] = (e % CD_MAX_K) < kk ? mt->V[(e / CD_MAX_K) * m + e % CD_MAX_K] : 0.0;
-    for (int j = threadIdx.x; j < CD_MAX_K; j += 256) sInvS[j] = (j < kk && mt->S[j] > 0.0) ? 1.0 / mt->S[j] : 0.0;
+    for (int e = threadIdx.x; e < m * MS_NMF_MAX_K; e += 256) sV[e] = (e % MS_NMF_MAX_K) < kk ? mt->V[(e / MS_NMF_MAX_K) * m + e % MS_NMF_MAX_K] : 0.0;
+    for (int j = threadIdx.x; j < MS_NMF_MAX_K; j += 256) sInvS[j] = (j < kk && mt->S[j] > 0.0) ? 1.0 / mt->S[j] : 0.0;
     __syncthreads();
-    double pos[CD_MAX_K], neg[CD_MAX_K];
+    double pos[MS_NMF_MAX_K], neg[MS_NMF_MAX_K];
 #pragma unroll
-    for (int j = 0; j < CD_MAX_K; j++) pos[j] = neg[j] = 0.0;
+    for (int j = 0; j < MS_NMF_MAX_K; j++) pos[j] = neg[j] = 0.0;
     for (long long i = (long long)blockIdx.x * 256 + threadIdx.x; i < n; i += (long long)gridDim.x * 256) {
-        double u[CD_MAX_K];
+        double u[MS_NMF_MAX_K];
         nndsvd_u_row(Xb + i * m, m, sV, sInvS, kk, u);
 #pragma unroll
-        for (int j = 0; j < CD_MAX_K; j++) {
+        for (int j = 0; j < MS_NMF_MAX_K; j++) {
             if (u[j] > 0.0) pos[j] = fma(u[j], u[j], pos[j]);
             else neg[j] = fma(u[j], u[j], neg[j]);
         }
     }
 #pragma unroll
-    for (int j = 0; j < CD_MAX_K; j++) {
+    for (int j = 0; j < MS_NMF_MAX_K; j++) {
         if (j >= kk) break;
-        const double p = cd_warp_sum(pos[j]), q = cd_warp_sum(neg[j]);
+        const double p = ms_warp_sum_d(pos[j]), q = ms_warp_sum_d(neg[j]);
         if ((threadIdx.x & 31) == 0) {
             atomicAdd(&mt->U2[0][j], p);
             atomicAdd(&mt->U2[1][j], q);
@@ -700,10 +656,10 @@ __global__ void __launch_bounds__(256)
     ms_nndsvd_fill_kernel(const double* __restrict__ X, long long n, int m, const MsNmfProblem* __restrict__ problems,
                           const MsNndsvdMatrix* __restrict__ mats, int variant, double* __restrict__ Wg,
                           double* __restrict__ Hg, int32_t* __restrict__ status) {
-    __shared__ double sV[CD_MAX_M * CD_MAX_K];
-    __shared__ double sInvS[CD_MAX_K];
-    __shared__ double sScaleU[CD_MAX_K];  // W[:, j] = sScaleU[j] * (part of u_j); sign: +1 positive part, -1 negative
-    __shared__ double sSign[CD_MAX_K];
+    __shared__ double sV[MS_NMF_MAX_M * MS_NMF_MAX_K];
+    __shared__ double sInvS[MS_NMF_MAX_K];
+    __shared__ double sScaleU[MS_NMF_MAX_K];  // W[:, j] = sScaleU[j] * (part of u_j); sign: +1 positive part, -1 negative
+    __shared__ double sSign[MS_NMF_MAX_K];
     const MsNmfProblem pb = problems[blockIdx.y];
     const int k = pb.k;
     const long long b = pb.x_off / (n * m);
@@ -711,8 +667,8 @@ __global__ void __launch_bounds__(256)
     const double* Xb = X + pb.x_off;
     const double avg = mt->sum / ((double)n * m);
     const double eps = 1e-6;
-    for (int e = threadIdx.x; e < m * CD_MAX_K; e += 256) sV[e] = (e % CD_MAX_K) < k ? mt->V[(e / CD_MAX_K) * m + e % CD_MAX_K] : 0.0;
-    for (int j = threadIdx.x; j < CD_MAX_K; j += 256) sInvS[j] = (j < k && mt->S[j] > 0.0) ? 1.0 / mt->S[j] : 0.0;
+    for (int e = threadIdx.x; e < m * MS_NMF_MAX_K; e += 256) sV[e] = (e % MS_NMF_MAX_K) < k ? mt->V[(e / MS_NMF_MAX_K) * m + e % MS_NMF_MAX_K] : 0.0;
+    for (int j = threadIdx.x; j < MS_NMF_MAX_K; j += 256) sInvS[j] = (j < k && mt->S[j] > 0.0) ? 1.0 / mt->S[j] : 0.0;
     __syncthreads();
     if (threadIdx.x < k) {
         const int j = threadIdx.x;
@@ -720,7 +676,7 @@ __global__ void __launch_bounds__(256)
         bool bad = !(mt->S[j] > 0.0);
         double yp2 = 0.0, yn2 = 0.0;
         for (int c = 0; c < m; c++) {
-            const double v = sV[c * CD_MAX_K + j];
+            const double v = sV[c * MS_NMF_MAX_K + j];
             if (v > 0.0) yp2 += v * v;
             else yn2 += v * v;
         }
@@ -739,7 +695,7 @@ __global__ void __launch_bounds__(256)
             // H row j: lbd * (part of v) / its norm
             if (blockIdx.x == 0)
                 for (int c = 0; c < m; c++) {
-                    const double v = sign * sV[c * CD_MAX_K + j];
+                    const double v = sign * sV[c * MS_NMF_MAX_K + j];
                     double h = v > 0.0 ? lbd * v / yn_ : 0.0;
                     if (h < eps) h = variant ? avg : 0.0;
                     Hg[pb.h_off + (long long)j * m + c] = h;
@@ -747,7 +703,7 @@ __global__ void __launch_bounds__(256)
         }
         if (j == 0 && blockIdx.x == 0)
             for (int c = 0; c < m; c++) {
-                double h = scale * fabs(sV[c * CD_MAX_K]);
+                double h = scale * fabs(sV[c * MS_NMF_MAX_K]);
                 if (h < eps) h = variant ? avg : 0.0;
                 Hg[pb.h_off + c] = h;
             }
@@ -757,10 +713,10 @@ __global__ void __launch_bounds__(256)
     }
     __syncthreads();
     for (long long i = (long long)blockIdx.x * 256 + threadIdx.x; i < n; i += (long long)gridDim.x * 256) {
-        double u[CD_MAX_K];
+        double u[MS_NMF_MAX_K];
         nndsvd_u_row(Xb + i * m, m, sV, sInvS, k, u);
 #pragma unroll
-        for (int j = 0; j < CD_MAX_K; j++) {
+        for (int j = 0; j < MS_NMF_MAX_K; j++) {
             if (j >= k) break;
             const double s = sSign[j];
             const double part = s == 0.0 ? fabs(u[j]) : (s * u[j] > 0.0 ? s * u[j] : 0.0);
@@ -780,7 +736,7 @@ extern "C" int ms_nndsvd_init(const double* d_X, int64_t n, int32_t m, int32_t n
                               int32_t n_problems, int32_t kmax, int32_t variant, void* d_work, double* d_W, double* d_H,
                               int32_t* d_status, void* stream) {
     if (!d_X || !d_table || !d_work || !d_W || !d_H || !d_status) return MS_E_INVALID;
-    if (n < 1 || m < 1 || m > CD_MAX_M || n_matrices < 1 || n_problems < 0 || kmax < 1 || kmax > CD_MAX_K ||
+    if (n < 1 || m < 1 || m > MS_NMF_MAX_M || n_matrices < 1 || n_problems < 0 || kmax < 1 || kmax > MS_NMF_MAX_K ||
         kmax > m || kmax > n || (variant != 0 && variant != 1))
         return MS_E_INVALID;
     if (n_problems == 0) return MS_OK;
@@ -791,7 +747,7 @@ extern "C" int ms_nndsvd_init(const double* d_X, int64_t n, int32_t m, int32_t n
     const long long n_tiles = (n + CDS_ROWS - 1) / CDS_ROWS;
     long long ctas = (148LL * 4 + n_matrices - 1) / n_matrices;
     if (ctas > n_tiles) ctas = n_tiles;
-    const size_t smem = sizeof(double) * ((size_t)CDS_ROWS * cd_odd(m) + 32);
+    const size_t smem = sizeof(double) * ((size_t)CDS_ROWS * ms_odd(m) + 32);
     MS_CUDA_CHECK(cudaFuncSetAttribute(ms_nndsvd_gram_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     ms_nndsvd_gram_kernel<<<dim3((unsigned)ctas, n_matrices), CDS_ROWS, smem, st>>>(d_X, n, m, mats);
     MS_COUNT_LAUNCH();

@@ -25,27 +25,13 @@
 //
 // Every reduction behind a stop decision or an output has a fixed order (no floating-point atomics): two identical
 // calls give bit-identical W, n_iter, err and VAF.
-#include <stdio.h>
-
-#include "ms_common.cuh"
+#include "ms_nmf_common.cuh"
 
 #define FX_THREADS 256
-#define FX_MAX_K 16
-#define FX_MAX_M 64
 #define FX_CHUNK 32                                  // iterations a streaming row runs in registers per launch
 #define FX_MU_EPS 1.1920928955078125e-07             // np.finfo(np.float32).eps, sklearn's EPSILON
 #define FX_SOLVER_CD 0
 #define FX_SOLVER_MU 1
-
-// ms_nmf_plan's table (csrc/ms_nmf.cu): offsets are element counts, so they serve fp64 factors unchanged
-struct MsNmfProblem {
-    int k;
-    long long w_off;
-    long long h_off;
-    long long x_off;
-};
-
-__host__ __device__ inline int fx_odd(int v) { return v | 1; }  // shared row stride in doubles: no bank conflicts
 
 // ---------------------------------------------------------------------------------------------------
 // per-row functions shared by both regimes
@@ -130,37 +116,17 @@ __device__ __forceinline__ double fx_mu_row_err(const double (&w)[K], const doub
     return fma(-2.0, wx, xx) + q;
 }
 
-// fixed-order sum over the CTA (warp trees, then the warps in order); every thread gets the total
-__device__ __forceinline__ double fx_block_sum(double v, double* s_red) {
-    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-    __syncthreads();  // s_red is free
-    if ((threadIdx.x & 31) == 0) s_red[threadIdx.x >> 5] = v;
-    __syncthreads();
-    double total = 0.0;
-    for (int w = 0; w < (int)(blockDim.x >> 5); w++) total += s_red[w];
-    return total;
-}
-
-#define FX_K_SWITCH(KEXPR, CALL)                                                                                      \
-    switch (KEXPR) {                                                                                                  \
-        case 1: CALL(1); break;   case 2: CALL(2); break;   case 3: CALL(3); break;   case 4: CALL(4); break;         \
-        case 5: CALL(5); break;   case 6: CALL(6); break;   case 7: CALL(7); break;   case 8: CALL(8); break;         \
-        case 9: CALL(9); break;   case 10: CALL(10); break; case 11: CALL(11); break; case 12: CALL(12); break;       \
-        case 13: CALL(13); break; case 14: CALL(14); break; case 15: CALL(15); break; case 16: CALL(16); break;       \
-        default: break;                                                                                               \
-    }
-
 // ---------------------------------------------------------------------------------------------------
 // resident regime
 // ---------------------------------------------------------------------------------------------------
-// Shared memory (doubles): sX [n][XS], sW [n][WS], sXHt [n][WS], sXX [n], sH [K][m], sHHt [K][K], sPart [2][FX_MAX_M],
+// Shared memory (doubles): sX [n][XS], sW [n][WS], sXHt [n][WS], sXX [n], sH [K][m], sHHt [K][K], sPart [2][MS_NMF_MAX_M],
 // s_red [32]
 template <int K>
 __device__ __forceinline__ void fx_resident_body(const double* __restrict__ X, int n, int m, long long rs, long long cs,
                                                  double* __restrict__ Wp, const double* __restrict__ Hp, int solver,
                                                  int max_iter, double tol, int32_t* n_iter_out, double* err_out,
                                                  double* vaf_out, double* sm) {
-    const int XS = fx_odd(m), WS = fx_odd(K);
+    const int XS = ms_odd(m), WS = ms_odd(K);
     double* sX = sm;
     double* sW = sX + (size_t)n * XS;
     double* sXHt = sW + (size_t)n * WS;
@@ -168,7 +134,7 @@ __device__ __forceinline__ void fx_resident_body(const double* __restrict__ X, i
     double* sH = sXX + n;
     double* sHHt = sH + K * m;
     double* sPart = sHHt + K * K;
-    double* s_red = sPart + 2 * FX_MAX_M;
+    double* s_red = sPart + 2 * MS_NMF_MAX_M;
     const int tid = threadIdx.x;
 
     for (int i = tid; i < n * m; i += FX_THREADS) sX[(i / m) * XS + i % m] = X[(i / m) * rs + (i % m) * cs];
@@ -196,7 +162,7 @@ __device__ __forceinline__ void fx_resident_body(const double* __restrict__ X, i
             for (int t = 0; t < K; t++) w[t] = sW[i * WS + t], xht[t] = sXHt[i * WS + t];
             e += fx_mu_row_err<K>(w, xht, sXX[i], sHHt);
         }
-        stop_ref = prev = sqrt(fmax(fx_block_sum(e, s_red), 0.0));
+        stop_ref = prev = sqrt(fmax(ms_block_sum_d(e, s_red), 0.0));
     }
     int it = 0;
     for (it = 1; it <= max_iter; it++) {
@@ -216,7 +182,7 @@ __device__ __forceinline__ void fx_resident_body(const double* __restrict__ X, i
             for (int t = 0; t < K; t++) sW[i * WS + t] = w[t];
         }
         if (!check) continue;
-        const double total = fx_block_sum(part, s_red);
+        const double total = ms_block_sum_d(part, s_red);
         if (mu) {
             const double err = sqrt(fmax(total, 0.0));
             if ((prev - err) / stop_ref < tol) break;
@@ -241,13 +207,13 @@ __device__ __forceinline__ void fx_resident_body(const double* __restrict__ X, i
             r2 = fma(r, r, r2);
         }
         sPart[j] = r2;
-        sPart[FX_MAX_M + j] = c2;
+        sPart[MS_NMF_MAX_M + j] = c2;
         vaf_out[1 + j] = 1.0 - r2 / c2;
     }
     __syncthreads();
     if (tid == 0) {
         double r2 = 0.0, c2 = 0.0;
-        for (int j = 0; j < m; j++) r2 += sPart[j], c2 += sPart[FX_MAX_M + j];
+        for (int j = 0; j < m; j++) r2 += sPart[j], c2 += sPart[MS_NMF_MAX_M + j];
         *n_iter_out = it;
         *err_out = sqrt(r2);
         vaf_out[0] = 1.0 - r2 / c2;
@@ -265,18 +231,16 @@ __global__ void __launch_bounds__(FX_THREADS)
 #define FX_RESIDENT(KK)                                                                                               \
     fx_resident_body<KK>(X + pb.x_off, n, m, rs, cs, Wg + pb.w_off, Hg + pb.h_off, solver, max_iter, tol,             \
                          n_iter_out + p, err_out + p, vaf_out + (long long)p * (m + 1), fx_sm)
-    FX_K_SWITCH(pb.k, FX_RESIDENT)
+    MS_NMF_K_SWITCH(pb.k, FX_RESIDENT)
 #undef FX_RESIDENT
 }
 
-static size_t fx_resident_fixed(int m, int kmax) { return (size_t)kmax * m + (size_t)kmax * kmax + 2 * FX_MAX_M + 32; }
-static size_t fx_resident_row(int m, int kmax) { return (size_t)fx_odd(m) + 2 * (size_t)fx_odd(kmax) + 1; }
+static size_t fx_resident_fixed(int m, int kmax) { return (size_t)kmax * m + (size_t)kmax * kmax + 2 * MS_NMF_MAX_M + 32; }
+static size_t fx_resident_row(int m, int kmax) { return (size_t)ms_odd(m) + 2 * (size_t)ms_odd(kmax) + 1; }
 
 // Largest n the resident fixed-H kernel takes for (m, kmax); 0 if the shape is unsupported.
 extern "C" int32_t ms_nmf_fixed_h_resident_max_rows(int32_t m, int32_t kmax) {
-    if (m < 1 || m > FX_MAX_M || kmax < 1 || kmax > FX_MAX_K) return 0;
-    const size_t budget = 227 * 1024 - 1024;
-    return (int32_t)((budget - sizeof(double) * fx_resident_fixed(m, kmax)) / (sizeof(double) * fx_resident_row(m, kmax)));
+    return ms_nmf_max_rows(m, kmax, sizeof(double), fx_resident_fixed, fx_resident_row);
 }
 
 // ---------------------------------------------------------------------------------------------------
@@ -300,8 +264,6 @@ struct FxLayout {  // the workspace, carved by fx_layout
     double* vparts;     // [P][vctas][2][m]: per-CTA residual / total sums of squares per column
 };
 
-static size_t fx_align(size_t b) { return (b + 255) / 256 * 256; }
-
 static long long fx_ctas(long long n, int n_problems) {  // CTAs per problem in the streaming kernels
     long long ctas = (148LL * 8 + n_problems - 1) / n_problems, need = (n + FX_THREADS - 1) / FX_THREADS;
     return ctas < need ? ctas : need;
@@ -321,7 +283,7 @@ static size_t fx_layout(long long n, int m, int n_problems, int kmax, char* base
     void* ptrs[6];
     for (int s = 0; s < 6; s++) {
         ptrs[s] = base ? base + off : nullptr;
-        off += fx_align(sizes[s]);
+        off += ms_align256(sizes[s]);
     }
     if (L) {
         L->states = (MsFxState*)ptrs[0];
@@ -400,7 +362,7 @@ __global__ void __launch_bounds__(FX_THREADS)
 #define FX_CHUNK_BODY(KK)                                                                                             \
     fx_chunk_body<KK>(X + pb.x_off, n, m, rs, cs, Wg + pb.w_off, Hg + pb.h_off, solver, tol, it0, iters, first, xhtp,  \
                       L.xx + (long long)p * n, wsavep, parts, fx_sm)
-    FX_K_SWITCH(pb.k, FX_CHUNK_BODY)
+    MS_NMF_K_SWITCH(pb.k, FX_CHUNK_BODY)
 #undef FX_CHUNK_BODY
 }
 
@@ -421,7 +383,7 @@ __global__ void __launch_bounds__(FX_THREADS)
         if (mu && !(mu_checks && (s == 0 || it % 10 == 0))) continue;
         double v = 0.0;
         for (int c = threadIdx.x; c < ctas; c += FX_THREADS) v += parts[(long long)s * ctas + c];
-        const double total = fx_block_sum(v, s_red);  // the same value in every thread
+        const double total = ms_block_sum_d(v, s_red);  // the same value in every thread
         if (mu) {
             const double err = sqrt(fmax(total, 0.0));
             if (s == 0) {
@@ -487,7 +449,7 @@ __global__ void __launch_bounds__(FX_THREADS)
 #define FX_REPLAY(KK)                                                                                                 \
     fx_replay_body<KK>(n, m, Wg + pb.w_off, Hg + pb.h_off, solver, L.xht + (long long)p * n * kmax,                   \
                        L.wsave + (long long)p * n * kmax, st.replay_iters, fx_sm)
-    FX_K_SWITCH(pb.k, FX_REPLAY)
+    MS_NMF_K_SWITCH(pb.k, FX_REPLAY)
 #undef FX_REPLAY
 }
 
@@ -496,7 +458,7 @@ __global__ void __launch_bounds__(FX_THREADS)
     ms_fx_vaf_kernel(const double* __restrict__ X, long long n, int m, long long rs, long long cs,
                      const MsNmfProblem* __restrict__ problems, const double* __restrict__ Wg,
                      const double* __restrict__ Hg, FxLayout L) {
-    __shared__ double sH[FX_MAX_K * FX_MAX_M];
+    __shared__ double sH[MS_NMF_MAX_K * MS_NMF_MAX_M];
     __shared__ double sR[2][FX_THREADS];
     const MsNmfProblem pb = problems[blockIdx.y];
     const int k = pb.k;
@@ -526,7 +488,7 @@ __global__ void __launch_bounds__(FX_THREADS)
 
 __global__ void ms_fx_finish_kernel(int m, int vctas, FxLayout L, int32_t* __restrict__ n_iter, double* __restrict__ err,
                                     double* __restrict__ vaf) {
-    __shared__ double s_cols[2][FX_MAX_M];
+    __shared__ double s_cols[2][MS_NMF_MAX_M];
     const int p = blockIdx.x;
     const double* vp = L.vparts + (long long)p * vctas * 2 * m;
     for (int e = threadIdx.x; e < 2 * m; e += blockDim.x) {
@@ -549,7 +511,7 @@ __global__ void ms_fx_finish_kernel(int m, int vctas, FxLayout L, int32_t* __res
 // C ABI
 // ---------------------------------------------------------------------------------------------------
 extern "C" int64_t ms_nmf_fixed_h_workspace_bytes(int64_t n, int32_t m, int32_t n_problems, int32_t kmax) {
-    if (n < 1 || m < 1 || m > FX_MAX_M || n_problems < 0 || kmax < 1 || kmax > FX_MAX_K) return 0;
+    if (n < 1 || m < 1 || m > MS_NMF_MAX_M || n_problems < 0 || kmax < 1 || kmax > MS_NMF_MAX_K) return 0;
     if (n_problems == 0) return 256;
     return (int64_t)fx_layout(n, m, n_problems, kmax, nullptr, nullptr) + 256;
 }
@@ -559,7 +521,7 @@ extern "C" int ms_nmf_fixed_h(const double* d_X, int64_t n, int32_t m, int64_t r
                               int32_t solver, int32_t max_iter, double tol, int32_t regime, void* d_work,
                               int32_t* d_n_iter, double* d_err, double* d_vaf, void* stream) {
     if (!d_X || !d_table || !d_W || !d_H || !d_n_iter || !d_err || !d_vaf) return MS_E_INVALID;
-    if (n < 1 || m < 1 || m > FX_MAX_M || kmax < 1 || kmax > FX_MAX_K || n_problems < 0 || max_iter < 0 ||
+    if (n < 1 || m < 1 || m > MS_NMF_MAX_M || kmax < 1 || kmax > MS_NMF_MAX_K || n_problems < 0 || max_iter < 0 ||
         !(tol >= 0.0) || (solver != FX_SOLVER_CD && solver != FX_SOLVER_MU) || (regime != 0 && regime != 1) ||
         row_stride < 0 || col_stride < 0)
         return MS_E_INVALID;
@@ -581,11 +543,9 @@ extern "C" int ms_nmf_fixed_h(const double* d_X, int64_t n, int32_t m, int64_t r
     fx_layout(n, m, n_problems, kmax, (char*)d_work, &L);
     const int ctas = (int)fx_ctas(n, n_problems), vctas = (int)fx_vaf_ctas(n, m, n_problems);
     MS_CUDA_CHECK(cudaMemsetAsync(L.states, 0, sizeof(MsFxState) * (size_t)n_problems, st));
-    const size_t smem_chunk = sizeof(double) * ((size_t)kmax * FX_MAX_M + kmax * kmax + (FX_CHUNK + 1) * FX_THREADS);
-    const size_t smem_replay = sizeof(double) * ((size_t)kmax * FX_MAX_M + kmax * kmax);
+    const size_t smem_chunk = sizeof(double) * ((size_t)kmax * MS_NMF_MAX_M + kmax * kmax + (FX_CHUNK + 1) * FX_THREADS);
+    const size_t smem_replay = sizeof(double) * ((size_t)kmax * MS_NMF_MAX_M + kmax * kmax);
     MS_CUDA_CHECK(cudaFuncSetAttribute(ms_fx_chunk_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_chunk));
-    int32_t* h_states = (int32_t*)malloc(sizeof(MsFxState) * (size_t)n_problems);
-    if (!h_states) return MS_E_INVALID;
     for (int it0 = 0, chunk = 0; it0 < max_iter || chunk == 0; it0 += FX_CHUNK, chunk++) {
         const int iters = max_iter - it0 < FX_CHUNK ? max_iter - it0 : FX_CHUNK;
         const int first = chunk == 0;
@@ -597,22 +557,12 @@ extern "C" int ms_nmf_fixed_h(const double* d_X, int64_t n, int32_t m, int64_t r
         ms_fx_replay_kernel<<<dim3(ctas, n_problems), FX_THREADS, smem_replay, st>>>(n, m, d_problems, d_W, d_H, solver,
                                                                                      chunk, L, kmax);
         MS_COUNT_LAUNCH();
-        if (chunk % 2 == 1 && it0 + iters < max_iter) {
-            // stop early once every problem is done (pageable copy: waits for the stream)
-            cudaError_t e = cudaMemcpyAsync(h_states, L.states, sizeof(MsFxState) * (size_t)n_problems,
-                                            cudaMemcpyDeviceToHost, st);
-            if (e == cudaSuccess) e = cudaStreamSynchronize(st);
-            if (e != cudaSuccess) {
-                free(h_states);
-                MS_CUDA_CHECK(e);
-            }
-            const MsFxState* hs = (const MsFxState*)h_states;
-            int all_done = 1;
-            for (int p = 0; p < n_problems; p++) all_done &= hs[p].done != 0;
-            if (all_done) break;
+        if (chunk % 2 == 1 && it0 + iters < max_iter) {  // stop early once every problem is done
+            const int done = ms_nmf_all_done(L.states, n_problems, st);
+            if (done < 0) return done;
+            if (done) break;
         }
     }
-    free(h_states);
     ms_fx_vaf_kernel<<<dim3(vctas, n_problems), FX_THREADS, 0, st>>>(d_X, n, m, row_stride, col_stride, d_problems, d_W,
                                                                      d_H, L);
     MS_COUNT_LAUNCH();
